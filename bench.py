@@ -14,6 +14,7 @@ Contract (driver): ``python bench.py --gpus N --steps K --warmup W`` prints ONE 
   * ``cpu_baseline``: the oracle stack (reference env logic restated in numpy + float64 MuJoCo-restatement physics in C)
     on a bounded sample, single core ("port").
   * ``--impl reference``: the same oracle stack on all host cores, one process per core (what SubprocVecEnv does).
+  * ``--dump-outputs DIR``: the outputs of the headline leg's last timed step as DIR/<name>.npy (see write_outputs).
 """
 from __future__ import annotations
 
@@ -124,15 +125,35 @@ def fp32_peak_tflops(device_index: int) -> float:
     return out.value
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(directory: str, arrays: dict, shared: dict = None, limit: int = DUMP_LIMIT_BYTES) -> None:
+    """DIR/<name>.npy for every per-environment output array (first axis = environment) and every ``shared`` array
+    (written whole).  Above ``limit`` bytes in all, the same fixed, seeded sample of environments is kept in every
+    per-environment array and its indices go to env_index.npy."""
+    import numpy as np
+    shared = shared or {}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes // n for a in arrays.values())
+    fixed = 128 * (len(arrays) + len(shared) + 1) + sum(a.nbytes for a in shared.values())   # + .npy headers
+    if row_bytes * n + fixed > limit:
+        keep = (limit - fixed) // (row_bytes + 8)                # + 8: the float64 index of each kept environment
+        rows = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in {**arrays, **shared}.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 _WORKER = {}
 
 
 def _reference_tree():
-    """baseline/_ref (copy of the reference's Python made by baseline/build_ref.py) or the container's checkout"""
-    for root in (os.path.join(REPO, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(root, "drloco", "mujoco")):
-            return root
-    return None
+    """baseline/_ref (copy of the reference's Python made by baseline/build_ref.py), or None when it was not made"""
+    root = os.path.join(REPO, "baseline", "_ref")
+    return root if os.path.isdir(os.path.join(root, "drloco", "mujoco")) else None
 
 
 def _oracle_init(n_envs, seed_base, want_reference=True):
@@ -159,10 +180,21 @@ def _oracle_init(n_envs, seed_base, want_reference=True):
     from drloco_b200.walkers import make_spec
     from oracle.env_oracle import OracleVecEnv
     from oracle.physics import OraclePhysics
+    phys = [0.0]
+
+    class TimedPhysics(OraclePhysics):
+        """times the control-step integration, as ref_runner's MjSim stand-in does for the reference arm"""
+
+        def step(self, *a):
+            t0 = time.perf_counter()
+            bad = super().step(*a)
+            phys[0] += time.perf_counter() - t0
+            return bad
+
     spec = make_spec()
-    venv = OracleVecEnv(spec, n_envs, lambda: OraclePhysics(spec.model))
+    venv = OracleVecEnv(spec, n_envs, lambda: TimedPhysics(spec.model))
     venv.reset()
-    _WORKER.update(kind="port", venv=venv, rng=np.random.default_rng(seed), n=n_envs, act=spec.act_dim, phys=[0.0])
+    _WORKER.update(kind="port", venv=venv, rng=np.random.default_rng(seed), n=n_envs, act=spec.act_dim, phys=phys)
 
 
 def _oracle_run(n_steps):
@@ -288,7 +320,15 @@ def main():
     ap.add_argument("--pre-warmup", type=int, default=1500,
                     help="untimed steps before the W warm-up steps of the headline leg (clock / power-state ramp)")
     ap.add_argument("--no-extra", action="store_true", help="skip the time-bounded legs for BASELINE.json configs[2] / [3]")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of the headline leg, write the outputs of its last step (rank 0) as "
+                         "DIR/<name>.npy (float32; the normalisation statistics float64); the inputs depend only on the "
+                         "arguments, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA arm (--impl b200)")
     args.warmup = max(args.warmup, 3)
     # the contract is ONE JSON line on stdout: keep a private handle to the real stdout and point fd 1 at stderr so
     # that library chatter (e.g. NCCL's version banner) cannot end up in front of it
@@ -331,8 +371,9 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def measure(env_id, n, integrator, steps, warmup, with_clocks=False, flushed_steps=0, e2e_steps=0):
-        """one workload on this rank's GPU: W warm-up steps, then K timed steps of every flavour"""
+    def measure(env_id, n, integrator, steps, warmup, with_clocks=False, flushed_steps=0, e2e_steps=0, dump=False):
+        """one workload on this rank's GPU: W warm-up steps, then K timed steps of every flavour; dump=True keeps the
+        outputs of the last device-resident timed step as host arrays (out["outputs"])"""
         sampler = ClockSampler(local) if with_clocks else None
         if sampler:
             sampler.start()
@@ -382,6 +423,18 @@ def main():
         out["kernel_ms"] = float(np.mean([a.elapsed_time(b) for a, b in kev]))
         out["launches"] = env.launches + vn.launches - launches0
         out["stats"] = env.stats()
+        if dump:
+            # what a caller of this loop holds after its last step: the env's outputs, their normalised form and the
+            # running statistics they were normalised with (VecNormalize.obs_rms / ret_rms, float64).  Terminal
+            # observations exist for finished environments only; the other rows are zeroed.
+            fin = done.bool()
+            outputs = {"obs": obs, "reward": rew, "done": done, "norm_obs": vn.norm_obs_buf,
+                       "norm_reward": vn.norm_rew_buf,
+                       "terminal_obs": torch.where(fin[:, None], env.terminal_obs, torch.zeros_like(env.terminal_obs))}
+            out["outputs"] = {k: v.float().cpu().numpy() for k, v in outputs.items()}
+            orms, rrms = vn.obs_rms, vn.ret_rms
+            out["rms"] = {"obs_rms_mean": orms.mean, "obs_rms_var": orms.var,
+                          "ret_rms_var": np.array([rrms.var], np.float64)}
         # ---- the same steps as a policy sees them: the normalised observation of step k before step k+1 starts ----
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
         barrier()
@@ -437,7 +490,10 @@ def main():
 
     n = args.envs_per_gpu
     head = measure(args.env_id, n, args.integrator, args.steps, args.warmup, with_clocks=True,
-                   flushed_steps=min(args.steps, 50), e2e_steps=0 if args.no_e2e else args.steps)
+                   flushed_steps=min(args.steps, 50), e2e_steps=0 if args.no_e2e else args.steps,
+                   dump=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, head["outputs"], head["rms"])
     # ---- the other GPU configurations of BASELINE.json, time-bounded (a few dozen steps each) ----
     extra = {}
     if not args.no_extra and args.env_id == ENV_ID and args.integrator == "rk4":

@@ -7,7 +7,9 @@ import pytest
 
 from drloco_b200 import model as M
 
-REF_XML = "/root/reference/drloco/mujoco/xml/"
+# the reference's own MJCF files, in the verbatim copy of its `drloco` package that baseline/build_ref.py makes
+REF_XML = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
+                       "baseline", "_ref", "drloco", "mujoco", "xml", "")
 
 
 @pytest.mark.parametrize("env_id,xml,nv,nu,nb,mass", [
@@ -19,7 +21,7 @@ def test_builtin_specs(env_id, xml, nv, nu, nb, mass):
     assert abs(m.total_mass - mass) < 1e-9                     # SURVEY.md §8a (a4)
     assert np.all(m.act_ctrlrange == [-300, 300]) and np.all(m.act_forcerange == [-300, 300])
     assert len(m.site_body) == 8
-    if os.path.exists(REF_XML + xml):                          # only in the build container
+    if os.path.exists(REF_XML + xml):                          # only where the reference copy was made
         ref = M.load_mjcf(REF_XML + xml)
         for f in dataclasses.fields(m):
             x, y = getattr(m, f.name), getattr(ref, f.name)
