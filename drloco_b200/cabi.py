@@ -9,8 +9,9 @@ import ctypes as C
 
 import numpy as np
 
-DRL_ABI_VERSION = 2
+DRL_ABI_VERSION = 3
 MAX_DOF, MAX_BODY, MAX_ACT, MAX_SPHERE, MAX_BOX, MAX_SITE, MAX_OBS, MAX_PHASE_JOINTS = 24, 12, 16, 16, 8, 16, 64, 4
+MAX_EE = 4
 INTEGRATOR_RK4, INTEGRATOR_EULER = 0, 1
 CURSOR_STEPWISE, CURSOR_WRAP = 0, 1
 PHASE_FROM_CURSOR, PHASE_FROM_JOINTS = 0, 1
@@ -43,6 +44,7 @@ class DrlWalkerModel(C.Structure):
         ("box_body", i32 * MAX_BOX), ("box_center", d * 3 * MAX_BOX), ("box_corner", d * 3 * 8 * MAX_BOX),
         ("box_mu", d * MAX_BOX),
         ("site_body", i32 * MAX_SITE), ("site_pos", d * 3 * MAX_SITE),
+        ("n_ee", i32), ("ee_body", i32 * MAX_EE), ("ee_pos", d * 3 * MAX_EE),
     ]
 
 
@@ -57,6 +59,7 @@ class DrlConfig(C.Structure):
         ("mirror_obs_idx", i32 * MAX_OBS), ("mirror_obs_sign", C.c_float * MAX_OBS),
         ("mirror_act_idx", i32 * MAX_ACT), ("mirror_act_sign", C.c_float * MAX_ACT),
         ("lanes_per_env", i32), ("early_termination", i32), ("monitor_median_torque", i32),
+        ("ee_weight", d), ("ee_scale", d),
     ]
 
 
@@ -73,11 +76,12 @@ def pack_model(m) -> DrlWalkerModel:
     """drloco_b200.model.WalkerModel -> DrlWalkerModel."""
     from .model import GRAVITY_Z, SOLREF, SOLIMP
     if m.nv > MAX_DOF or m.nb > MAX_BODY or m.nu > MAX_ACT or len(m.sphere_body) > MAX_SPHERE \
-            or len(m.box_body) > MAX_BOX or len(m.site_body) > MAX_SITE:
+            or len(m.box_body) > MAX_BOX or len(m.site_body) > MAX_SITE or len(m.ee_body) > MAX_EE:
         raise ValueError("model exceeds the fixed capacities of DrlWalkerModel")
     s = DrlWalkerModel()
     s.nv, s.nb, s.nu = m.nv, m.nb, m.nu
     s.n_sphere, s.n_box, s.n_site = len(m.sphere_body), len(m.box_body), len(m.site_body)
+    s.n_ee = len(m.ee_body)
     s.timestep, s.gravity_z = m.timestep, GRAVITY_Z
     _fill(s.solref, SOLREF)
     _fill(s.solimp, SOLIMP)
@@ -85,6 +89,6 @@ def pack_model(m) -> DrlWalkerModel:
                  "dof_type", "dof_axis_idx", "dof_axis_sign", "dof_ref", "dof_damping", "dof_armature", "dof_limited",
                  "dof_range", "dof_invweight0", "act_dof", "act_gear", "act_ctrlrange", "act_forcerange", "sphere_body",
                  "sphere_pos", "sphere_radius", "sphere_mu", "box_body", "box_center", "box_corner", "box_mu",
-                 "site_body", "site_pos"):
+                 "site_body", "site_pos", "ee_body", "ee_pos"):
         _fill(getattr(s, name), getattr(m, name))
     return s

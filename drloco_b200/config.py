@@ -41,6 +41,10 @@ class EnvConfig:
                                                         # median_abs_torque_smoothed (monitor_wrapper.py:131; 4 *
                                                         # ep_dur_max bytes per env and a radix-select median at every
                                                         # episode end).  The reference's callback never reads it.
+    ee_weight: float = 0.0                              # DeepMimic end-effector (foot position) reward term, added to
+                                                        # the imitation reward with this weight; 0 = off, as in the
+                                                        # reference (see README "End-effector reward")
+    ee_scale: float = 40.0                              # ee_rew = exp(-ee_scale * sum of squared foot-position errors)
     gamma: float = 0.0                                  # 0 -> by ctrl_freq, hypers.py:68
     integrator: str = "rk4"                             # xml:11; "euler" = MuJoCo semi-implicit Euler (fast mode)
     seed: int = 33                                      # utils.py:97

@@ -91,6 +91,9 @@ struct DrlEnv {
   int stage_barrier = 1;
   float* tor_hist = nullptr;
   float* med_tor_sm = nullptr;
+  // end-effector term (cfg.ee_weight > 0): last / smoothed ee_rew, lifetime sum
+  float* ee_f = nullptr;
+  double* ee_d = nullptr;
   // per-step statistics rows (one per thread block of the step kernel) + the ticket that elects the summing block
   double* cta_rows = nullptr;
   unsigned* cta_ticket = nullptr;
@@ -116,6 +119,10 @@ extern "C" int drl_create(const DrlConfig* cfg, DrlEnv** out) {
   if (cfg->frame_skip < 0) return fail(DRL_ERR_INVALID, "drl_create: frame_skip must be >= 0");
   if (cfg->integrator != DRL_INTEGRATOR_RK4 && cfg->integrator != DRL_INTEGRATOR_EULER)
     return fail(DRL_ERR_INVALID, "drl_create: unknown integrator");
+  if (!isfinite(cfg->ee_weight) || cfg->ee_weight < 0.0)
+    return fail(DRL_ERR_INVALID, "drl_create: ee_weight must be finite and >= 0");
+  if (cfg->ee_weight > 0.0 && !(cfg->ee_scale > 0.0 && isfinite(cfg->ee_scale)))
+    return fail(DRL_ERR_INVALID, "drl_create: ee_scale must be positive and finite when ee_weight > 0");
   int ndev = 0;
   CUDA_TRY(cudaGetDeviceCount(&ndev));
   if (cfg->device < 0 || cfg->device >= ndev) return fail(DRL_ERR_INVALID, "drl_create: no CUDA device %d", cfg->device);
@@ -133,7 +140,7 @@ extern "C" int drl_destroy(DrlEnv* e) {
   void* ptrs[] = {e->d_model, e->state_f, e->state_i, e->state_as, e->state_d, e->extras_last, e->stats, e->ref, e->step_vel,
                   e->step_last_comx, e->des_vel_prefix, e->step_off, e->step_len, e->left_step, e->ring_len,
                   e->ring_ret, e->ring_head, e->debug, e->speed_profile, e->ring_rsi_pos, e->ring_et_pos, e->ring_difficult,
-                  e->cta_rows, e->cta_ticket, e->tor_hist, e->med_tor_sm};
+                  e->cta_rows, e->cta_ticket, e->tor_hist, e->med_tor_sm, e->ee_f, e->ee_d};
   for (void* p : ptrs)
     if (p) cudaFree(p);
   delete e;
@@ -162,6 +169,12 @@ static int alloc_state(DrlEnv* e, size_t N) {
     CUDA_TRY(cudaMemset(e->tor_hist, 0, N * cap * sizeof(float)));
     CUDA_TRY(cudaMalloc(&e->med_tor_sm, N * sizeof(float)));
     CUDA_TRY(cudaMemset(e->med_tor_sm, 0, N * sizeof(float)));
+  }
+  if (e->cfg.ee_weight > 0.0) {
+    CUDA_TRY(cudaMalloc(&e->ee_f, N * 2 * sizeof(float)));
+    CUDA_TRY(cudaMemset(e->ee_f, 0, N * 2 * sizeof(float)));
+    CUDA_TRY(cudaMalloc(&e->ee_d, N * sizeof(double)));
+    CUDA_TRY(cudaMemset(e->ee_d, 0, N * sizeof(double)));
   }
   {
     // the smallest CTA the library launches carries 32 / G environments
@@ -192,7 +205,7 @@ static void free_state(DrlEnv* e) {
                    (void**)&e->state_d, (void**)&e->extras_last, (void**)&e->stats, (void**)&e->ring_len,
                    (void**)&e->ring_ret, (void**)&e->ring_head, (void**)&e->ring_rsi_pos, (void**)&e->ring_et_pos,
                    (void**)&e->ring_difficult, (void**)&e->cta_rows, (void**)&e->cta_ticket,
-                   (void**)&e->tor_hist, (void**)&e->med_tor_sm};
+                   (void**)&e->tor_hist, (void**)&e->med_tor_sm, (void**)&e->ee_f, (void**)&e->ee_d};
   for (void** p : ptrs) {
     if (*p) cudaFree(*p);
     *p = nullptr;
@@ -327,6 +340,16 @@ extern "C" int drl_upload_model(DrlEnv* e, const DrlWalkerModel* m) {
     for (int k = 0; k < 3; k++) d.site_pos[s][k] = (float)m->site_pos[s][k];
   }
   if (m->n_site == 0) return fail(DRL_ERR_INVALID, "model: foot-corner sites are required (mimic_env.py:546-559)");
+  if (m->n_ee < 0 || m->n_ee > DRL_MAX_EE || m->n_ee > kMaxEE)
+    return fail(DRL_ERR_INVALID, "model: n_ee must be in 0..%d", DRL_MAX_EE);
+  d.n_ee = m->n_ee;
+  for (int x = 0; x < m->n_ee; x++) {
+    if (m->ee_body[x] < 0 || m->ee_body[x] >= m->nb) return fail(DRL_ERR_INVALID, "model: ee_body[%d] out of range", x);
+    d.ee_body[x] = m->ee_body[x];
+    for (int k = 0; k < 3; k++) d.ee_pos[x][k] = (float)m->ee_pos[x][k];
+  }
+  if (c.ee_weight > 0.0 && m->n_ee == 0)
+    return fail(DRL_ERR_INVALID, "config: ee_weight > 0 needs end-effector points in the model (n_ee == 0)");
   // ---- configuration ----
   d.frame_skip = c.frame_skip; d.integrator = c.integrator; d.ep_dur_max = c.ep_dur_max;
   d.mirror_policy = c.mirror_policy; d.phase_mode = c.phase_mode; d.n_phase_joints = c.n_phase_joints;
@@ -339,6 +362,7 @@ extern "C" int drl_upload_model(DrlEnv* e, const DrlWalkerModel* m) {
   d.ctrl_freq_inv = (float)(1.0 / c.ctrl_freq);
   d.w_pos = (float)c.rew_weights[0]; d.w_vel = (float)c.rew_weights[1]; d.w_com = (float)c.rew_weights[2];
   d.rew_scale = (float)c.rew_scale; d.alive_bonus = (float)c.alive_bonus; d.fall_z = (float)c.fall_z;
+  d.w_ee = (float)c.ee_weight; d.ee_scale = (float)c.ee_scale;
   for (int i = 0; i < c.obs_dim; i++) {
     d.mirror_obs_idx[i] = c.mirror_obs_idx[i]; d.mirror_obs_sign[i] = c.mirror_obs_sign[i];
     if (c.mirror_obs_idx[i] < 0 || c.mirror_obs_idx[i] >= c.obs_dim) return fail(DRL_ERR_INVALID, "config: mirror_obs_idx");
@@ -449,6 +473,7 @@ static StepArgs make_args(DrlEnv* e) {
   a.stage_barrier = e->stage_barrier;
   a.cta_rows = e->cta_rows; a.cta_ticket = e->cta_ticket;
   a.tor_hist = e->tor_hist; a.med_tor_sm = e->med_tor_sm;
+  a.ee_f = e->ee_f; a.ee_d = e->ee_d;
   a.vn_ret = e->vn_ret; a.vn_gamma = e->vn_gamma; a.packed = e->vn_packed;
   if (e->playback) a.frame_skip = 0;
   a.debug = e->debug;
@@ -584,6 +609,23 @@ extern "C" int drl_get_median_torque(DrlEnv* e, float* out, void* stream) {
   if (!e->med_tor_sm) return fail(DRL_ERR_STATE, "drl_get_median_torque: the env was created with monitor_median_torque = 0");
   CUDA_TRY(cudaMemcpyAsync(out, e->med_tor_sm, (size_t)e->cfg.num_envs * sizeof(float), cudaMemcpyDeviceToDevice,
                            (cudaStream_t)stream));
+  return DRL_OK;
+}
+
+extern "C" int drl_get_ee_reward(DrlEnv* e, float* last, float* smoothed, void* stream) {
+  int rc = ready(e, "drl_get_ee_reward");
+  if (rc) return rc;
+  DeviceGuard guard__(e->cfg.device);
+  if (!e->ee_f) return fail(DRL_ERR_STATE, "drl_get_ee_reward: the env was created with ee_weight = 0");
+  const size_t n = (size_t)e->cfg.num_envs;
+  cudaStream_t st = (cudaStream_t)stream;
+  // columns of the [N][2] rows
+  if (last)
+    CUDA_TRY(cudaMemcpy2DAsync(last, sizeof(float), e->ee_f, 2 * sizeof(float), sizeof(float), n,
+                               cudaMemcpyDeviceToDevice, st));
+  if (smoothed)
+    CUDA_TRY(cudaMemcpy2DAsync(smoothed, sizeof(float), e->ee_f + 1, 2 * sizeof(float), sizeof(float), n,
+                               cudaMemcpyDeviceToDevice, st));
   return DRL_OK;
 }
 

@@ -13,6 +13,7 @@ constexpr int kMaxAct = 16;
 constexpr int kMaxCand = 64;     // contact candidates: 8 corners per box, 1 per capsule end
 constexpr int kMaxSite = 16;
 constexpr int kMaxObs = 64;
+constexpr int kMaxEE = 4;        // end-effector points (DRL_MAX_EE)
 
 // alignas(16): the step kernel stages this struct into shared memory in 16-byte chunks (sizeof must be a multiple of 16)
 struct alignas(16) DevModel {
@@ -59,6 +60,10 @@ struct alignas(16) DevModel {
   int cursor_mode, increment, n_steps, n_samples, com_z_col, des_vel_window;
   unsigned long long seed;
   long long env_id_offset;
+  // ---- optional end-effector reward term (DrlConfig.ee_weight; w_ee == 0: off) ----
+  int n_ee, ee_body[kMaxEE];
+  float ee_pos[kMaxEE][3];           // point in the body frame
+  float w_ee, ee_scale;
 };
 
 static_assert(sizeof(DevModel) % 16 == 0, "DevModel is copied in int4 chunks");
@@ -125,6 +130,9 @@ struct StepArgs {
   float* vn_ret;                     // [N] discounted-return accumulator, in/out
   float vn_gamma;
   double* packed;                    // [2*obs_dim + 3] batch moments of the step, out
+  // end-effector term, allocated only when it is on (DevModel::w_ee != 0), null otherwise
+  float* ee_f;                       // [N][2] ee_rew of the last step (1 after a reset), Monitor-smoothed mean
+  double* ee_d;                      // [N] lifetime sum of ee_rew (Monitor never clears its per-step lists)
 };
 
 }  // namespace drl

@@ -265,6 +265,44 @@ __device__ __forceinline__ void write_obs(const DevModel& M, ES& E, int l, bool 
   __syncwarp();
 }
 
+// cos / sin of every hinge angle (slides: displacement) of the joint configuration q into E.cssn, the input of
+// tree_kinematics
+template <class ES>
+__device__ __forceinline__ void publish_joint_trig(const DevModel& M, ES& E, const LaneConst& L, float q) {
+  const int l = L.l;
+  const float ref = M.dof_ref[L.isdof ? l : 0];
+  float s = q - ref, cc = 1.f;
+  if (L.isdof && L.type == 1) sincos_joint(M.dof_sign[l] * (q - ref), s, cc);
+  if (L.isdof) *reinterpret_cast<float2*>(&E.cssn[l][0]) = make_float2(cc, s);
+  __syncwarp();
+}
+
+// Sum over the end-effector points of |p(q) - p(rq)|^2, p = the point relative to the root-body origin in world axes
+// (the frame of E.bodyR, so the root slides drop out).  Lane e < n_ee owns point e.  Overwrites E.cssn and the body
+// frames / joint axes of the first EnvSmem union; E.obsbuf and E.Mt are untouched.  Called by every lane of the warp.
+template <int NV, int G, class ES>
+__device__ __noinline__ float ee_sq_error(const DevModel& M, ES& E, const LaneConst& L, const ChainLane& CL, float q,
+                                          float rq) {
+  const int l = L.l;
+  const bool own = l < M.n_ee;
+  const int e = own ? l : 0;
+  const int b = M.ee_body[e];
+  const float p0 = M.ee_pos[e][0], p1 = M.ee_pos[e][1], p2 = M.ee_pos[e][2];
+  float d[3] = {0.f, 0.f, 0.f};
+#pragma unroll 1
+  for (int pass = 0; pass < 2; pass++) {
+    publish_joint_trig(M, E, L, pass == 0 ? q : rq);
+    tree_kinematics<NV, G>(M, E, CL, l);
+#pragma unroll
+    for (int r = 0; r < 3; r++) {
+      const float4 row = *reinterpret_cast<const float4*>(&E.bodyR[b][4 * r]);
+      const float x = row.w + row.x * p0 + row.y * p1 + row.z * p2;
+      d[r] = pass == 0 ? x : d[r] - x;
+    }
+  }
+  return group_sum<G>(own ? d[0] * d[0] + d[1] * d[1] + d[2] * d[2] : 0.f);
+}
+
 template <int NV, int G, class ES>
 __device__ __noinline__ void reset_env(const DevModel& M, const StepArgs& A, ES& E, const LaneConst& L,
                                        const ChainLane& CL, int env, Cursor& c, float& q, float& v, float& dist,
@@ -300,13 +338,7 @@ __device__ __noinline__ void reset_env(const DevModel& M, const StepArgs& A, ES&
   ref_lookup(M, A, c, dist, zoff, l, G, L.isdof, rq, rv);
   q = rq; v = rv;
   // set_state + sim.forward: lowest foot-corner site (mimic_env.py:546-559)
-  {
-    const float ref = M.dof_ref[L.isdof ? l : 0];
-    float s = q - ref, cc = 1.f;
-    if (L.isdof && L.type == 1) sincos_joint(M.dof_sign[l] * (q - ref), s, cc);
-    if (L.isdof) *reinterpret_cast<float2*>(&E.cssn[l][0]) = make_float2(cc, s);
-  }
-  __syncwarp();
+  publish_joint_trig(M, E, L, q);
   float zO = M.root_z0;
   for (int j = 0; j < M.nslide; j++) zO = fmaf(M.dof_slide_z[j], E.cssn[j][1], zO);
   tree_kinematics<NV, G>(M, E, CL, l);
@@ -392,6 +424,7 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
         sf[3 * G + kMiscDist] = dist; sf[3 * G + kMiscZoff] = zoff;
         sf[3 * G + kMiscWalked] = 0.f; sf[3 * G + kMiscEpRet] = 0.f; sf[3 * G + kMiscEpTor] = 0.f;
         sf[3 * G + kMiscPrevPos] = 1.f; sf[3 * G + kMiscPrevVel] = 1.f; sf[3 * G + kMiscPrevCom] = 1.f;
+        if (A.ee_f) A.ee_f[2 * (size_t)env] = 1.f;
         si[kCurIstep] = c.i_step; si[kCurPos] = c.pos; si[kCurCount] = c.count; si[kCurEpDur] = 0;
         si[kCurRsiStep] = c.rsi_step; si[kCurNDet] = c.n_det; si[kCurResets] = c.resets; si[kCurFlags] = c.flags;
       }
@@ -539,6 +572,14 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
       com_rew = expf(-16.f * sc);
     }
   }
+  // optional DeepMimic end-effector term (w_ee lives in the CTA's shared model block: warp-uniform).  Same rules as the
+  // three terms above: kept from the previous step on a terminal step or a blow-up, 1 after a reset.
+  float ee_rew = 1.f;
+  if (M.w_ee != 0.f) {
+    ee_rew = A.ee_f[2 * (size_t)env];
+    const float se = ee_sq_error<NV, G>(M, E, L, CL, q, rq);
+    if (!done && !bad) ee_rew = expf(-M.ee_scale * se);
+  }
   if (bad) {
     // MujocoException path (mimic_env.py:86-91): reset, reward 0, done; the VecEnv then resets again (Q19) — here a
     // single reset serves both, and the terminal observation is the post-reset observation as in the reference
@@ -547,7 +588,9 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
   } else if (done) {
     reward = timeout ? 0.f : -0.f;                              // _get_ET_reward always evaluates to +-0 (Q1)
   } else {
-    reward = (M.w_pos * pos_rew + M.w_vel * vel_rew + M.w_com * com_rew) * M.rew_scale + M.alive_bonus;
+    float imit = M.w_pos * pos_rew + M.w_vel * vel_rew + M.w_com * com_rew;
+    if (M.w_ee != 0.f) imit = fmaf(M.w_ee, ee_rew, imit);
+    reward = imit * M.rew_scale + M.alive_bonus;
   }
   {
     const bool left1 = M.mirror_policy && A.left_step[c.i_step];
@@ -582,6 +625,7 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
   double* sd = A.state_d + (size_t)env * 4;
   if (l == 0 && live) {
     sd[0] += (double)pos_rew; sd[1] += (double)vel_rew; sd[2] += (double)com_rew; sd[3] += 1.0;
+    if (A.ee_d) A.ee_d[env] += (double)ee_rew;
     srow[kRowStats + DRL_STAT_ENV_STEPS] = 1.0;
     srow[kRowStats + DRL_STAT_POS_REW_SUM] = (double)pos_rew;
     srow[kRowStats + DRL_STAT_VEL_REW_SUM] = (double)vel_rew;
@@ -625,6 +669,11 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
     smooth(kMiscEpLenSm, 1, (float)ep_len, 0.75f);
     smooth(kMiscTorSm, 1, ep_tor / (float)ep_len, 0.75f);
     if (A.tor_hist) A.med_tor_sm[env] = (fl >> 1) & 1 ? 0.75f * med_tor + 0.25f * A.med_tor_sm[env] : med_tor;
+    if (A.ee_f) {
+      const float nv = (float)(A.ee_d[env] / sd[3]);
+      float& sm = A.ee_f[2 * (size_t)env + 1];
+      sm = (fl >> 1) & 1 ? 0.9f * nv + (1.f - 0.9f) * sm : nv;
+    }
     c.flags |= 2;
     ms[kMiscMoved] = walked;
     srow[kRowStats + DRL_STAT_EPISODES] = 1.0;
@@ -660,6 +709,7 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
       AS.bits[0] = AS.bits[1] = 0u; AS.prev_act = 0u; AS.lbit = AS.prev_lim = false;
       walked = 0.f; ep_ret = 0.f; ep_tor = 0.f;
       pos_rew = vel_rew = com_rew = 1.f;      // get_imitation_reward() inside reset_model (mimic_env.py:562)
+      ee_rew = 1.f;
     }
   }
   // ---- store -------------------------------------------------------------------------------------------------------
@@ -673,6 +723,7 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
       float* ms = sf + 3 * G;
       ms[kMiscDist] = dist; ms[kMiscZoff] = zoff; ms[kMiscWalked] = walked; ms[kMiscEpRet] = ep_ret;
       ms[kMiscEpTor] = ep_tor; ms[kMiscPrevPos] = pos_rew; ms[kMiscPrevVel] = vel_rew; ms[kMiscPrevCom] = com_rew;
+      if (A.ee_f) A.ee_f[2 * (size_t)env] = ee_rew;
       si[kCurIstep] = c.i_step; si[kCurPos] = c.pos; si[kCurCount] = c.count; si[kCurEpDur] = c.ep_dur;
       si[kCurRsiStep] = c.rsi_step; si[kCurNDet] = c.n_det; si[kCurResets] = c.resets; si[kCurFlags] = c.flags;
     }

@@ -35,6 +35,7 @@ PROTOTYPES = {
     "drl_get_episode_positions": (C.c_int, [vp, vp, vp, vp, i32, vp]),
     "drl_get_running_rsi_positions": (C.c_int, [vp, vp, vp]),
     "drl_get_median_torque": (C.c_int, [vp, vp, vp]),
+    "drl_get_ee_reward": (C.c_int, [vp, vp, vp, vp]),
     "drl_set_eval_mode": (C.c_int, [vp, i32]),
     "drl_set_det_init_counters": (C.c_int, [vp, vp]),
     "drl_set_speed_profile": (C.c_int, [vp, vp, i32]),

@@ -75,6 +75,11 @@ class WalkerModel:
     # foot-corner sites used by reset (reference: mimic_env.py:546-559)
     site_body: np.ndarray        # [nsite] int32
     site_pos: np.ndarray         # [nsite,3]
+    # end-effector points of the optional DeepMimic end-effector reward: the centre of every box geom on a leaf body
+    # that does not hang directly from the root (a leaf on the root, like walker_165cm_65kg's torso, is a trunk
+    # segment, not the end of a limb).  Both walkers: the two foot boxes.
+    ee_body: np.ndarray = None           # [n_ee] int32
+    ee_pos: np.ndarray = None            # [n_ee,3] body frame
     # compile-time constants at qpos0
     dof_invweight0: np.ndarray = None    # [nv]
     body_invweight0: np.ndarray = None   # [nb,2] translational, rotational
@@ -288,6 +293,11 @@ class _Builder:
             site_body=np.array([s["body"] for s in self.sites], np.int32),
             site_pos=np.array([s["pos"] for s in self.sites], f64).reshape(-1, 3),
         )
+        parents = {b["parent"] for b in B}
+        ee = [bx for bx in self.boxes if bx["body"] not in parents and B[bx["body"]]["parent"] >= 0
+              and B[B[bx["body"]]["parent"]]["parent"] >= 0]
+        m.ee_body = np.array([bx["body"] for bx in ee], np.int32)
+        m.ee_pos = np.array([bx["center"] for bx in ee], f64).reshape(-1, 3)
         _set_const(m)
         return m
 

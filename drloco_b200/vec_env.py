@@ -228,6 +228,8 @@ class B200MimicVecEnv:
         if self._median_torque and hist_bytes > (4 << 30):
             raise lib.DrlError(f"median_torque: the torque history would need {hist_bytes >> 20} MiB")
         c.monitor_median_torque = int(self._median_torque)
+        c.ee_weight, c.ee_scale = float(cfg.ee_weight), float(cfg.ee_scale)
+        self._ee_term = c.ee_weight > 0.0
         return c
 
     def _upload_mocap(self):
@@ -412,6 +414,16 @@ class B200MimicVecEnv:
                 out = torch.zeros(self.num_envs, device=self.device)
                 lib.check(self._lib.drl_get_median_torque(self._handle, _ptr(out), self._stream()),
                           "drl_get_median_torque")
+            vals = out.cpu().numpy()
+            return [float(vals[i]) for i in idx]
+        if attr_name in ("ee_rew", "mean_ep_ee_rew_smoothed"):   # the optional end-effector term (EnvConfig.ee_weight)
+            if not self._ee_term:
+                raise AttributeError(f"{attr_name}: the env was built with EnvConfig(ee_weight=0), the term is off")
+            with torch.cuda.device(self.device):
+                out = torch.zeros(self.num_envs, device=self.device)
+                last, smoothed = (out, None) if attr_name == "ee_rew" else (None, out)
+                lib.check(self._lib.drl_get_ee_reward(self._handle, _ptr(last), _ptr(smoothed), self._stream()),
+                          "drl_get_ee_reward")
             vals = out.cpu().numpy()
             return [float(vals[i]) for i in idx]
         if attr_name == "ep_lens":

@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define DRL_ABI_VERSION 2
+#define DRL_ABI_VERSION 3
 
 #define DRL_MAX_DOF 24
 #define DRL_MAX_BODY 12
@@ -31,6 +31,7 @@ extern "C" {
 #define DRL_MAX_SITE 16
 #define DRL_MAX_OBS 64
 #define DRL_MAX_PHASE_JOINTS 4
+#define DRL_MAX_EE 4
 
 typedef enum {
   DRL_OK = 0,
@@ -83,6 +84,12 @@ typedef struct {
   double box_mu[DRL_MAX_BOX];
   int32_t site_body[DRL_MAX_SITE];
   double site_pos[DRL_MAX_SITE][3];
+  /* end-effector points of the optional DeepMimic end-effector reward (DrlConfig.ee_weight): the centre of every box
+   * geom on a leaf body that does not hang directly from the root (both walkers: the two foot boxes), in the frame of
+   * its body.  n_ee may be 0 when the term stays off. */
+  int32_t n_ee;
+  int32_t ee_body[DRL_MAX_EE];
+  double ee_pos[DRL_MAX_EE][3];
 } DrlWalkerModel;
 
 /* Environment configuration: the fields of drloco/config/config.py + hypers.py that the step path reads. */
@@ -119,6 +126,12 @@ typedef struct {
   int32_t monitor_median_torque; /* 1 = keep every env's per-episode history of the mean |actuator torque| (4 * ep_dur_max
                                   * bytes per env) so that Monitor.median_abs_torque_smoothed (monitor_wrapper.py:131) can
                                   * be served (drl_get_median_torque); 0 = skip it */
+  /* DeepMimic end-effector term, an extension the reference does not have: with S = sum over the model's end-effector
+   * points of |p_sim - p_ref|^2 (positions relative to the root-body origin, world axes; p_ref from the reference qpos
+   * at the cursor), ee_rew = exp(-ee_scale * S) and the reward becomes
+   * (w_pos*pos + w_vel*vel + w_com*com + ee_weight*ee_rew) * rew_scale + alive_bonus.  ee_weight = 0 switches the term
+   * off (the reference's reward, no per-env buffers); ee_weight > 0 needs n_ee > 0 and ee_scale > 0 (DeepMimic: 40). */
+  double ee_weight, ee_scale;
 } DrlConfig;
 
 typedef struct DrlEnv DrlEnv;    /* opaque: persistent per-env state, mocap tables, RNG counters */
@@ -219,6 +232,12 @@ int drl_get_running_rsi_positions(DrlEnv* env, int32_t* rsi_pos, void* stream);
  * the per-step mean |actuator torque|, exponentially smoothed (0.75) at every episode end.  out: device float [N].
  * DRL_ERR_STATE when the env was created with monitor_median_torque == 0. */
 int drl_get_median_torque(DrlEnv* env, float* out, void* stream);
+
+/* the end-effector term (DrlConfig.ee_weight > 0) of every env: last = ee_rew of the latest step (not updated on a
+ * terminal step, 1 after a reset, as the pose / velocity / COM terms), smoothed = Monitor-style mean of ee_rew over all
+ * steps of the env so far, exponentially smoothed (0.9) at every episode end.  last, smoothed: device float [N], each
+ * nullable.  DRL_ERR_STATE when the env was created with ee_weight == 0. */
+int drl_get_ee_reward(DrlEnv* env, float* last, float* smoothed, void* stream);
 
 /* MimicEnv.activate_evaluation (mimic_env.py:245): deterministic init states (straight_walk_trajecs.py:237-265) */
 int drl_set_eval_mode(DrlEnv* env, int32_t on);
