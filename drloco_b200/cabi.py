@@ -9,7 +9,7 @@ import ctypes as C
 
 import numpy as np
 
-DRL_ABI_VERSION = 3
+DRL_ABI_VERSION = 4
 MAX_DOF, MAX_BODY, MAX_ACT, MAX_SPHERE, MAX_BOX, MAX_SITE, MAX_OBS, MAX_PHASE_JOINTS = 24, 12, 16, 16, 8, 16, 64, 4
 MAX_EE = 4
 INTEGRATOR_RK4, INTEGRATOR_EULER = 0, 1

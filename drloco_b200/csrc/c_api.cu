@@ -5,16 +5,12 @@
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <vector>
 
 #include "../../include/drloco_b200.h"
 #include "dev_model.h"
-#ifndef DRL_STEP_MAX_BLOCK
-#define DRL_STEP_MAX_BLOCK 128
-#endif
 
 namespace drl {
 size_t step_smem_bytes(int G, int envs_per_block);
@@ -86,9 +82,6 @@ struct DrlEnv {
   int playback = 0;
   int frame_skip_override = -1;
   float* debug = nullptr;
-  // developer hook (environment variable read at drl_create): placement of the per-evaluation CTA barrier, for A/B runs
-  // without rebuilding
-  int stage_barrier = 1;
   float* tor_hist = nullptr;
   float* med_tor_sm = nullptr;
   // end-effector term (cfg.ee_weight > 0): last / smoothed ee_rew, lifetime sum
@@ -102,11 +95,6 @@ struct DrlEnv {
   float vn_gamma = 0.f;
   double* vn_packed = nullptr;
 };
-
-static int env_int(const char* name, int dflt) {
-  const char* s = getenv(name);
-  return (s && *s) ? atoi(s) : dflt;
-}
 
 extern "C" int drl_version(void) { return DRL_ABI_VERSION; }
 extern "C" const char* drl_last_error(void) { return g_err; }
@@ -128,19 +116,30 @@ extern "C" int drl_create(const DrlConfig* cfg, DrlEnv** out) {
   if (cfg->device < 0 || cfg->device >= ndev) return fail(DRL_ERR_INVALID, "drl_create: no CUDA device %d", cfg->device);
   DrlEnv* e = new DrlEnv();
   e->cfg = *cfg;
-  e->stage_barrier = env_int("DRLOCO_B200_STAGE_BARRIER", 1);      // 0 none, 1 start of evaluation, 2 before the solver
-  if (e->stage_barrier < 0 || e->stage_barrier > 2) e->stage_barrier = 1;
   *out = e;
   return DRL_OK;
+}
+
+// the buffers of alloc_state; drl_destroy frees the rest
+static void free_state(DrlEnv* e) {
+  void** ptrs[] = {(void**)&e->d_model, (void**)&e->state_f, (void**)&e->state_i, (void**)&e->state_as,
+                   (void**)&e->state_d, (void**)&e->extras_last, (void**)&e->stats, (void**)&e->ring_len,
+                   (void**)&e->ring_ret, (void**)&e->ring_head, (void**)&e->ring_rsi_pos, (void**)&e->ring_et_pos,
+                   (void**)&e->ring_difficult, (void**)&e->cta_rows, (void**)&e->cta_ticket,
+                   (void**)&e->tor_hist, (void**)&e->med_tor_sm, (void**)&e->ee_f, (void**)&e->ee_d};
+  for (void** p : ptrs) {
+    if (*p) cudaFree(*p);
+    *p = nullptr;
+  }
 }
 
 extern "C" int drl_destroy(DrlEnv* e) {
   if (!e) return DRL_OK;
   DeviceGuard guard__(e->cfg.device);
-  void* ptrs[] = {e->d_model, e->state_f, e->state_i, e->state_as, e->state_d, e->extras_last, e->stats, e->ref, e->step_vel,
-                  e->step_last_comx, e->des_vel_prefix, e->step_off, e->step_len, e->left_step, e->ring_len,
-                  e->ring_ret, e->ring_head, e->debug, e->speed_profile, e->ring_rsi_pos, e->ring_et_pos, e->ring_difficult,
-                  e->cta_rows, e->cta_ticket, e->tor_hist, e->med_tor_sm, e->ee_f, e->ee_d};
+  free_state(e);
+  // mocap tables, speed profile, debug dump
+  void* ptrs[] = {e->ref, e->step_off, e->step_len, e->left_step, e->step_vel, e->step_last_comx, e->des_vel_prefix,
+                  e->speed_profile, e->debug};
   for (void* p : ptrs)
     if (p) cudaFree(p);
   delete e;
@@ -198,18 +197,6 @@ static int alloc_state(DrlEnv* e, size_t N) {
   for (size_t i = 0; i < N; i++) init[i * kCurCount8 + kCurCount] = 1;
   CUDA_TRY(cudaMemcpy(e->state_i, init.data(), init.size() * sizeof(int), cudaMemcpyHostToDevice));
   return DRL_OK;
-}
-
-static void free_state(DrlEnv* e) {
-  void** ptrs[] = {(void**)&e->d_model, (void**)&e->state_f, (void**)&e->state_i, (void**)&e->state_as,
-                   (void**)&e->state_d, (void**)&e->extras_last, (void**)&e->stats, (void**)&e->ring_len,
-                   (void**)&e->ring_ret, (void**)&e->ring_head, (void**)&e->ring_rsi_pos, (void**)&e->ring_et_pos,
-                   (void**)&e->ring_difficult, (void**)&e->cta_rows, (void**)&e->cta_ticket,
-                   (void**)&e->tor_hist, (void**)&e->med_tor_sm, (void**)&e->ee_f, (void**)&e->ee_d};
-  for (void** p : ptrs) {
-    if (*p) cudaFree(*p);
-    *p = nullptr;
-  }
 }
 
 extern "C" int drl_upload_model(DrlEnv* e, const DrlWalkerModel* m) {
@@ -380,18 +367,11 @@ extern "C" int drl_upload_model(DrlEnv* e, const DrlWalkerModel* m) {
   e->G = G;
   e->block = 128;
   DeviceGuard guard__(c.device);
-  {
-    const int b = env_int("DRLOCO_B200_BLOCK", 0);     // developer hook: CTA size of the step kernel
-    if (b == 32 || b == 64 || b == 96 || b == 128 || (b == 256 && DRL_STEP_MAX_BLOCK >= 256)) e->block = b;
-  }
-  const size_t N = (size_t)c.num_envs;
-  if (!e->d_model) {
-    const int rc = alloc_state(e, N);
-    if (rc != DRL_OK) {          // e.g. out of memory for a very large batch: leave the env without a model
-      free_state(e);
-      (void)cudaGetLastError();   // a failed cudaMalloc also parks its code as the "last error": clear it
-      return rc;
-    }
+  const int rc = alloc_state(e, (size_t)c.num_envs);
+  if (rc != DRL_OK) {            // e.g. out of memory for a very large batch: leave the env without a model
+    free_state(e);
+    (void)cudaGetLastError();     // a failed cudaMalloc also parks its code as the "last error": clear it
+    return rc;
   }
   e->have_model = true;
   if (e->have_mocap) CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
@@ -470,7 +450,6 @@ static StepArgs make_args(DrlEnv* e) {
   a.speed_profile = e->speed_profile_len > 0 ? e->speed_profile : nullptr;
   a.speed_profile_len = e->speed_profile_len;
   a.playback = e->playback;
-  a.stage_barrier = e->stage_barrier;
   a.cta_rows = e->cta_rows; a.cta_ticket = e->cta_ticket;
   a.tor_hist = e->tor_hist; a.med_tor_sm = e->med_tor_sm;
   a.ee_f = e->ee_f; a.ee_d = e->ee_d;

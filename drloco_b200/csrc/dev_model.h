@@ -117,7 +117,6 @@ struct StepArgs {
   const float* speed_profile;        // desired speed per control step (activate_speed_control), null when off
   int speed_profile_len;
   int playback;                      // kinematic playback: the state is set from the mocap instead of simulated
-  int stage_barrier;                 // CTA barrier before every dynamics evaluation (instruction-cache sharing)
   float* debug;                      // nullable: per-env dump of one forward evaluation (tests)
   // Monitor.median_abs_torque_smoothed (monitor_wrapper.py:131): per-episode history of the mean |torque| of every step
   float* tor_hist;                   // [N][ep_dur_max], nullable (DrlConfig.monitor_median_torque)

@@ -434,7 +434,7 @@ __device__ __forceinline__ void mass_column(const DevModel& M, EnvSmem<G>& E, co
 template <int NV, int G, bool DBG>
 __device__ __forceinline__ void forward_dynamics(const DevModel& M, EnvSmem<G>& E, const LaneConst& L,
                                                   const ChainLane& C, float q, float v, float tau, float& a,
-                                                  ActiveSet& AS, Vec6& S, float* dbg, bool solver_barrier) {
+                                                  ActiveSet& AS, Vec6& S, float* dbg) {
   using T = Topo<NV>;
   using ES = EnvSmem<G>;
   const int l = L.l;
@@ -618,10 +618,6 @@ __device__ __forceinline__ void forward_dynamics(const DevModel& M, EnvSmem<G>& 
     if (body_subtree_mask<NV>(b) & conmask) subcon |= 1u << b;
   int n_iter = 0;
   bool capped = false;
-  // Optional CTA barrier here instead of at the start of the evaluation (StepArgs::stage_barrier == 2): warps whose
-  // previous evaluation converged in one solver pass run ahead through the kinematics / bias-force half of this one
-  // while the others finish their extra pass, and the block lines up again for the solver (shared instruction stream).
-  if (solver_barrier) __syncthreads();
   float H[NV + 1];
   for (int it = 0; it < kMaxSolverIter; it++) {
     if (constrained) n_iter++;

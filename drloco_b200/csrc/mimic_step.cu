@@ -351,13 +351,8 @@ __device__ __noinline__ void reset_env(const DevModel& M, const StepArgs& A, ES&
   __syncwarp();
 }
 
-// developer build switch (-DDRL_STEP_MAX_BLOCK=256): largest CTA the step kernel may be launched with; the shipped
-// library is built for 128-thread CTAs, four per SM
-#ifndef DRL_STEP_MAX_BLOCK
-#define DRL_STEP_MAX_BLOCK 128
-#endif
 template <int NV, int G, bool RK4, bool DBG>
-__global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) mimic_step_kernel(const StepArgs A, const int do_reset_only) {
+__global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, const int do_reset_only) {
   using ES = EnvSmem<G>;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   DevModel& M = *reinterpret_cast<DevModel*>(smem_raw);
@@ -477,10 +472,11 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
       for (int st = 0; st < 4; st++) {
         // keep the warps of a CTA within one evaluation of each other: they then share instruction-cache lines
         // (the dynamics evaluation is ~80 KB of straight-line code); measured +3 %
-        // (one barrier per substep instead of per stage loses the gain; a second barrier inside the evaluation adds none)
-        if (A.stage_barrier == 1) __syncthreads();
+        // (one barrier per substep instead of per stage loses the gain; a second barrier inside the evaluation adds none;
+        // no barrier or one before the solver is slower at 64, 96 and 128 threads per CTA: profiles/r02_kernel_ab.md)
+        __syncthreads();
         Vec6 Sj;
-        forward_dynamics<NV, G, DBG>(M, E, L, CL, q, v, tau, a, AS, Sj, dbgp, A.stage_barrier == 2);
+        forward_dynamics<NV, G, DBG>(M, E, L, CL, q, v, tau, a, AS, Sj, dbgp);
         const float bw = (st == 0 || st == 3) ? (1.f / 6.f) : (1.f / 3.f);
         accq = fmaf(bw, v, accq);
         accv = fmaf(bw, a, accv);
@@ -498,7 +494,7 @@ __global__ void __launch_bounds__(DRL_STEP_MAX_BLOCK, 512 / DRL_STEP_MAX_BLOCK) 
       float Hc[NV + 1];
       float Ma = 0.f;
       Vec6 Sj;
-      forward_dynamics<NV, G, DBG>(M, E, L, CL, q, v, tau, a, AS, Sj, dbgp, false);
+      forward_dynamics<NV, G, DBG>(M, E, L, CL, q, v, tau, a, AS, Sj, dbgp);
       pure_mass_column<NV, G>(M, E, L, Sj, Hc);     // E.acc holds the constrained qacc of every dof
 #pragma unroll
       for (int r = 0; r < NV; r++) {

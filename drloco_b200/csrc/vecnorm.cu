@@ -1,9 +1,10 @@
 // vecnorm.cu — VecNormalize on the device (SB3 1.0 VecNormalize as built at reference drloco/common/utils.py:130-132).
 //
-// Two kernels per step, with the (optional) NCCL all-reduce of the packed moments between them:
-//   moments: ret = ret*gamma + rew;  packed = [ sum_obs[D], sumsq_obs[D], n, sum_ret, sumsq_ret ]   (float64 sums)
-//   apply  : Chan merge of the batch moments into the running statistics (identical on every rank after the
-//            all-reduce), obs <- clip((obs-mean)/sqrt(var+eps)), rew <- clip(rew/sqrt(ret_var+eps)), ret[done] = 0
+//   moments : ret = ret*gamma + rew;  packed = [ sum_obs[D], sumsq_obs[D], n, sum_ret, sumsq_ret ]   (float64 sums)
+//             (the step kernel computes the same moments itself when drl_attach_vecnorm is on)
+//   step    : exchange of the packed moments between ranks, Chan merge into the running statistics,
+//             obs <- clip((obs-mean)/sqrt(var+eps)), rew <- clip(rew/sqrt(ret_var+eps)), ret[done] = 0
+//   terminal: the observations of finished environments, normalised and compacted
 // Running statistics layout (float64): rms = [ mean[D], var[D], count, ret_mean, ret_var, ret_count ].
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -75,55 +76,7 @@ __device__ __forceinline__ void chan_merge(double mean, double var, double count
   ncount = tot;
 }
 
-__global__ void vecnorm_apply_kernel(const float* __restrict__ obs_in, float* __restrict__ obs_out,
-                                     const float* __restrict__ rew_in, float* __restrict__ rew_out, int n, int d,
-                                     const double* __restrict__ packed, const double* __restrict__ rms_in,
-                                     double* __restrict__ rms_out, float* __restrict__ ret,
-                                     const unsigned char* __restrict__ done, float clip_obs, float clip_rew, float eps,
-                                     int training, int norm_obs, int norm_rew) {
-  extern __shared__ float shf[];     // mean[d], inv_std[d], ret_inv_std
-  float* s_mean = shf;
-  float* s_inv = shf + d;
-  for (int k = threadIdx.x; k <= d; k += blockDim.x) {
-    double mean, var, count;
-    if (k < d) { mean = rms_in[k]; var = rms_in[d + k]; count = rms_in[2 * d]; }
-    else { mean = rms_in[2 * d + 1]; var = rms_in[2 * d + 2]; count = rms_in[2 * d + 3]; }
-    const double bn = packed ? packed[2 * d] : 0.0;
-    if (training && bn > 0.0) {
-      const double bs = k < d ? packed[k] : packed[2 * d + 1];
-      const double bss = k < d ? packed[d + k] : packed[2 * d + 2];
-      if (k < d || rew_in != nullptr) chan_merge(mean, var, count, bs, bss, bn, mean, var, count);
-    }
-    if (blockIdx.x == 0) {
-      if (k < d) { rms_out[k] = mean; rms_out[d + k] = var; if (k == 0) rms_out[2 * d] = count; }
-      else { rms_out[2 * d + 1] = mean; rms_out[2 * d + 2] = var; rms_out[2 * d + 3] = count; }
-    }
-    if (k < d) { s_mean[k] = (float)mean; s_inv[k] = (float)(1.0 / sqrt(var + (double)eps)); }
-    else s_inv[d] = (float)(1.0 / sqrt(var + (double)eps));
-  }
-  __syncthreads();
-  const long long total = (long long)n * d;
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += stride) {
-    const int col = (int)(e % d);
-    float x = obs_in[e];
-    if (norm_obs) x = fminf(fmaxf((x - s_mean[col]) * s_inv[col], -clip_obs), clip_obs);
-    obs_out[e] = x;
-  }
-  if (rew_in != nullptr) {
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-      float r = rew_in[i];
-      if (norm_rew) r = fminf(fmaxf(r * s_inv[d], -clip_rew), clip_rew);
-      rew_out[i] = r;
-      if (done != nullptr && done[i]) ret[i] = 0.f;
-    }
-  }
-}
-
 }  // namespace drl
-
-static thread_local char g_verr[256] = "";
-extern "C" const char* drl_vecnorm_last_error(void) { return g_verr; }
 
 // obs [n][d] device, rew [n] device (nullable: reset-time update of the observation statistics only), ret [n] device
 // in/out, packed device float64 [2d+3] (zeroed here, then filled).
@@ -141,25 +94,8 @@ extern "C" int drl_vecnorm_moments(const float* obs, int32_t n, int32_t d, const
   return cudaGetLastError() == cudaSuccess ? DRL_OK : DRL_ERR_CUDA;
 }
 
-// rms_in / rms_out device float64 [2d+4] (may not alias); obs_in/obs_out may alias; rew_in/rew_out may alias.
-extern "C" int drl_vecnorm_apply(const float* obs_in, float* obs_out, const float* rew_in, float* rew_out, int32_t n,
-                                 int32_t d, const double* packed, const double* rms_in, double* rms_out, float* ret,
-                                 const uint8_t* done, float clip_obs, float clip_rew, float eps, int32_t flags,
-                                 void* stream) {
-  if (!obs_in || !obs_out || !rms_in || !rms_out || n <= 0 || d <= 0 || rms_in == rms_out) return DRL_ERR_INVALID;
-  cudaStream_t st = (cudaStream_t)stream;
-  long long work = (long long)n * d;
-  int blocks = (int)((work + drl::kVnThreads * 4 - 1) / (drl::kVnThreads * 4));
-  if (blocks < 1) blocks = 1;
-  if (blocks > 148 * 8) blocks = 148 * 8;
-  drl::vecnorm_apply_kernel<<<blocks, drl::kVnThreads, (2 * d + 1) * sizeof(float), st>>>(
-      obs_in, obs_out, rew_in, rew_out, n, d, packed, rms_in, rms_out, ret, done, clip_obs, clip_rew, eps, flags & 1,
-      (flags >> 1) & 1, (flags >> 2) & 1);
-  return cudaGetLastError() == cudaSuccess ? DRL_OK : DRL_ERR_CUDA;
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
-// Fused statistics exchange + normalisation: ONE kernel per step replaces moments -> all-reduce -> apply.
+// Statistics exchange + merge + normalisation: ONE kernel per step.
 //
 // The batch moments of the step arrive in `packed` (written by the step kernel's own epilogue, drl_attach_vecnorm).
 // With more than one rank (one process per GPU of a node) every rank owns a small mailbox in its HBM that its peers map
@@ -411,42 +347,14 @@ extern "C" int drl_vecnorm_step(const float* obs_in, float* obs_out, const float
   return cudaGetLastError() == cudaSuccess ? DRL_OK : DRL_ERR_CUDA;
 }
 
-// terminal observations of the environments that finished this step, normalised with the current statistics
-// (what VecNormalize hands to SB3 in infos[i]["terminal_observation"]); rows of running environments are skipped
-namespace drl {
-__global__ void vecnorm_terminal_kernel(const float* __restrict__ tin, float* __restrict__ tout,
-                                        const unsigned char* __restrict__ done, int n, int d,
-                                        const double* __restrict__ rms, float clip_obs, float eps, int norm_obs) {
-  const long long total = (long long)n * d;
-  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total;
-       e += (long long)gridDim.x * blockDim.x) {
-    const int row = (int)(e / d), col = (int)(e % d);
-    if (!done[row]) continue;
-    float x = tin[e];
-    if (norm_obs)
-      x = fminf(fmaxf((x - (float)rms[col]) * (float)(1.0 / sqrt(rms[d + col] + (double)eps)), -clip_obs), clip_obs);
-    tout[e] = x;
-  }
-}
-}  // namespace drl
-
-extern "C" int drl_vecnorm_terminal(const float* tobs_in, float* tobs_out, const uint8_t* done, int32_t n, int32_t d,
-                                    const double* rms, float clip_obs, float eps, int32_t norm_obs, void* stream) {
-  if (!tobs_in || !tobs_out || !done || !rms || n <= 0 || d <= 0) return DRL_ERR_INVALID;
-  long long work = (long long)n * d;
-  int blocks = (int)((work + drl::kVnThreads * 4 - 1) / (drl::kVnThreads * 4));
-  if (blocks > 148 * 8) blocks = 148 * 8;
-  drl::vecnorm_terminal_kernel<<<blocks, drl::kVnThreads, 0, (cudaStream_t)stream>>>(tobs_in, tobs_out, done, n, d, rms,
-                                                                                    clip_obs, eps, norm_obs);
-  return cudaGetLastError() == cudaSuccess ? DRL_OK : DRL_ERR_CUDA;
-}
-
-// The same, compacted: only the rows of finished environments leave the device.  out = 4 header words (out[0] = number of
-// finished environments) followed by one record per finished environment, record = { env index (int32 bits), d floats }.
-// Record order is arbitrary (one atomic slot per finished row); the host maps rows back through the index.  `out` may
-// be device memory or pinned host memory mapped into the device's address space (the records are then written across
-// PCIe by the kernel itself: no copy node).  counters: device int32 [2] = { slot counter, block ticket }, zero before the
-// first launch; the last block to finish publishes the count in the header and zeroes both again.
+// Terminal observations of the environments that finished this step, normalised with the current statistics (what
+// VecNormalize hands to SB3 in infos[i]["terminal_observation"]), compacted: only the rows of finished environments
+// leave the device.  out = 4 header words (out[0] = number of finished environments) followed by one record per
+// finished environment, record = { env index (int32 bits), d floats }.  Record order is arbitrary (one atomic slot per
+// finished row); the host maps rows back through the index.  `out` may be device memory or pinned host memory mapped
+// into the device's address space (the records are then written across PCIe by the kernel itself: no copy node).
+// counters: device int32 [2] = { slot counter, block ticket }, zero before the first launch; the last block to finish
+// publishes the count in the header and zeroes both again.
 namespace drl {
 __global__ void vecnorm_terminal_compact_kernel(const float* __restrict__ tin, const unsigned char* __restrict__ done,
                                                 int n, int d, const double* __restrict__ rms, float clip_obs, float eps,

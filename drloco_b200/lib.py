@@ -50,11 +50,9 @@ PROTOTYPES = {
     "drl_comm_connect": (C.c_int, [vp, vp]),
     "drl_comm_destroy": (C.c_int, [vp]),
     "drl_vecnorm_step": (C.c_int, [vp, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, f32, f32, f32, i32, vp, i32, vp]),
-    "drl_vecnorm_terminal": (C.c_int, [vp, vp, vp, i32, i32, vp, f32, f32, i32, vp]),
     "drl_vecnorm_terminal_compact": (C.c_int, [vp, vp, i32, i32, vp, f32, f32, i32, vp, vp, vp]),
     "drl_fp32_peak_probe": (C.c_int, [i32, C.POINTER(C.c_double)]),
     "drl_vecnorm_moments": (C.c_int, [vp, i32, i32, vp, vp, f32, vp, vp]),
-    "drl_vecnorm_apply": (C.c_int, [vp, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, f32, f32, f32, i32, vp]),
 }
 
 

@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define DRL_ABI_VERSION 3
+#define DRL_ABI_VERSION 4
 
 #define DRL_MAX_DOF 24
 #define DRL_MAX_BODY 12
@@ -271,17 +271,12 @@ int drl_debug_set(DrlEnv* env, int32_t frame_skip_override, int32_t block_thread
 int drl_debug_read(DrlEnv* env, float* host_out, int32_t n_floats);
 
 /* VecNormalize on the device — replaces SB3 VecNormalize.step_wait / reset around the env (utils.py:130-132).
- * moments: ret = ret*gamma + rew (in place; skipped when rew == NULL) and
- *          packed[2d+3] = { sum_obs[d], sumsq_obs[d], n, sum_ret, sumsq_ret } in float64 — the all-reduce(sum) payload.
- * apply  : merges `packed` into the running statistics rms = { mean[d], var[d], count, ret_mean, ret_var, ret_count }
- *          (RunningMeanStd.update_from_moments; rms_in -> rms_out, must not alias), then writes
- *          obs_out = clip((obs_in-mean)/sqrt(var+eps), +-clip_obs), rew_out = clip(rew_in/sqrt(ret_var+eps), +-clip_rew),
- *          ret[done] = 0.  flags: bit0 training (update statistics), bit1 norm_obs, bit2 norm_reward. */
+ * drl_vecnorm_moments: the batch moments of obs [n][d] (device), for the statistics update of observations the step
+ *   kernel did not produce (the reset observations).  ret = ret*gamma + rew (in place; skipped when rew == NULL) and
+ *   packed[2d+3] = { sum_obs[d], sumsq_obs[d], n, sum_ret, sumsq_ret } in float64 (device; zeroed, then filled) — the
+ *   all-reduce(sum) payload that drl_vecnorm_step merges into the running statistics. */
 int drl_vecnorm_moments(const float* obs, int32_t n, int32_t d, const float* rew, float* ret, float gamma,
                         double* packed, void* stream);
-int drl_vecnorm_apply(const float* obs_in, float* obs_out, const float* rew_in, float* rew_out, int32_t n, int32_t d,
-                      const double* packed, const double* rms_in, double* rms_out, float* ret, const uint8_t* done,
-                      float clip_obs, float clip_rew, float eps, int32_t flags, void* stream);
 
 /* Fused VecNormalize path (what B200VecNormalize uses): ONE kernel per step after drl_step.
  *
@@ -295,7 +290,9 @@ int drl_vecnorm_apply(const float* obs_in, float* obs_out, const float* rew_in, 
  *   handles of all ranks by any means (torch.distributed.all_gather) and maps its peers' mailboxes (drl_comm_connect,
  *   handles = world x 64 bytes in rank order).  world == 1 needs no export / connect.
  * drl_vecnorm_step: exchange (peer stores into the mailboxes over NVLink + flags, summed in rank order: identical bits
- *   on every rank) + Chan merge into rms (rms_in -> rms_out, must not alias) + normalisation of obs / rew +
+ *   on every rank) + Chan merge into the running statistics rms = { mean[d], var[d], count, ret_mean, ret_var,
+ *   ret_count } in float64 (RunningMeanStd.update_from_moments; rms_in -> rms_out, must not alias) + normalisation
+ *   obs_out = clip((obs_in-mean)/sqrt(var+eps), +-clip_obs), rew_out = clip(rew_in/sqrt(ret_var+eps), +-clip_rew) +
  *   ret[done] = 0.  flags: bit0 update the observation statistics, bit1 norm_obs, bit2 norm_reward, bit3 update the
  *   return statistics.  packed == NULL or no update bit: normalise only.  done_out (nullable): a copy of `done`
  *   next to the normalised outputs, so that one device-to-host copy can fetch a whole step.  sync_every = K >= 1: a "cycle" call - the
@@ -314,13 +311,10 @@ int drl_vecnorm_step(const float* obs_in, float* obs_out, const float* rew_in, f
                      uint8_t* done_out, float clip_obs, float clip_rew, float eps, int32_t flags, DrlComm* comm,
                      int32_t sync_every, void* stream);
 
-/* rows of tobs_in whose done byte is set, normalised with rms ({mean[d], var[d], ...}) into tobs_out: the
- * infos[i]["terminal_observation"] VecNormalize returns (SB3 VecNormalize.step_wait). Other rows are left untouched. */
-int drl_vecnorm_terminal(const float* tobs_in, float* tobs_out, const uint8_t* done, int32_t n, int32_t d,
-                         const double* rms, float clip_obs, float eps, int32_t norm_obs, void* stream);
-
-/* the same, compacted so that only finished environments cross PCIe: out_words (4 + n*(d+1) 32-bit words) = header
- * { count, -, -, - } + one record { env index (int32), d floats } per finished environment, in arbitrary order.
+/* rows of tobs_in whose done byte is set, normalised with rms ({mean[d], var[d], ...}): the
+ * infos[i]["terminal_observation"] VecNormalize returns (SB3 VecNormalize.step_wait), compacted so that only finished
+ * environments cross PCIe: out_words (4 + n*(d+1) 32-bit words) = header { count, -, -, - } + one record
+ * { env index (int32), d floats } per finished environment, in arbitrary order.
  * out_words may be device memory or pinned host memory (mapped into the device's address space: the kernel then writes
  * the records across PCIe itself).  The same holds for obs_out / rew_out / done_out of drl_vecnorm_step.
  * counters: device int32 [2], zero before the first call, left zero by every call (slot counter, block ticket).

@@ -198,7 +198,7 @@ def test_defaults_leave_the_term_off():
 # --------------------------------------------------------------------------------------------------------------------
 # CPU: C ABI layout and argument checks that run before any device is touched
 # --------------------------------------------------------------------------------------------------------------------
-def test_abi_fields_are_appended(tmp_path):
+def test_abi_v4_keeps_the_ee_fields_appended(tmp_path):
     import subprocess
     probe = tmp_path / "probe.c"
     probe.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "drloco_b200.h"\n'
@@ -212,7 +212,7 @@ def test_abi_fields_are_appended(tmp_path):
     W, Cf = cabi.DrlWalkerModel, cabi.DrlConfig
     assert got == [cabi.DRL_ABI_VERSION, cabi.MAX_EE, W.n_ee.offset, W.ee_body.offset, W.ee_pos.offset,
                    Cf.ee_weight.offset, Cf.ee_scale.offset]
-    assert cabi.DRL_ABI_VERSION == 3
+    assert cabi.DRL_ABI_VERSION == 4
     # appended: every field of the previous layout keeps its offset
     assert W.n_ee.offset > W.site_pos.offset and Cf.ee_weight.offset > Cf.monitor_median_torque.offset
 
