@@ -15,6 +15,7 @@ MAX_EE = 4
 INTEGRATOR_RK4, INTEGRATOR_EULER = 0, 1
 CURSOR_STEPWISE, CURSOR_WRAP = 0, 1
 PHASE_FROM_CURSOR, PHASE_FROM_JOINTS = 0, 1
+ACTUATION_TORQUE, ACTUATION_PD = 0, 1
 EXTRA_NAMES = ("pos_rew", "vel_rew", "com_rew", "walked_distance", "mean_abs_torque", "des_vel", "phase", "z_offset",
                "ep_len_smoothed", "ep_ret_smoothed", "mean_reward_smoothed", "mean_ep_pos_rew_smoothed",
                "mean_ep_vel_rew_smoothed", "mean_ep_com_rew_smoothed", "moved_distance", "mean_abs_ep_torque_smoothed")

@@ -7,7 +7,10 @@ process (tests, benchmarks), with the reference's values as defaults.
 from __future__ import annotations
 
 import dataclasses
-from typing import Tuple
+import math
+from typing import Optional, Tuple, Union
+
+import numpy as np
 
 # environment ids (reference drloco/mujoco/config.py:5-6)
 STRAIGHT_WALKER = "StraightMimicWalker"
@@ -45,6 +48,13 @@ class EnvConfig:
                                                         # the imitation reward with this weight; 0 = off, as in the
                                                         # reference (see README "End-effector reward")
     ee_scale: float = 40.0                              # ee_rew = exp(-ee_scale * sum of squared foot-position errors)
+    actuation: str = "torque"                           # "torque": the action is the motor force (the reference);
+                                                        # "pd": every motor is a position servo, MuJoCo <position kp kv>,
+                                                        # and the action picks its target in the joint's range (see
+                                                        # README "PD actuation")
+    pd_kp: Union[None, float, Tuple[float, ...]] = None   # servo stiffness, > 0: one value for every actuator or one
+                                                        # per actuator in actuator order; required with "pd"
+    pd_kv: Union[None, float, Tuple[float, ...]] = None   # servo damping, >= 0, as pd_kp; None = 0 (MuJoCo's default)
     gamma: float = 0.0                                  # 0 -> by ctrl_freq, hypers.py:68
     integrator: str = "rk4"                             # xml:11; "euler" = MuJoCo semi-implicit Euler (fast mode)
     seed: int = 33                                      # utils.py:97
@@ -57,6 +67,35 @@ class EnvConfig:
         if self.env_id == WALKER_165 and self.is_mod(MOD_MIRR_POLICY):
             # mirroring is only defined for the straight walker (hypers.py:31-39; loco3d refs have no is_step_left)
             self.modifications = tuple(m for m in self.modifications if m != MOD_MIRR_POLICY)
+        if self.actuation not in ("torque", "pd"):
+            raise ValueError(f"actuation must be 'torque' or 'pd', got {self.actuation!r}")
+        if self.actuation == "torque":
+            if self.pd_kp is not None or self.pd_kv is not None:
+                raise ValueError("pd_kp / pd_kv are the gains of actuation='pd'; the torque mode has none")
+        else:
+            if self.pd_kp is None:
+                raise ValueError("actuation='pd' needs pd_kp (there are no default gains)")
+            self.pd_gains()
+
+    def pd_gains(self, nu: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """(kp, kv) of actuation='pd' as float64 arrays in actuator order, scalars broadcast to the walker's nu
+        actuators; raises ValueError for a wrong length or a gain out of range (kp finite and > 0, kv finite and >= 0)."""
+        if nu is None:
+            from .model import get_model
+            nu = get_model(self.env_id).nu
+
+        def per_actuator(x, name):
+            a = np.full(nu, float(x)) if np.ndim(x) == 0 else np.array([float(g) for g in x], np.float64)
+            if a.shape != (nu,):
+                raise ValueError(f"{name}: {a.size} gains for {nu} actuators")
+            return a
+        kp = per_actuator(self.pd_kp, "pd_kp")
+        kv = per_actuator(0.0 if self.pd_kv is None else self.pd_kv, "pd_kv")
+        if not all(math.isfinite(g) and g > 0.0 for g in kp):
+            raise ValueError(f"pd_kp must be finite and > 0, got {self.pd_kp}")
+        if not all(math.isfinite(g) and g >= 0.0 for g in kv):
+            raise ValueError(f"pd_kv must be finite and >= 0, got {self.pd_kv}")
+        return kp, kv
 
     def is_mod(self, mod_str: str) -> bool:
         """reference hypers.py:26-29 (substring test on the joined modification string)."""

@@ -13,8 +13,8 @@
 #include "dev_model.h"
 
 namespace drl {
-size_t step_smem_bytes(int G, int envs_per_block);
-cudaError_t launch_step(const StepArgs& a, int nv, int G, int rk4, int reset_only, int block, bool debug,
+size_t step_smem_bytes(int G, int envs_per_block, bool pd);
+cudaError_t launch_step(const StepArgs& a, int nv, int G, int rk4, int reset_only, int block, bool debug, bool pd,
                         cudaStream_t st);
 cudaError_t launch_running_rsi(const int* state_i, int* out, int n, cudaStream_t st);
 bool topology_matches(int nv, int nb, const int* body_parent, const int* dof_body, const int* dof_type);
@@ -59,6 +59,8 @@ struct DrlEnv {
   DevModel hm;                 // host copy
   bool have_model = false, have_mocap = false;
   int G = 16, block = 128, nv = 0;
+  int actuation = DRL_ACTUATION_TORQUE;   // drl_set_actuation
+  double dof_range[kMaxDof][2];           // joint ranges in float64: the PD target map is computed from them
   DevModel* d_model = nullptr;
   float* state_f = nullptr;
   int* state_i = nullptr;
@@ -251,6 +253,7 @@ extern "C" int drl_upload_model(DrlEnv* e, const DrlWalkerModel* m) {
     d.dof_sign[j] = (float)m->dof_axis_sign[j]; d.dof_ref[j] = (float)m->dof_ref[j];
     d.dof_damping[j] = (float)m->dof_damping[j]; d.dof_armature[j] = (float)m->dof_armature[j];
     d.dof_lo[j] = (float)m->dof_range[j][0]; d.dof_hi[j] = (float)m->dof_range[j][1];
+    e->dof_range[j][0] = m->dof_range[j][0]; e->dof_range[j][1] = m->dof_range[j][1];
     d.dof_invw[j] = (float)m->dof_invweight0[j];
     if (m->dof_type[j] == 0) {
       if (b != 0 || seen_hinge_root) return fail(DRL_ERR_UNSUPPORTED, "model: slides are supported on the root body, before its hinges");
@@ -468,7 +471,8 @@ extern "C" int drl_reset(DrlEnv* e, const uint8_t* mask, const int32_t* inj_iste
   StepArgs a = make_args(e);
   a.reset_mask = mask; a.inj_istep = inj_istep; a.inj_pos = inj_pos; a.obs = obs;
   a.debug = nullptr;
-  CUDA_TRY(launch_step(a, e->nv, e->G, e->cfg.integrator == DRL_INTEGRATOR_RK4, 1, e->block, false, (cudaStream_t)stream));
+  CUDA_TRY(launch_step(a, e->nv, e->G, e->cfg.integrator == DRL_INTEGRATOR_RK4, 1, e->block, false, false,
+                       (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -481,9 +485,10 @@ extern "C" int drl_step(DrlEnv* e, const float* actions, float* obs, float* rew,
   StepArgs a = make_args(e);
   a.actions = actions; a.obs = obs; a.rew = rew; a.done = done; a.terminal_obs = terminal_obs;
   a.inj_istep = inj_istep; a.inj_pos = inj_pos;
-    const bool rk4 = e->cfg.integrator == DRL_INTEGRATOR_RK4;
+  const bool rk4 = e->cfg.integrator == DRL_INTEGRATOR_RK4, pd = e->actuation == DRL_ACTUATION_PD;
   if (e->debug && rk4) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for the Euler integrator only");
-  CUDA_TRY(launch_step(a, e->nv, e->G, rk4, 0, e->block, e->debug != nullptr, (cudaStream_t)stream));
+  if (e->debug && pd) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for torque actuation only");
+  CUDA_TRY(launch_step(a, e->nv, e->G, rk4, 0, e->block, e->debug != nullptr, pd, (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -639,6 +644,45 @@ extern "C" int drl_set_seed(DrlEnv* e, uint64_t seed) {
   return DRL_OK;
 }
 
+extern "C" int drl_set_actuation(DrlEnv* e, int32_t mode, const double* kp, const double* kv) {
+  if (!e) return fail(DRL_ERR_INVALID, "drl_set_actuation: null env");
+  if (mode != DRL_ACTUATION_TORQUE && mode != DRL_ACTUATION_PD)
+    return fail(DRL_ERR_INVALID, "drl_set_actuation: unknown mode %d", mode);
+  if (!e->have_model) return fail(DRL_ERR_STATE, "drl_set_actuation: upload the model first");
+  DevModel& d = e->hm;
+  if (mode == DRL_ACTUATION_PD) {
+    if (!kp || !kv) return fail(DRL_ERR_INVALID, "drl_set_actuation: PD needs kp and kv");
+    for (int u = 0; u < d.nu; u++) {
+      if (!(isfinite(kp[u]) && kp[u] > 0.0))
+        return fail(DRL_ERR_INVALID, "drl_set_actuation: kp[%d] = %g must be finite and > 0", u, kp[u]);
+      if (!(isfinite(kv[u]) && kv[u] >= 0.0))
+        return fail(DRL_ERR_INVALID, "drl_set_actuation: kv[%d] = %g must be finite and >= 0", u, kv[u]);
+      const int j = d.act_dof[u];
+      if (!d.dof_limited[j] || !(e->dof_range[j][1] > e->dof_range[j][0]))
+        return fail(DRL_ERR_INVALID, "drl_set_actuation: actuator %d drives dof %d, which has no joint range", u, j);
+    }
+  }
+  // the gains and the target map are rewritten in full: switching back to torque leaves the block as after the upload
+  memset(d.pd_kp, 0, sizeof d.pd_kp); memset(d.pd_kv, 0, sizeof d.pd_kv); memset(d.pd_gear, 0, sizeof d.pd_gear);
+  memset(d.pd_flo, 0, sizeof d.pd_flo); memset(d.pd_fhi, 0, sizeof d.pd_fhi);
+  memset(d.pd_mid, 0, sizeof d.pd_mid); memset(d.pd_half, 0, sizeof d.pd_half);
+  if (mode == DRL_ACTUATION_PD) {
+    for (int u = 0; u < d.nu; u++) {
+      const int j = d.act_dof[u];
+      d.pd_kp[j] = (float)kp[u]; d.pd_kv[j] = (float)kv[u]; d.pd_gear[j] = d.act_gear[u];
+      d.pd_flo[j] = d.act_flo[u]; d.pd_fhi[j] = d.act_fhi[u];
+      const double lo = e->dof_range[j][0], hi = e->dof_range[j][1];
+      d.pd_mid[u] = (float)(0.5 * (lo + hi));
+      d.pd_half[u] = (float)(0.5 * (hi - lo));
+    }
+  }
+  e->actuation = mode;
+  DeviceGuard guard__(e->cfg.device);
+  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the model block
+  CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
+  return DRL_OK;
+}
+
 extern "C" int drl_set_playback(DrlEnv* e, int32_t on) {
   if (!e) return fail(DRL_ERR_INVALID, "drl_set_playback: null env");
   e->playback = on ? 1 : 0;
@@ -669,7 +713,7 @@ extern "C" int drl_launch_info(DrlEnv* e, int32_t* lanes_per_env, int32_t* block
   if (lanes_per_env) *lanes_per_env = e->G;
   if (block_threads) *block_threads = e->block;
   if (grid_blocks) *grid_blocks = (e->cfg.num_envs + epb - 1) / epb;
-  if (smem_bytes) *smem_bytes = (int)step_smem_bytes(e->G, epb);
+  if (smem_bytes) *smem_bytes = (int)step_smem_bytes(e->G, epb, e->actuation == DRL_ACTUATION_PD);
   return DRL_OK;
 }
 

@@ -3,6 +3,7 @@
 // Built on the host from DrlWalkerModel / DrlConfig (include/drloco_b200.h) in drl_upload_model(), stored once in
 // global memory and staged into shared memory by every thread block of the step kernel.
 #pragma once
+#include <stddef.h>
 #include <stdint.h>
 
 namespace drl {
@@ -64,9 +65,19 @@ struct alignas(16) DevModel {
   int n_ee, ee_body[kMaxEE];
   float ee_pos[kMaxEE][3];           // point in the body frame
   float w_ee, ee_scale;
+  // ---- PD position servos (drl_set_actuation; read by the PD instances of the step kernel only, which alone stage
+  // this tail of the block into shared memory: kModelBytesTorque) ----
+  // per dof, zero on dofs without an actuator: f = clamp(kp (ctrl - gear q) - kv gear v, flo, fhi), tau = gear f
+  alignas(16) float pd_kp[kMaxDof];
+  float pd_kv[kMaxDof], pd_gear[kMaxDof], pd_flo[kMaxDof], pd_fhi[kMaxDof];
+  // per actuator: action a in [-1, 1] -> target ctrl = mid + a * half over the range of the joint it drives
+  float pd_mid[kMaxAct], pd_half[kMaxAct];
 };
 
 static_assert(sizeof(DevModel) % 16 == 0, "DevModel is copied in int4 chunks");
+// bytes of DevModel a torque-actuated step kernel stages and reserves (everything before the PD tables)
+constexpr size_t kModelBytesTorque = offsetof(DevModel, pd_kp);
+static_assert(kModelBytesTorque % 16 == 0, "the PD tables start on an int4 boundary");
 
 // per-env persistent state rows (see DESIGN.md "data layout in HBM")
 constexpr int kMiscDist = 0, kMiscZoff = 1, kMiscWalked = 2, kMiscEpRet = 3, kMiscEpTor = 4, kMiscPrevPos = 5,

@@ -351,17 +351,27 @@ __device__ __noinline__ void reset_env(const DevModel& M, const StepArgs& A, ES&
   __syncwarp();
 }
 
-template <int NV, int G, bool RK4, bool DBG>
+// PD position servo of dof lane jd (MuJoCo <position kp kv>, actuator length gear*q, velocity gear*v): the actuator
+// force f for the target ctrl at the state (q, v).  Zero on dofs without an actuator (their gains, gear and force
+// range are zero in DevModel).
+__device__ __forceinline__ float pd_force(const DevModel& M, int jd, float ctrl, float q, float v) {
+  const float g = M.pd_gear[jd];
+  return fminf(fmaxf(M.pd_kp[jd] * (ctrl - g * q) - M.pd_kv[jd] * (g * v), M.pd_flo[jd]), M.pd_fhi[jd]);
+}
+
+// PD: the instance drives every motor as a position servo whose force is recomputed from the state of every dynamics
+// evaluation (drl_set_actuation); false: the force is the clipped action, held for the whole control step.
+template <int NV, int G, bool RK4, bool DBG, bool PD>
 __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, const int do_reset_only) {
   using ES = EnvSmem<G>;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   DevModel& M = *reinterpret_cast<DevModel*>(smem_raw);
-  constexpr int kModelBytes = (sizeof(DevModel) + 15) / 16 * 16;
+  constexpr int kModelBytes = PD ? sizeof(DevModel) : kModelBytesTorque;   // torque: the PD tables stay in HBM
   ES* envs = reinterpret_cast<ES*>(smem_raw + kModelBytes);
   {
     const int4* src = reinterpret_cast<const int4*>(A.model);
     int4* dst = reinterpret_cast<int4*>(smem_raw);
-    for (int i = threadIdx.x; i < (int)(sizeof(DevModel) / 16); i += blockDim.x) dst[i] = src[i];
+    for (int i = threadIdx.x; i < kModelBytes / 16; i += blockDim.x) dst[i] = src[i];
   }
   __syncthreads();
   const int epb = blockDim.x / G;
@@ -428,6 +438,8 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
   }
 
   // ---- actions -> joint torques (mimic_env.py:170-192, :483-489; MuJoCo ctrl/force clamps) ---------------------
+  // PD: actions -> servo targets over the joint ranges, then the same mirror; the target is clamped to the range of
+  // the joint (the servo's ctrlrange)
   const bool left0 = M.mirror_policy && A.left_step[c.i_step];
   float force = 0.f;
   {
@@ -435,7 +447,8 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     if (l < M.nu) {
       float act = A.actions[(size_t)env * M.act_dim + l];
       act = fminf(fmaxf(act, -1.f), 1.f);
-      sc = act > 0.f ? __fmul_rn(act, M.act_chi[l]) : __fmul_rn(fabsf(act), M.act_clo[l]);
+      if (PD) sc = __fadd_rn(M.pd_mid[l], __fmul_rn(act, M.pd_half[l]));
+      else sc = act > 0.f ? __fmul_rn(act, M.act_chi[l]) : __fmul_rn(fabsf(act), M.act_clo[l]);
     }
     {
       const int src = l < M.nu ? M.mirror_act_idx[l] : 0;
@@ -445,13 +458,25 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     E.tau[l] = 0.f;
     __syncwarp();
     if (l < M.nu) {
-      const float cc = fminf(fmaxf(sc, M.act_clo[l]), M.act_chi[l]);
-      force = fminf(fmaxf(M.act_gear[l] * cc, M.act_flo[l]), M.act_fhi[l]);
-      E.tau[M.act_dof[l]] = M.act_gear[l] * force;
+      const int j = M.act_dof[l];
+      if (PD) {
+        E.tau[j] = fminf(fmaxf(sc, M.dof_lo[j]), M.dof_hi[j]);
+      } else {
+        const float cc = fminf(fmaxf(sc, M.act_clo[l]), M.act_chi[l]);
+        force = fminf(fmaxf(M.act_gear[l] * cc, M.act_flo[l]), M.act_fhi[l]);
+        E.tau[j] = M.act_gear[l] * force;
+      }
     }
     __syncwarp();
   }
-  const float tau = E.tau[l];
+  // torque: the generalised actuator force of this dof for the whole step; PD: the servo target of this dof
+  const float tau_in = E.tau[l];
+  if (PD) {
+    // Monitor torque: the servo forces at the state the step starts from, gathered to the actuator lanes
+    const float f0 = L.isdof ? pd_force(M, jd, tau_in, q, v) : 0.f;
+    const float fu = __shfl_sync(kFull, f0, l < M.nu ? M.act_dof[l] : 0, G);
+    if (l < M.nu) force = fu;
+  }
   const float mean_abs_torque = group_sum<G>(l < M.nu ? fabsf(force) : 0.f) / (float)M.nu;
 
   // ---- physics: frame_skip x (RK4 | semi-implicit Euler) ---------------------------------------------------------
@@ -476,6 +501,7 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
         // no barrier or one before the solver is slower at 64, 96 and 128 threads per CTA: profiles/r02_kernel_ab.md)
         __syncthreads();
         Vec6 Sj;
+        const float tau = PD ? (L.isdof ? M.pd_gear[jd] * pd_force(M, jd, tau_in, q, v) : 0.f) : tau_in;
         forward_dynamics<NV, G, DBG>(M, E, L, CL, q, v, tau, a, AS, Sj, dbgp);
         const float bw = (st == 0 || st == 3) ? (1.f / 6.f) : (1.f / 3.f);
         accq = fmaf(bw, v, accq);
@@ -494,6 +520,8 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
       float Hc[NV + 1];
       float Ma = 0.f;
       Vec6 Sj;
+      // (PD: kv acts explicitly, as in MuJoCo's Euler; only joint damping is implicit)
+      const float tau = PD ? (L.isdof ? M.pd_gear[jd] * pd_force(M, jd, tau_in, q, v) : 0.f) : tau_in;
       forward_dynamics<NV, G, DBG>(M, E, L, CL, q, v, tau, a, AS, Sj, dbgp);
       pure_mass_column<NV, G>(M, E, L, Sj, Hc);     // E.acc holds the constrained qacc of every dof
 #pragma unroll
@@ -855,19 +883,19 @@ __global__ void state_copy_kernel(float* state_f, int* state_i, int* state_as, f
 // ------------------------------------------------------------------------------------------------------------------
 // BASELINE.json configs[1] (4096 walker3d envs = 27.7 envs per SM) is one wave only if four 128-thread blocks fit an SM:
 // 4 x (model + 8 environments + 1 KB reserved) <= 228 KB
-static_assert(4 * ((sizeof(DevModel) + 15) / 16 * 16 + 8 * sizeof(EnvSmem<16>) + 1024) <= 228 * 1024,
+static_assert(4 * (sizeof(DevModel) + 8 * sizeof(EnvSmem<16>) + 1024) <= 228 * 1024,
               "walker3d: four blocks per SM must fit in shared memory");
 
-size_t step_smem_bytes(int G, int envs_per_block) {
-  const size_t model = (sizeof(DevModel) + 15) / 16 * 16;
+size_t step_smem_bytes(int G, int envs_per_block, bool pd) {
+  const size_t model = pd ? sizeof(DevModel) : kModelBytesTorque;
   return model + (size_t)envs_per_block * (G == 16 ? sizeof(EnvSmem<16>) : sizeof(EnvSmem<32>));
 }
 
-template <int NV, int G, bool RK4, bool DBG>
+template <int NV, int G, bool RK4, bool DBG, bool PD>
 static cudaError_t launch_one(const StepArgs& a, int reset_only, int block, cudaStream_t st) {
   const int epb = block / G;
-  const size_t smem = step_smem_bytes(G, epb);
-  auto kern = mimic_step_kernel<NV, G, RK4, DBG>;
+  const size_t smem = step_smem_bytes(G, epb, PD);
+  auto kern = mimic_step_kernel<NV, G, RK4, DBG, PD>;
   // function attributes are per device: set them once for every device this process launches on
   static unsigned long long attr_done = 0ull;
   int dev = 0;
@@ -887,19 +915,23 @@ static cudaError_t launch_one(const StepArgs& a, int reset_only, int block, cuda
 }
 
 template <int NV, int G>
-static cudaError_t launch_model(const StepArgs& a, int rk4, int reset_only, int block, bool debug, cudaStream_t st) {
-  if (rk4) return launch_one<NV, G, true, false>(a, reset_only, block, st);
-  return debug ? launch_one<NV, G, false, true>(a, reset_only, block, st)
-               : launch_one<NV, G, false, false>(a, reset_only, block, st);
+static cudaError_t launch_model(const StepArgs& a, int rk4, int reset_only, int block, bool debug, bool pd,
+                                cudaStream_t st) {
+  if (pd) return rk4 ? launch_one<NV, G, true, false, true>(a, reset_only, block, st)
+                     : launch_one<NV, G, false, false, true>(a, reset_only, block, st);
+  if (rk4) return launch_one<NV, G, true, false, false>(a, reset_only, block, st);
+  return debug ? launch_one<NV, G, false, true, false>(a, reset_only, block, st)
+               : launch_one<NV, G, false, false, false>(a, reset_only, block, st);
 }
 
-// instantiated: walker3d (nv 14, 16 lanes) and walker_165cm_65kg (nv 19, 32 lanes), RK4 and Euler; the dump variant
-// exists for the Euler kernels only (tests evaluate single forward passes with it)
-cudaError_t launch_step(const StepArgs& a, int nv, int G, int rk4, int reset_only, int block, bool debug,
+// instantiated: walker3d (nv 14, 16 lanes) and walker_165cm_65kg (nv 19, 32 lanes), RK4 and Euler, torque and PD
+// actuation; the dump variant exists for the torque Euler kernels only (tests evaluate single forward passes with it).
+// A reset-only launch never reads the actions: callers use the torque instance for it.
+cudaError_t launch_step(const StepArgs& a, int nv, int G, int rk4, int reset_only, int block, bool debug, bool pd,
                         cudaStream_t st) {
-  if (debug && rk4) return cudaErrorInvalidValue;
-  if (nv == 14 && G == 16) return launch_model<14, 16>(a, rk4, reset_only, block, debug, st);
-  if (nv == 19 && G == 32) return launch_model<19, 32>(a, rk4, reset_only, block, debug, st);
+  if (debug && (rk4 || pd)) return cudaErrorInvalidValue;
+  if (nv == 14 && G == 16) return launch_model<14, 16>(a, rk4, reset_only, block, debug, pd, st);
+  if (nv == 19 && G == 32) return launch_model<19, 32>(a, rk4, reset_only, block, debug, pd, st);
   return cudaErrorInvalidValue;
 }
 

@@ -169,6 +169,13 @@ class B200MimicVecEnv:
         lib.check(self._lib.drl_create(C.byref(c), C.byref(self._handle)), "drl_create")
         self._cm = cabi.pack_model(m)
         lib.check(self._lib.drl_upload_model(self._handle, C.byref(self._cm)), "drl_upload_model")
+        if self.cfg.actuation == "pd":
+            # position servos (EnvConfig.actuation): the action picks each servo's target in its joint's range, so
+            # the policy acts in [-1, 1] (SB3 clips its samples to the action space before stepping)
+            kp, kv = self.cfg.pd_gains(m.nu)
+            lib.check(self._lib.drl_set_actuation(self._handle, cabi.ACTUATION_PD, kp.ctypes.data_as(C.c_void_p),
+                                                  kv.ctypes.data_as(C.c_void_p)), "drl_set_actuation")
+            self.action_space = Box(-1.0, 1.0, (m.nu,), dtype=np.float32)
         self._upload_mocap()
         with torch.cuda.device(self.device):
             N, D = self.num_envs, self.obs_dim

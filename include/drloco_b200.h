@@ -258,6 +258,25 @@ int drl_set_seed(DrlEnv* env, uint64_t seed);
  * linspace regions); n = 0 switches speed control off.  Synchronises the device (not for the stepping loop). */
 int drl_set_speed_profile(DrlEnv* env, const float* speeds, int32_t n);
 
+/* Actuation of the walker's motors.  The reference drives every joint with a motor whose force is the (rescaled)
+ * action, held for the whole control step (mimic_env.py:170-192): DRL_ACTUATION_TORQUE, the state after
+ * drl_upload_model.  DRL_ACTUATION_PD turns every motor into a MuJoCo position servo, <position kp kv> (the
+ * "PD/torque actuation" of the step kernel's scope, BASELINE.json north_star):
+ *   - the clipped action a_u in [-1, 1] of actuator u maps to the target ctrl_u = mid_u + a_u * half_u over the range
+ *     [lo, hi] of the joint it drives (mid = (lo + hi) / 2, half = (hi - lo) / 2, rounded to float32), then the policy
+ *     mirror applies as in torque mode; ctrl is held for the control step and clamped to the joint range;
+ *   - at every dynamics evaluation (all four RK4 stages of every substep; the one Euler evaluation, where kv is explicit
+ *     and only joint damping is implicit) the actuator force is f_u = clamp(kp_u (ctrl_u - gear_u q) - kv_u gear_u v,
+ *     forcerange_u) at that evaluation's q, v, and the generalised force gear_u f_u;
+ *   - the Monitor torque (DRL_EXTRA_MEAN_ABS_TORQUE, DRL_STAT_ABS_TORQUE_SUM, the median history) is mean_u |f_u| at
+ *     the state the step starts from.
+ * kp, kv: HOST float64 [nu] in actuator order, kp finite and > 0, kv finite and >= 0; ignored (may be NULL) for
+ * DRL_ACTUATION_TORQUE.  Every actuated joint must be limited.  DRL_ERR_STATE before drl_upload_model,
+ * DRL_ERR_INVALID for an unknown mode, bad gains or an unlimited actuated joint.  May be called again to switch modes.
+ * Synchronises the device (not for the stepping loop; a captured CUDA graph keeps the instance it captured). */
+typedef enum { DRL_ACTUATION_TORQUE = 0, DRL_ACTUATION_PD = 1 } DrlActuation;
+int drl_set_actuation(DrlEnv* env, int32_t mode, const double* kp, const double* kv);
+
 /* MimicEnv.playback_ref_trajectories (mimic_env.py:265-282): while on, drl_step skips the physics and, after
  * refs.next(), sets qpos / qvel from the mocap (set_joint_kinematics_in_sim, mimic_env.py:284-293) before the
  * observation, reward and termination logic run.  A kinematic check of tables, cursor and ground shift: the imitation

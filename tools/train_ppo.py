@@ -6,6 +6,7 @@ Usage: python tools/train_ppo.py --envs 4096 --steps 16000000 --out gpurun_out/p
               tools/train_ppo.py --envs 512 --steps 16000000 --out gpurun_out/ppo_8gpu.json     (data parallel)
        python tools/train_ppo.py --cpu-oracle --envs 8 --steps 1000000 --reference-hypers --out ...   (the same learner
               on the CPU oracle stack: the comparison curve of BASELINE.json configs[4])
+       python tools/train_ppo.py --actuation pd --kp 300 --kv 10 ...   (PD position servos instead of torque motors)
 """
 import argparse
 import json
@@ -36,6 +37,10 @@ def main():
     ap.add_argument("--reference-hypers", action="store_true",
                     help="the reference's rollout shape: 16384 samples per update, minibatch 2048 (hypers.py:78-79)")
     ap.add_argument("--no-eval", action="store_true")
+    ap.add_argument("--actuation", choices=("torque", "pd"), default="torque",
+                    help="torque: the action is the motor force (the reference); pd: position servos (EnvConfig.actuation)")
+    ap.add_argument("--kp", type=float, nargs="+", help="servo stiffness: one value or one per actuator (--actuation pd)")
+    ap.add_argument("--kv", type=float, nargs="+", help="servo damping, as --kp (default 0)")
     args = ap.parse_args()
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", "0"), ("WORLD_SIZE", "1"), ("LOCAL_RANK", "0")))
     if world > 1:
@@ -44,12 +49,20 @@ def main():
         # a short collective timeout: a rank that falls out of step must fail the run quickly, not hold the GPUs
         torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local),
                                              timeout=datetime.timedelta(seconds=90))
+    env_cfg = None
+    if args.actuation == "pd":
+        if args.cpu_oracle:
+            ap.error("--actuation pd runs on the GPU env only")
+        from drloco_b200.config import EnvConfig
+        gain = lambda g: None if g is None else (g[0] if len(g) == 1 else tuple(g))   # noqa: E731
+        env_cfg = EnvConfig(env_id="StraightMimicWalker", seed=33 + args.seed + 100 * rank, actuation="pd",
+                            pd_kp=gain(args.kp), pd_kv=gain(args.kv))
     if args.cpu_oracle:
         from tools.oracle_tensor_env import OracleTensorEnv
         env = OracleTensorEnv("StraightMimicWalker", args.envs, seed=33 + args.seed)
     else:
         env = vec_env("StraightMimicWalker", num_envs=args.envs, seed=33 + args.seed + 100 * rank, norm_rew=True,
-                      device=f"cuda:{local}", env_id_offset=rank * args.envs)
+                      device=f"cuda:{local}", env_id_offset=rank * args.envs, cfg=env_cfg)
     cfg = PPOConfig(total_steps=args.steps)
     if args.reference_hypers:
         cfg.batch_size, cfg.minibatch_size = 4096 * 4, 512 * 4
@@ -98,6 +111,7 @@ def main():
                        "total_steps": agent.num_timesteps, "wall_s": wall,
                        "env_steps_per_s_incl_learning": agent.num_timesteps / wall,
                        "replicas_bit_identical": lockstep,
+                       "actuation": args.actuation, "pd_kp": args.kp, "pd_kv": args.kv,
                        "config": {k: v for k, v in vars(cfg).items()}, "curve": agent.log, "evaluation": ev,
                        "evaluation_steady_state_counters": ev2}, f, indent=1)
         print("done: %.1f s, %.2e env-steps/s incl. learning, replicas bit-identical: %s"
