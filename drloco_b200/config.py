@@ -55,6 +55,9 @@ class EnvConfig:
     pd_kp: Union[None, float, Tuple[float, ...]] = None   # servo stiffness, > 0: one value for every actuator or one
                                                         # per actuator in actuator order; required with "pd"
     pd_kv: Union[None, float, Tuple[float, ...]] = None   # servo damping, >= 0, as pd_kp; None = 0 (MuJoCo's default)
+    contact_termination: bool = False                   # DeepMimic early termination: the episode also ends when a
+                                                        # body other than the feet touches the floor; off = the
+                                                        # reference (see README "Contact termination")
     gamma: float = 0.0                                  # 0 -> by ctrl_freq, hypers.py:68
     integrator: str = "rk4"                             # xml:11; "euler" = MuJoCo semi-implicit Euler (fast mode)
     seed: int = 33                                      # utils.py:97

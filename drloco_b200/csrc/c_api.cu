@@ -89,6 +89,8 @@ struct DrlEnv {
   // end-effector term (cfg.ee_weight > 0): last / smoothed ee_rew, lifetime sum
   float* ee_f = nullptr;
   double* ee_d = nullptr;
+  // contact termination (drl_set_contact_termination): per-env episode count, allocated when first enabled
+  int* contact_et = nullptr;
   // per-step statistics rows (one per thread block of the step kernel) + the ticket that elects the summing block
   double* cta_rows = nullptr;
   unsigned* cta_ticket = nullptr;
@@ -128,7 +130,8 @@ static void free_state(DrlEnv* e) {
                    (void**)&e->state_d, (void**)&e->extras_last, (void**)&e->stats, (void**)&e->ring_len,
                    (void**)&e->ring_ret, (void**)&e->ring_head, (void**)&e->ring_rsi_pos, (void**)&e->ring_et_pos,
                    (void**)&e->ring_difficult, (void**)&e->cta_rows, (void**)&e->cta_ticket,
-                   (void**)&e->tor_hist, (void**)&e->med_tor_sm, (void**)&e->ee_f, (void**)&e->ee_d};
+                   (void**)&e->tor_hist, (void**)&e->med_tor_sm, (void**)&e->ee_f, (void**)&e->ee_d,
+                   (void**)&e->contact_et};
   for (void** p : ptrs) {
     if (*p) cudaFree(*p);
     *p = nullptr;
@@ -456,6 +459,7 @@ static StepArgs make_args(DrlEnv* e) {
   a.cta_rows = e->cta_rows; a.cta_ticket = e->cta_ticket;
   a.tor_hist = e->tor_hist; a.med_tor_sm = e->med_tor_sm;
   a.ee_f = e->ee_f; a.ee_d = e->ee_d;
+  a.contact_et = e->hm.et_contact_mask ? e->contact_et : nullptr;
   a.vn_ret = e->vn_ret; a.vn_gamma = e->vn_gamma; a.packed = e->vn_packed;
   if (e->playback) a.frame_skip = 0;
   a.debug = e->debug;
@@ -680,6 +684,38 @@ extern "C" int drl_set_actuation(DrlEnv* e, int32_t mode, const double* kp, cons
   DeviceGuard guard__(e->cfg.device);
   CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the model block
   CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
+  return DRL_OK;
+}
+
+extern "C" int drl_set_contact_termination(DrlEnv* e, uint32_t body_mask) {
+  if (!e) return fail(DRL_ERR_INVALID, "drl_set_contact_termination: null env");
+  if (!e->have_model) return fail(DRL_ERR_STATE, "drl_set_contact_termination: upload the model first");
+  DevModel& d = e->hm;
+  if (body_mask >> d.nb) return fail(DRL_ERR_INVALID, "drl_set_contact_termination: mask 0x%x names a body >= nb = %d",
+                                     body_mask, d.nb);
+  // the reset puts the lowest foot-corner site on the floor: a body that carries one would end every episode at once
+  for (int s = 0; s < d.nsite; s++)
+    if ((body_mask >> d.site_body[s]) & 1u)
+      return fail(DRL_ERR_INVALID, "drl_set_contact_termination: body %d carries a foot-corner site", d.site_body[s]);
+  DeviceGuard guard__(e->cfg.device);
+  if (body_mask && !e->contact_et) {
+    const size_t N = (size_t)e->cfg.num_envs;
+    CUDA_TRY(cudaMalloc(&e->contact_et, N * sizeof(int)));
+    CUDA_TRY(cudaMemset(e->contact_et, 0, N * sizeof(int)));
+  }
+  d.et_contact_mask = body_mask;
+  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the model block
+  CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
+  return DRL_OK;
+}
+
+extern "C" int drl_get_contact_terminations(DrlEnv* e, int32_t* out, void* stream) {
+  if (!e || !out) return fail(DRL_ERR_INVALID, "drl_get_contact_terminations: null argument");
+  if (!e->contact_et)
+    return fail(DRL_ERR_STATE, "drl_get_contact_terminations: contact termination was never enabled on this env");
+  DeviceGuard guard__(e->cfg.device);
+  CUDA_TRY(cudaMemcpyAsync(out, e->contact_et, (size_t)e->cfg.num_envs * sizeof(int32_t), cudaMemcpyDeviceToDevice,
+                           (cudaStream_t)stream));
   return DRL_OK;
 }
 

@@ -56,7 +56,10 @@ struct alignas(16) DevModel {
   unsigned box_body_mask;            // bodies that carry a box geom (their contact accumulators are segment-written)
   unsigned com_mask;                 // dofs excluded from the pose / velocity reward (COM indices 0,1,2)
   int com_z_dof;
-  int early_termination, trunk_dof0, pad_et[2];   // do_terminate_early: off/on, first of the three trunk rotation dofs
+  int early_termination, trunk_dof0;   // do_terminate_early: off/on, first of the three trunk rotation dofs
+  unsigned et_contact_mask;          // DeepMimic contact termination (drl_set_contact_termination): bodies that end
+                                     // the episode when they touch the floor; 0 = off
+  int pad_et_;
   // ---- mocap ----
   int cursor_mode, increment, n_steps, n_samples, com_z_col, des_vel_window;
   unsigned long long seed;
@@ -143,6 +146,8 @@ struct StepArgs {
   // end-effector term, allocated only when it is on (DevModel::w_ee != 0), null otherwise
   float* ee_f;                       // [N][2] ee_rew of the last step (1 after a reset), Monitor-smoothed mean
   double* ee_d;                      // [N] lifetime sum of ee_rew (Monitor never clears its per-step lists)
+  // contact termination (DevModel::et_contact_mask != 0), null while it is off
+  int* contact_et;                   // [N] lifetime count of episodes that ended on a step with a listed body on the floor
 };
 
 }  // namespace drl

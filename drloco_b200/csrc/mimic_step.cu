@@ -303,6 +303,42 @@ __device__ __noinline__ float ee_sq_error(const DevModel& M, ES& E, const LaneCo
   return group_sum<G>(own ? d[0] * d[0] + d[1] * d[1] + d[2] * d[2] : 0.f);
 }
 
+// DeepMimic contact termination: does a body of M.et_contact_mask touch the floor at the joint configuration q?  A
+// contact candidate touches when its signed distance to the floor is <= 0, the test with which forward_dynamics
+// activates it, taken before the plane-box cap of four corners (which does not change whether a body touches).  The
+// root height and the distances restate forward_dynamics (fd_tree.cuh, steps 1 and 7) so that its hot loop stays as it
+// is.  Overwrites E.cssn and the body frames / joint axes of the first EnvSmem union; E.obsbuf and E.Mt are untouched.
+// Called by every lane of the warp; every lane of an environment gets its environment's answer.
+template <int NV, int G, class ES>
+__device__ __noinline__ bool floor_contact(const DevModel& M, ES& E, const LaneConst& L, const ChainLane& CL,
+                                           float q) {
+  using T = Topo<NV>;
+  const int l = L.l;
+  const unsigned mask = M.et_contact_mask;
+  publish_joint_trig(M, E, L, q);
+  float zO = M.root_z0;
+#pragma unroll
+  for (int j = 0; j < T::NSLIDE; j++) zO = fmaf(M.dof_slide_z[j], E.cssn[j][1], zO);
+  tree_kinematics<NV, G>(M, E, CL, l);
+  bool touch = false;
+  if (l < M.nbox_cand) {                       // box corner s = l
+    const int b = M.cand_body[l];
+    const float4 r2 = *reinterpret_cast<const float4*>(&E.bodyR[b][8]);
+    const float rz = r2.x * M.cand_pos[l][0] + r2.y * M.cand_pos[l][1] + r2.z * M.cand_pos[l][2];
+    const float cz = zO + r2.w + r2.x * M.cand_aux[l][0] + r2.y * M.cand_aux[l][1] + r2.z * M.cand_aux[l][2];
+    touch = ((mask >> b) & 1u) && !(cz + rz > 0.f);
+  }
+  const int s1 = G + l;                        // capsule end sphere s = G + l
+  if (s1 < M.ncand) {
+    const int b1 = M.cand_body[s1];
+    const float4 r2 = *reinterpret_cast<const float4*>(&E.bodyR[b1][8]);
+    const float rz = r2.x * M.cand_pos[s1][0] + r2.y * M.cand_pos[s1][1] + r2.z * M.cand_pos[s1][2];
+    const float dist1 = zO + r2.w + rz - M.cand_aux[s1][0];
+    touch = touch || (((mask >> b1) & 1u) && !(dist1 > 0.f));
+  }
+  return env_any(touch, L.emask);
+}
+
 template <int NV, int G, class ES>
 __device__ __noinline__ void reset_env(const DevModel& M, const StepArgs& A, ES& E, const LaneConst& L,
                                        const ChainLane& CL, int env, Cursor& c, float& q, float& v, float& dist,
@@ -583,7 +619,16 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     if (A.playback) et_low = et_trunk = et_drunk = false;
   }
   const bool et_done = M.early_termination && (et_low || et_trunk || et_drunk);
-  done = (comz < M.fall_z) || timeout || et_done;               // mimic_env.py:113-120
+  // optional DeepMimic contact termination (et_contact_mask lives in the CTA's shared model block, playback is a launch
+  // argument: warp-uniform), at the state the step ends in.  A blow-up wins, and playback skips it like the reasons
+  // above.  Runs before ee_sq_error: both overwrite the body frames.  A step on which it holds is always terminal, so
+  // the episode counter is incremented here (A.contact_et is non-null whenever the mask is).
+  bool et_contact = false;
+  if (M.et_contact_mask != 0u && !A.playback) {
+    et_contact = floor_contact<NV, G>(M, E, L, CL, q) && !bad;
+    if (et_contact && l == 0 && live) A.contact_et[env] += 1;
+  }
+  done = (comz < M.fall_z) || timeout || et_done || et_contact;   // mimic_env.py:113-120
   {
     const float dq = L.isdof ? q - rq : 0.f, dv = L.isdof ? v - rv : 0.f;
     const bool iscom = (M.com_mask >> l) & 1u;

@@ -187,6 +187,13 @@ def mass_matrix(m: WalkerModel, q: np.ndarray) -> np.ndarray:
     return M
 
 
+def contact_body_mask(m: WalkerModel) -> int:
+    """Bodies whose floor contact ends an episode under EnvConfig.contact_termination (bit b = body b): every body that
+    carries none of the foot-corner sites, i.e. all but the feet."""
+    feet = set(int(b) for b in m.site_body)
+    return sum(1 << b for b in range(m.nb) if b not in feet)
+
+
 def _set_const(m: WalkerModel) -> None:
     """dof_invweight0 / body_invweight0 as MuJoCo's mj_setConst defines them at qpos0."""
     q0 = m.qpos0

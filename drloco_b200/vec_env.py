@@ -21,6 +21,7 @@ import numpy as np
 import torch
 
 from . import cabi, config as cfgm, lib
+from .model import contact_body_mask
 from .walkers import WalkerSpec, make_spec, speed_profile
 
 
@@ -176,6 +177,10 @@ class B200MimicVecEnv:
             lib.check(self._lib.drl_set_actuation(self._handle, cabi.ACTUATION_PD, kp.ctypes.data_as(C.c_void_p),
                                                   kv.ctypes.data_as(C.c_void_p)), "drl_set_actuation")
             self.action_space = Box(-1.0, 1.0, (m.nu,), dtype=np.float32)
+        if self.cfg.contact_termination:
+            # DeepMimic contact termination (EnvConfig.contact_termination): every body without a foot-corner site
+            lib.check(self._lib.drl_set_contact_termination(self._handle, contact_body_mask(m)),
+                      "drl_set_contact_termination")
         self._upload_mocap()
         with torch.cuda.device(self.device):
             N, D = self.num_envs, self.obs_dim
@@ -433,6 +438,16 @@ class B200MimicVecEnv:
                           "drl_get_ee_reward")
             vals = out.cpu().numpy()
             return [float(vals[i]) for i in idx]
+        if attr_name == "contact_terminations":            # EnvConfig.contact_termination
+            if not self.cfg.contact_termination:
+                raise AttributeError("contact_terminations: the env was built with "
+                                     "EnvConfig(contact_termination=False)")
+            with torch.cuda.device(self.device):
+                out = torch.zeros(self.num_envs, dtype=torch.int32, device=self.device)
+                lib.check(self._lib.drl_get_contact_terminations(self._handle, _ptr(out), self._stream()),
+                          "drl_get_contact_terminations")
+            vals = out.cpu().numpy()
+            return [int(vals[i]) for i in idx]
         if attr_name == "ep_lens":
             # the reference returns one list per env and the callback flattens them (callback.py:227-230)
             lens = self.episode_lengths().tolist()

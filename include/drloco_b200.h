@@ -277,6 +277,22 @@ int drl_set_speed_profile(DrlEnv* env, const float* speeds, int32_t n);
 typedef enum { DRL_ACTUATION_TORQUE = 0, DRL_ACTUATION_PD = 1 } DrlActuation;
 int drl_set_actuation(DrlEnv* env, int32_t mode, const double* kp, const double* kv);
 
+/* DeepMimic contact termination (not in the reference): the episode also ends when a body of body_mask (bit b = body b)
+ * touches the floor, i.e. when a contact candidate of one of its geoms (a box corner, or a capsule end sphere at
+ * centre_z - radius) is at or below z = 0.  Checked once per control step, at the state the step ends in (not at the
+ * intermediate RK4 stages), and skipped on a simulator blow-up and in playback.  Such a step is terminal like a fall:
+ * reward -0 (+0 when it is also the timeout), counted in DRL_STAT_FALLS (DRL_STAT_TIMEOUTS with the timeout).
+ * body_mask = 0 turns it off, the state after drl_upload_model.  DRL_ERR_STATE before drl_upload_model,
+ * DRL_ERR_INVALID for a bit >= nb or a body that carries a foot-corner site (the reset puts the lowest of those on the
+ * floor).  The first call with a non-zero mask allocates and zeroes the per-env counter of drl_get_contact_terminations.
+ * Synchronises the device (not for the stepping loop; a captured CUDA graph keeps the arguments it captured). */
+int drl_set_contact_termination(DrlEnv* env, uint32_t body_mask);
+
+/* lifetime count per env of the episodes that ended on a step where the contact check held (blow-ups excluded; also
+ * the ones that fell or timed out on the same step).  out: device int32 [N].  DRL_ERR_STATE when contact termination
+ * was never enabled on this env. */
+int drl_get_contact_terminations(DrlEnv* env, int32_t* out, void* stream);
+
 /* MimicEnv.playback_ref_trajectories (mimic_env.py:265-282): while on, drl_step skips the physics and, after
  * refs.next(), sets qpos / qvel from the mocap (set_joint_kinematics_in_sim, mimic_env.py:284-293) before the
  * observation, reward and termination logic run.  A kinematic check of tables, cursor and ground shift: the imitation

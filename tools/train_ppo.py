@@ -7,6 +7,7 @@ Usage: python tools/train_ppo.py --envs 4096 --steps 16000000 --out gpurun_out/p
        python tools/train_ppo.py --cpu-oracle --envs 8 --steps 1000000 --reference-hypers --out ...   (the same learner
               on the CPU oracle stack: the comparison curve of BASELINE.json configs[4])
        python tools/train_ppo.py --actuation pd --kp 300 --kv 10 ...   (PD position servos instead of torque motors)
+       python tools/train_ppo.py --contact-termination ...   (DeepMimic early termination on non-foot floor contact)
 """
 import argparse
 import json
@@ -41,6 +42,9 @@ def main():
                     help="torque: the action is the motor force (the reference); pd: position servos (EnvConfig.actuation)")
     ap.add_argument("--kp", type=float, nargs="+", help="servo stiffness: one value or one per actuator (--actuation pd)")
     ap.add_argument("--kv", type=float, nargs="+", help="servo damping, as --kp (default 0)")
+    ap.add_argument("--contact-termination", action="store_true",
+                    help="end an episode when a body other than the feet touches the floor "
+                         "(EnvConfig.contact_termination)")
     args = ap.parse_args()
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", "0"), ("WORLD_SIZE", "1"), ("LOCAL_RANK", "0")))
     if world > 1:
@@ -50,13 +54,16 @@ def main():
         torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local),
                                              timeout=datetime.timedelta(seconds=90))
     env_cfg = None
-    if args.actuation == "pd":
+    if args.actuation == "pd" or args.contact_termination:
         if args.cpu_oracle:
-            ap.error("--actuation pd runs on the GPU env only")
+            ap.error("--actuation pd and --contact-termination run on the GPU env only")
         from drloco_b200.config import EnvConfig
-        gain = lambda g: None if g is None else (g[0] if len(g) == 1 else tuple(g))   # noqa: E731
-        env_cfg = EnvConfig(env_id="StraightMimicWalker", seed=33 + args.seed + 100 * rank, actuation="pd",
-                            pd_kp=gain(args.kp), pd_kv=gain(args.kv))
+        pd = dict()
+        if args.actuation == "pd":
+            gain = lambda g: None if g is None else (g[0] if len(g) == 1 else tuple(g))   # noqa: E731
+            pd = dict(actuation="pd", pd_kp=gain(args.kp), pd_kv=gain(args.kv))
+        env_cfg = EnvConfig(env_id="StraightMimicWalker", seed=33 + args.seed + 100 * rank,
+                            contact_termination=args.contact_termination, **pd)
     if args.cpu_oracle:
         from tools.oracle_tensor_env import OracleTensorEnv
         env = OracleTensorEnv("StraightMimicWalker", args.envs, seed=33 + args.seed)
@@ -112,6 +119,7 @@ def main():
                        "env_steps_per_s_incl_learning": agent.num_timesteps / wall,
                        "replicas_bit_identical": lockstep,
                        "actuation": args.actuation, "pd_kp": args.kp, "pd_kv": args.kv,
+                       "contact_termination": args.contact_termination,
                        "config": {k: v for k, v in vars(cfg).items()}, "curve": agent.log, "evaluation": ev,
                        "evaluation_steady_state_counters": ev2}, f, indent=1)
         print("done: %.1f s, %.2e env-steps/s incl. learning, replicas bit-identical: %s"
