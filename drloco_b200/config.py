@@ -58,6 +58,12 @@ class EnvConfig:
     contact_termination: bool = False                   # DeepMimic early termination: the episode also ends when a
                                                         # body other than the feet touches the floor; off = the
                                                         # reference (see README "Contact termination")
+    adaptive_rsi: float = 0.0                           # failure-weighted RSI: the share (0 < lambda <= 1) of random
+                                                        # RSI draws that favour the mocap phases where episodes end
+                                                        # early; 0 = off, the reference's uniform draw (see README
+                                                        # "Failure-weighted RSI")
+    adaptive_rsi_halflife: int = 2000                   # half-life of its per-phase counts, in control steps of the
+                                                        # batch (a choice, not a tuned value)
     gamma: float = 0.0                                  # 0 -> by ctrl_freq, hypers.py:68
     integrator: str = "rk4"                             # xml:11; "euler" = MuJoCo semi-implicit Euler (fast mode)
     seed: int = 33                                      # utils.py:97
@@ -79,6 +85,12 @@ class EnvConfig:
             if self.pd_kp is None:
                 raise ValueError("actuation='pd' needs pd_kp (there are no default gains)")
             self.pd_gains()
+        lam = self.adaptive_rsi
+        if isinstance(lam, bool) or not isinstance(lam, (int, float, np.integer, np.floating)) or not (0.0 <= lam <= 1.0):
+            raise ValueError(f"adaptive_rsi must be a number in [0, 1], got {lam!r}")
+        hl = self.adaptive_rsi_halflife
+        if isinstance(hl, bool) or not isinstance(hl, (int, np.integer)) or hl <= 0 or hl >= 2 ** 31:
+            raise ValueError(f"adaptive_rsi_halflife must be a positive int32 number of control steps, got {hl!r}")
 
     def pd_gains(self, nu: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
         """(kp, kv) of actuation='pd' as float64 arrays in actuator order, scalars broadcast to the walker's nu

@@ -19,6 +19,7 @@ cudaError_t launch_step(const StepArgs& a, int nv, int G, int rk4, int reset_onl
 cudaError_t launch_running_rsi(const int* state_i, int* out, int n, cudaStream_t st);
 bool topology_matches(int nv, int nb, const int* body_parent, const int* dof_body, const int* dof_type);
 cudaError_t launch_extras(const float* state_f, const float* last, float* out, int n, int G, cudaStream_t st);
+cudaError_t launch_adaptive_rsi_update(const AdaptiveRsiArgs& a, cudaStream_t st);
 cudaError_t launch_state_copy(float* state_f, int* state_i, int* state_as, float* qpos, float* qvel, int* cursor, int n,
                               int nv, int G, int to_state, cudaStream_t st);
 }  // namespace drl
@@ -91,6 +92,18 @@ struct DrlEnv {
   double* ee_d = nullptr;
   // contact termination (drl_set_contact_termination): per-env episode count, allocated when first enabled
   int* contact_et = nullptr;
+  // failure-weighted RSI (drl_set_adaptive_rsi): tables allocated when first enabled for a bin layout
+  std::vector<int> step_len_h;            // host copy of the mocap step lengths (the bin layout is built from them)
+  int mocap_gen = 0;                      // bumped by every drl_upload_mocap
+  int ars_gen = -1, ars_bin_samples = 0, ars_n_bins = 0, ars_halflife = 0;
+  float ars_lambda = 0.f;                 // 0 = off
+  double* ars_counts = nullptr;           // [2][n_bins] started, difficult
+  double* ars_u = nullptr;                // [n_bins]
+  double* ars_cdf = nullptr;              // [n_bins]
+  double* ars_prob = nullptr;             // [n_bins]
+  int* ars_bins = nullptr;                // [n_bins][3] step, first, width; [n_steps] first bin of each step
+  unsigned* ars_inc = nullptr;            // [2][n_bins]
+  int* ars_env_bin = nullptr;             // [N]
   // per-step statistics rows (one per thread block of the step kernel) + the ticket that elects the summing block
   double* cta_rows = nullptr;
   unsigned* cta_ticket = nullptr;
@@ -131,7 +144,8 @@ static void free_state(DrlEnv* e) {
                    (void**)&e->ring_ret, (void**)&e->ring_head, (void**)&e->ring_rsi_pos, (void**)&e->ring_et_pos,
                    (void**)&e->ring_difficult, (void**)&e->cta_rows, (void**)&e->cta_ticket,
                    (void**)&e->tor_hist, (void**)&e->med_tor_sm, (void**)&e->ee_f, (void**)&e->ee_d,
-                   (void**)&e->contact_et};
+                   (void**)&e->contact_et, (void**)&e->ars_counts, (void**)&e->ars_u, (void**)&e->ars_cdf,
+                   (void**)&e->ars_prob, (void**)&e->ars_bins, (void**)&e->ars_inc, (void**)&e->ars_env_bin};
   for (void** p : ptrs) {
     if (*p) cudaFree(*p);
     *p = nullptr;
@@ -402,6 +416,8 @@ extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t incremen
     return fail(DRL_ERR_INVALID, "drl_upload_mocap: null argument");
   if (!e->have_model) return fail(DRL_ERR_STATE, "drl_upload_mocap: upload the model first");
   if (n_samples <= 0 || n_steps <= 0 || increment <= 0) return fail(DRL_ERR_INVALID, "drl_upload_mocap: empty mocap");
+  if (e->ars_lambda > 0.f)
+    return fail(DRL_ERR_STATE, "drl_upload_mocap: failure-weighted RSI is on (its bins would go stale); set lambda 0 first");
   if (cursor_mode != DRL_CURSOR_STEPWISE && cursor_mode != DRL_CURSOR_WRAP)
     return fail(DRL_ERR_INVALID, "drl_upload_mocap: unknown cursor mode");
   if (cursor_mode == DRL_CURSOR_WRAP && (n_steps != 1 || !des_vel_prefix))
@@ -431,6 +447,8 @@ extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t incremen
   d.cursor_mode = cursor_mode; d.increment = increment; d.n_steps = n_steps; d.n_samples = n_samples;
   d.com_z_col = com_z_col; d.des_vel_window = des_vel_window;
   CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
+  e->step_len_h.assign(step_len, step_len + n_steps);
+  e->mocap_gen++;
   e->have_mocap = true;
   return DRL_OK;
 }
@@ -439,6 +457,13 @@ static int ready(DrlEnv* e, const char* who) {
   if (!e) return fail(DRL_ERR_INVALID, "%s: null env", who);
   if (!e->have_model || !e->have_mocap) return fail(DRL_ERR_STATE, "%s: model and mocap must be uploaded first", who);
   return DRL_OK;
+}
+
+static AdaptiveRsiArgs ars_args(DrlEnv* e, double rho) {
+  AdaptiveRsiArgs a;
+  a.n_bins = e->ars_n_bins; a.rho = rho; a.lambda = (double)e->ars_lambda;
+  a.u = e->ars_u; a.counts = e->ars_counts; a.inc = e->ars_inc; a.cdf = e->ars_cdf; a.prob = e->ars_prob;
+  return a;
 }
 
 static StepArgs make_args(DrlEnv* e) {
@@ -460,6 +485,11 @@ static StepArgs make_args(DrlEnv* e) {
   a.tor_hist = e->tor_hist; a.med_tor_sm = e->med_tor_sm;
   a.ee_f = e->ee_f; a.ee_d = e->ee_d;
   a.contact_et = e->hm.et_contact_mask ? e->contact_et : nullptr;
+  if (e->ars_lambda > 0.f) {
+    a.ars_coin = (unsigned long long)llround((double)e->ars_lambda * 4294967296.0);
+    a.ars_n_bins = e->ars_n_bins; a.ars_bin_samples = e->ars_bin_samples;
+    a.ars_cdf = e->ars_cdf; a.ars_bins = e->ars_bins; a.ars_inc = e->ars_inc; a.ars_env_bin = e->ars_env_bin;
+  }
   a.vn_ret = e->vn_ret; a.vn_gamma = e->vn_gamma; a.packed = e->vn_packed;
   if (e->playback) a.frame_skip = 0;
   a.debug = e->debug;
@@ -493,6 +523,8 @@ extern "C" int drl_step(DrlEnv* e, const float* actions, float* obs, float* rew,
   if (e->debug && rk4) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for the Euler integrator only");
   if (e->debug && pd) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for torque actuation only");
   CUDA_TRY(launch_step(a, e->nv, e->G, rk4, 0, e->block, e->debug != nullptr, pd, (cudaStream_t)stream));
+  if (e->ars_lambda > 0.f) CUDA_TRY(launch_adaptive_rsi_update(ars_args(e, pow(2.0, -1.0 / e->ars_halflife)),
+                                                               (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -519,6 +551,9 @@ extern "C" int drl_set_state(DrlEnv* e, const float* qpos, const float* qvel, co
   DeviceGuard guard__(e->cfg.device);
   CUDA_TRY(launch_state_copy(e->state_f, e->state_i, e->state_as, const_cast<float*>(qpos), const_cast<float*>(qvel),
                              const_cast<int32_t*>(cursor), e->cfg.num_envs, e->nv, e->G, 1, (cudaStream_t)stream));
+  // an episode that continues from a state set here is no longer one that started with a random RSI draw
+  if (e->ars_env_bin)
+    CUDA_TRY(cudaMemsetAsync(e->ars_env_bin, 0xFF, (size_t)e->cfg.num_envs * sizeof(int), (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -716,6 +751,106 @@ extern "C" int drl_get_contact_terminations(DrlEnv* e, int32_t* out, void* strea
   DeviceGuard guard__(e->cfg.device);
   CUDA_TRY(cudaMemcpyAsync(out, e->contact_et, (size_t)e->cfg.num_envs * sizeof(int32_t), cudaMemcpyDeviceToDevice,
                            (cudaStream_t)stream));
+  return DRL_OK;
+}
+
+// the bin layout of the failure-weighted RSI table for the current mocap: bins of at most bin_samples consecutive samples
+// inside each mocap step, in step order.  Fills bins ([n_bins][3] step, first, width, then [n_steps] first bin of each
+// step) and u (the probability of each bin under the reference's uniform draw).
+static void ars_layout(const std::vector<int>& step_len, int bin_samples, std::vector<int>& bins, std::vector<double>& u) {
+  bins.clear(); u.clear();
+  std::vector<int> first_bin;
+  const double inv_steps = 1.0 / (double)step_len.size();
+  for (size_t s = 0; s < step_len.size(); s++) {
+    first_bin.push_back((int)u.size());
+    for (int p = 0; p < step_len[s]; p += bin_samples) {
+      const int w = step_len[s] - p < bin_samples ? step_len[s] - p : bin_samples;
+      bins.push_back((int)s); bins.push_back(p); bins.push_back(w);
+      u.push_back(inv_steps * (double)w / (double)step_len[s]);
+    }
+  }
+  bins.insert(bins.end(), first_bin.begin(), first_bin.end());
+}
+
+extern "C" int drl_set_adaptive_rsi(DrlEnv* e, float lambda, int32_t halflife_steps, int32_t bin_samples) {
+  if (!e) return fail(DRL_ERR_INVALID, "drl_set_adaptive_rsi: null env");
+  if (!(lambda >= 0.f && lambda <= 1.f))
+    return fail(DRL_ERR_INVALID, "drl_set_adaptive_rsi: lambda = %g outside [0, 1]", (double)lambda);
+  if (halflife_steps <= 0) return fail(DRL_ERR_INVALID, "drl_set_adaptive_rsi: halflife_steps must be > 0");
+  if (bin_samples <= 0) return fail(DRL_ERR_INVALID, "drl_set_adaptive_rsi: bin_samples must be > 0");
+  if (!e->have_model || !e->have_mocap)
+    return fail(DRL_ERR_STATE, "drl_set_adaptive_rsi: model and mocap must be uploaded first");
+  DeviceGuard guard__(e->cfg.device);
+  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the tables
+  if (lambda > 0.f && (e->ars_gen != e->mocap_gen || e->ars_bin_samples != bin_samples)) {
+    // first enable for this mocap and bin width: a new, empty table; every running episode is uncounted
+    std::vector<int> bins;
+    std::vector<double> u;
+    ars_layout(e->step_len_h, bin_samples, bins, u);
+    const size_t nb = u.size(), N = (size_t)e->cfg.num_envs;
+    void** ptrs[] = {(void**)&e->ars_counts, (void**)&e->ars_u, (void**)&e->ars_cdf, (void**)&e->ars_prob,
+                     (void**)&e->ars_bins, (void**)&e->ars_inc, (void**)&e->ars_env_bin};
+    for (void** p : ptrs) {
+      if (*p) CUDA_TRY(cudaFree(*p));
+      *p = nullptr;
+    }
+    e->ars_gen = -1;
+    CUDA_TRY(cudaMalloc(&e->ars_counts, 2 * nb * sizeof(double)));
+    CUDA_TRY(cudaMalloc(&e->ars_u, nb * sizeof(double)));
+    CUDA_TRY(cudaMalloc(&e->ars_cdf, nb * sizeof(double)));
+    CUDA_TRY(cudaMalloc(&e->ars_prob, nb * sizeof(double)));
+    CUDA_TRY(cudaMalloc(&e->ars_bins, bins.size() * sizeof(int)));
+    CUDA_TRY(cudaMalloc(&e->ars_inc, 2 * nb * sizeof(unsigned)));
+    CUDA_TRY(cudaMalloc(&e->ars_env_bin, N * sizeof(int)));
+    CUDA_TRY(cudaMemset(e->ars_counts, 0, 2 * nb * sizeof(double)));
+    CUDA_TRY(cudaMemset(e->ars_inc, 0, 2 * nb * sizeof(unsigned)));
+    CUDA_TRY(cudaMemset(e->ars_env_bin, 0xFF, N * sizeof(int)));
+    CUDA_TRY(cudaMemcpy(e->ars_u, u.data(), nb * sizeof(double), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(e->ars_bins, bins.data(), bins.size() * sizeof(int), cudaMemcpyHostToDevice));
+    e->ars_n_bins = (int)nb;
+    e->ars_bin_samples = bin_samples;
+    e->ars_gen = e->mocap_gen;
+  }
+  e->ars_lambda = lambda;
+  e->ars_halflife = halflife_steps;
+  if (e->ars_counts) {                        // rebuild the sampling tables (and prob, which depends on lambda)
+    CUDA_TRY(launch_adaptive_rsi_update(ars_args(e, 1.0), nullptr));
+    CUDA_TRY(cudaDeviceSynchronize());
+  }
+  return DRL_OK;
+}
+
+extern "C" int drl_get_adaptive_rsi(DrlEnv* e, double* started, double* difficult, double* prob, int32_t* env_bin,
+                                    void* stream) {
+  if (!e) return fail(DRL_ERR_INVALID, "drl_get_adaptive_rsi: null env");
+  if (!e->ars_counts) return fail(DRL_ERR_STATE, "drl_get_adaptive_rsi: failure-weighted RSI was never enabled");
+  DeviceGuard guard__(e->cfg.device);
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t nb = (size_t)e->ars_n_bins;
+  if (started) CUDA_TRY(cudaMemcpyAsync(started, e->ars_counts, nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  if (difficult)
+    CUDA_TRY(cudaMemcpyAsync(difficult, e->ars_counts + nb, nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  if (prob) CUDA_TRY(cudaMemcpyAsync(prob, e->ars_prob, nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  if (env_bin)
+    CUDA_TRY(cudaMemcpyAsync(env_bin, e->ars_env_bin, (size_t)e->cfg.num_envs * sizeof(int), cudaMemcpyDeviceToDevice,
+                             st));
+  return DRL_OK;
+}
+
+extern "C" int drl_set_adaptive_rsi_counts(DrlEnv* e, const double* started, const double* difficult) {
+  if (!e || !started || !difficult) return fail(DRL_ERR_INVALID, "drl_set_adaptive_rsi_counts: null argument");
+  if (!e->ars_counts) return fail(DRL_ERR_STATE, "drl_set_adaptive_rsi_counts: failure-weighted RSI was never enabled");
+  const int nb = e->ars_n_bins;
+  for (int b = 0; b < nb; b++)
+    if (!(isfinite(started[b]) && difficult[b] >= 0.0 && difficult[b] <= started[b]))
+      return fail(DRL_ERR_INVALID, "drl_set_adaptive_rsi_counts: bin %d: need 0 <= difficult <= started < inf", b);
+  DeviceGuard guard__(e->cfg.device);
+  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the tables
+  CUDA_TRY(cudaMemcpy(e->ars_counts, started, nb * sizeof(double), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(e->ars_counts + nb, difficult, nb * sizeof(double), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemset(e->ars_inc, 0, 2 * (size_t)nb * sizeof(unsigned)));
+  CUDA_TRY(launch_adaptive_rsi_update(ars_args(e, 1.0), nullptr));
+  CUDA_TRY(cudaDeviceSynchronize());
   return DRL_OK;
 }
 

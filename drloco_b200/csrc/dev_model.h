@@ -148,6 +148,26 @@ struct StepArgs {
   double* ee_d;                      // [N] lifetime sum of ee_rew (Monitor never clears its per-step lists)
   // contact termination (DevModel::et_contact_mask != 0), null while it is off
   int* contact_et;                   // [N] lifetime count of episodes that ended on a step with a listed body on the floor
+  // failure-weighted reference state initialisation (drl_set_adaptive_rsi), null / 0 while it is off.  A random RSI
+  // draw takes the weighted branch when the low 32 bits of its coin are below ars_coin (= lambda * 2^32).
+  unsigned long long ars_coin;
+  int ars_n_bins, ars_bin_samples;
+  const double* ars_cdf;             // [n_bins] cumulative distribution of the weighted part, built by the update kernel
+  const int* ars_bins;               // [n_bins][3] mocap step, first sample, width; then [n_steps] first bin of each step
+  unsigned* ars_inc;                 // [2][n_bins] episodes started / difficult in each bin since the last update
+  int* ars_env_bin;                  // [N] start bin of the running episode, -1 = not counted
+};
+
+// one-block kernel that folds a step's increments into the decayed counts and rebuilds the sampling tables
+struct AdaptiveRsiArgs {
+  int n_bins;
+  double rho;                        // decay per update (2^(-1/halflife); 1 = fold in without decay)
+  double lambda;                     // mixture weight of the weighted part (for prob)
+  const double* u;                   // [n_bins] probability of each bin under the reference's uniform draw
+  double* counts;                    // [2][n_bins] started, difficult
+  unsigned* inc;                     // [2][n_bins]
+  double* cdf;                       // [n_bins]
+  double* prob;                      // [n_bins] full mixture (1 - lambda) u + lambda q
 };
 
 }  // namespace drl

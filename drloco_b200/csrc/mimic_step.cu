@@ -339,11 +339,39 @@ __device__ __noinline__ bool floor_contact(const DevModel& M, ES& E, const LaneC
   return env_any(touch, L.emask);
 }
 
+// Failure-weighted RSI, weighted branch: a bin by inverse CDF over the weighted part of the mixture (binary search in
+// global memory; the table is a few KB and stays in L2), then a sample uniform within the bin.  h: the draw's coin
+// hash; its high 32 bits pick the bin, mix64(h) the sample.  Returns the bin.
+__device__ __noinline__ int ars_weighted_draw(const StepArgs& A, unsigned long long h, int& i_step, int& pos) {
+  const double x = (double)(h >> 32) * 0x1p-32;
+  int lo = 0, hi = A.ars_n_bins - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(A.ars_cdf + mid) > x) hi = mid;
+    else lo = mid + 1;
+  }
+  const int* bin = A.ars_bins + 3 * lo;
+  i_step = __ldg(bin);
+  pos = __ldg(bin + 1) + (int)(((mix64(h) & 0xFFFFFFFFull) * (unsigned long long)__ldg(bin + 2)) >> 32);
+  return lo;
+}
+
+// Failure-weighted RSI, episode end: lane 0 of an episode whose start was a random RSI draw counts it in its start bin
+__device__ __noinline__ void ars_count_episode(const StepArgs& A, int env, bool difficult) {
+  const int b = A.ars_env_bin[env];
+  if (b < 0) return;
+  atomicAdd(A.ars_inc + b, 1u);
+  if (difficult) atomicAdd(A.ars_inc + A.ars_n_bins + b, 1u);
+}
+
+// Returns the start bin of the failure-weighted RSI table for a random RSI draw while the option is on, else -1 (the
+// episode is not counted): deterministic inits, injected draws, playback.
 template <int NV, int G, class ES>
-__device__ __noinline__ void reset_env(const DevModel& M, const StepArgs& A, ES& E, const LaneConst& L,
-                                       const ChainLane& CL, int env, Cursor& c, float& q, float& v, float& dist,
-                                       float& zoff) {
+__device__ __noinline__ int reset_env(const DevModel& M, const StepArgs& A, ES& E, const LaneConst& L,
+                                      const ChainLane& CL, int env, Cursor& c, float& q, float& v, float& dist,
+                                      float& zoff) {
   const int l = L.l;
+  int start_bin = -1;
   c.ep_dur = 0;
   if (A.eval_mode || A.speed_profile != nullptr) {   // mimic_env.py:536-537; straight:237-265 / base:69-77
     if (M.cursor_mode == DRL_CURSOR_STEPWISE) {
@@ -363,8 +391,17 @@ __device__ __noinline__ void reset_env(const DevModel& M, const StepArgs& A, ES&
     c.flags &= ~(kFlagReadStep0 | kFlagDetEpisode);
     const unsigned long long gid = (unsigned long long)(M.env_id_offset + env);
     const unsigned long long r = mix64(mix64(M.seed ^ (gid * 0xD1342543DE82EF95ull)) + (unsigned long long)c.resets);
-    c.i_step = (int)(((r & 0xFFFFFFFFull) * (unsigned long long)M.n_steps) >> 32);
-    c.pos = (int)(((r >> 32) * (unsigned long long)A.step_len[c.i_step]) >> 32);
+    // failure-weighted RSI: with probability lambda (its own counter-based coin) the weighted draw replaces the
+    // uniform one, which otherwise stays the draw of r, bit for bit
+    const unsigned long long h = A.ars_coin ? mix64(r ^ 0x6A09E667F3BCC909ull) : 0ull;
+    if ((h & 0xFFFFFFFFull) < A.ars_coin) {
+      start_bin = ars_weighted_draw(A, h, c.i_step, c.pos);
+    } else {
+      c.i_step = (int)(((r & 0xFFFFFFFFull) * (unsigned long long)M.n_steps) >> 32);
+      c.pos = (int)(((r >> 32) * (unsigned long long)A.step_len[c.i_step]) >> 32);
+      if (A.ars_env_bin) start_bin = A.ars_bins[3 * A.ars_n_bins + c.i_step] + c.pos / A.ars_bin_samples;
+    }
+    if (A.playback) start_bin = -1;
   }
   c.resets += 1;
   c.rsi_step = c.i_step;
@@ -385,6 +422,7 @@ __device__ __noinline__ void reset_env(const DevModel& M, const StepArgs& A, ES&
   zoff = lowest;                               // refs.adjust_COM_Z_pos(lowest)
   cursor_next(M, A, c, dist);                  // mimic_env.py:568
   __syncwarp();
+  return start_bin;
 }
 
 // PD position servo of dof lane jd (MuJoCo <position kp kv>, actuator length gear*q, velocity gear*v): the actuator
@@ -454,7 +492,7 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     // VecEnv.reset(): (masked) reset of the episode state
     const bool want = live && (A.reset_mask == nullptr || A.reset_mask[env]);
     if (!__any_sync(kFull, want)) return;
-    reset_env<NV, G>(M, A, E, L, CL, env, c, q, v, dist, zoff);
+    const int start_bin = reset_env<NV, G>(M, A, E, L, CL, env, c, q, v, dist, zoff);
     float ph, dv;
     build_obs<G>(M, A, E, L, c, q, v, ph, dv);
     const bool left = M.mirror_policy && A.left_step[c.i_step];
@@ -468,6 +506,7 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
         if (A.ee_f) A.ee_f[2 * (size_t)env] = 1.f;
         si[kCurIstep] = c.i_step; si[kCurPos] = c.pos; si[kCurCount] = c.count; si[kCurEpDur] = 0;
         si[kCurRsiStep] = c.rsi_step; si[kCurNDet] = c.n_det; si[kCurResets] = c.resets; si[kCurFlags] = c.flags;
+        if (A.ars_env_bin) A.ars_env_bin[env] = start_bin;
       }
     }
     return;
@@ -759,13 +798,15 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
       A.ring_et_pos[slot] = c.pos;                                      // :104-107
       A.ring_difficult[slot] = (float)ep_len < ms[kMiscEpLenSm] * 0.75f ? 1 : 0;   // :123-124 (after the smoothing)
     }
+    // failure-weighted RSI: Monitor's difficult bit of the episode, counted in its start bin (not in playback)
+    if (A.ars_env_bin && !A.playback) ars_count_episode(A, env, (float)ep_len < ms[kMiscEpLenSm] * 0.75f);
   }
   c.flags = __shfl_sync(kFull, c.flags, 0, G);
   // ---- auto-reset (DummyVecEnv.step_wait), warp-uniform: both environments compute it, only `done` ones commit -----
   if (__any_sync(kFull, done)) {
     Cursor c2 = c;
     float q2 = q, v2 = v, dist2 = dist, zoff2 = zoff;
-    reset_env<NV, G>(M, A, E, L, CL, env, c2, q2, v2, dist2, zoff2);
+    const int start_bin = reset_env<NV, G>(M, A, E, L, CL, env, c2, q2, v2, dist2, zoff2);
     float ph, dv;
     build_obs<G>(M, A, E, L, c2, q2, v2, ph, dv);
     const bool left2 = M.mirror_policy && A.left_step[c2.i_step];
@@ -779,6 +820,7 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
       walked = 0.f; ep_ret = 0.f; ep_tor = 0.f;
       pos_rew = vel_rew = com_rew = 1.f;      // get_imitation_reward() inside reset_model (mimic_env.py:562)
       ee_rew = 1.f;
+      if (l == 0 && live && A.ars_env_bin) A.ars_env_bin[env] = start_bin;
     }
   }
   // ---- store -------------------------------------------------------------------------------------------------------
@@ -898,6 +940,48 @@ __global__ void running_rsi_kernel(const int* __restrict__ state_i, int* __restr
   out[i] = si[kCurEpDur] > 0 ? (int)((unsigned)si[kCurFlags] >> 16) : -1;
 }
 
+// Failure-weighted RSI table update, one block after every step kernel: decay the counts and add the step's integer
+// increments (x <- rho x + dx, rounded in that order), zero the increments, then build the distribution of the
+// weighted part, w_b = u_b (f_b + 1) / (s_b + 2), as a float64 CDF in a fixed order: every thread sums a contiguous
+// run of bins, thread 0 scans the runs' totals.  The result does not depend on how the step kernel's atomics landed.
+constexpr int kArsThreads = 256;
+__global__ void __launch_bounds__(kArsThreads) adaptive_rsi_update_kernel(const AdaptiveRsiArgs a) {
+  __shared__ double run_off[kArsThreads + 1];
+  const int n = a.n_bins, per = (n + kArsThreads - 1) / kArsThreads;
+  const int b0 = min(n, (int)threadIdx.x * per), b1 = min(n, b0 + per);
+  double* s = a.counts;
+  double* f = a.counts + n;
+  auto weight = [&](int b) { return a.u[b] * ((f[b] + 1.0) / (s[b] + 2.0)); };
+  double run = 0.0;
+  for (int b = b0; b < b1; b++) {
+    s[b] = __dadd_rn(__dmul_rn(a.rho, s[b]), (double)a.inc[b]);
+    f[b] = __dadd_rn(__dmul_rn(a.rho, f[b]), (double)a.inc[n + b]);
+    a.inc[b] = 0u;
+    a.inc[n + b] = 0u;
+    run += weight(b);
+  }
+  run_off[threadIdx.x] = run;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double acc = 0.0;
+    for (int t = 0; t < kArsThreads; t++) {
+      const double x = run_off[t];
+      run_off[t] = acc;
+      acc += x;
+    }
+    run_off[kArsThreads] = acc;
+  }
+  __syncthreads();
+  const double total = run_off[kArsThreads];
+  double acc = run_off[threadIdx.x];
+  for (int b = b0; b < b1; b++) {
+    const double w = weight(b);
+    acc += w;
+    a.cdf[b] = b == n - 1 ? 1.0 : acc / total;
+    a.prob[b] = (1.0 - a.lambda) * a.u[b] + a.lambda * (w / total);
+  }
+}
+
 // strided copies between the padded state rows and dense [N][nv] user tensors
 __global__ void state_copy_kernel(float* state_f, int* state_i, int* state_as, float* qpos, float* qvel, int* cursor,
                                   int n, int nv, int G, int to_state) {
@@ -1013,6 +1097,11 @@ bool topology_matches(int nv, int nb, const int* body_parent, const int* dof_bod
 
 cudaError_t launch_running_rsi(const int* state_i, int* out, int n, cudaStream_t st) {
   running_rsi_kernel<<<(n + 255) / 256, 256, 0, st>>>(state_i, out, n);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_adaptive_rsi_update(const AdaptiveRsiArgs& a, cudaStream_t st) {
+  adaptive_rsi_update_kernel<<<1, kArsThreads, 0, st>>>(a);
   return cudaGetLastError();
 }
 

@@ -144,6 +144,25 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+ADAPTIVE_RSI_BIN_STEPS = 20      # failure-weighted RSI: a bin spans this many control steps of reference motion
+
+
+def adaptive_rsi_bins(step_len, bin_samples: int) -> dict:
+    """Bin layout of the failure-weighted RSI table (drl_set_adaptive_rsi): runs of at most bin_samples consecutive
+    samples inside each mocap step, in step order.  Per bin: ``step``, ``first`` sample, ``width``, and ``u``, the
+    probability of the bin under the reference's RSI draw (a uniform step, then a uniform sample in it)."""
+    step_len = np.asarray(step_len, np.int64)
+    steps, first, width = [], [], []
+    for s, n in enumerate(step_len.tolist()):
+        f = np.arange(0, n, bin_samples)
+        steps.append(np.full(f.size, s))
+        first.append(f)
+        width.append(np.minimum(bin_samples, n - f))
+    steps, first, width = (np.concatenate(x).astype(np.int32) for x in (steps, first, width))
+    u = (1.0 / step_len.size) * width.astype(np.float64) / step_len[steps].astype(np.float64)
+    return dict(step=steps, first=first, width=width, u=u)
+
+
 class B200MimicVecEnv:
     """Batched MimicEnv.  Same attribute / method names as SB3's VecEnv (SURVEY.md §8b)."""
 
@@ -182,6 +201,14 @@ class B200MimicVecEnv:
             lib.check(self._lib.drl_set_contact_termination(self._handle, contact_body_mask(m)),
                       "drl_set_contact_termination")
         self._upload_mocap()
+        self._ars_bins = None
+        if self.cfg.adaptive_rsi > 0.0:
+            # failure-weighted RSI (EnvConfig.adaptive_rsi): bins of 20 control steps of reference motion
+            bin_samples = ADAPTIVE_RSI_BIN_STEPS * self.spec.mocap.increment
+            self._ars_bins = adaptive_rsi_bins(self.spec.mocap.step_len, bin_samples)
+            lib.check(self._lib.drl_set_adaptive_rsi(self._handle, float(self.cfg.adaptive_rsi),
+                                                     int(self.cfg.adaptive_rsi_halflife), bin_samples),
+                      "drl_set_adaptive_rsi")
         with torch.cuda.device(self.device):
             N, D = self.num_envs, self.obs_dim
             dev = self.device
@@ -295,7 +322,7 @@ class B200MimicVecEnv:
         with torch.cuda.device(self.device):
             lib.check(self._lib.drl_step(self._handle, _ptr(actions), _ptr(o["obs"]), _ptr(o["rew"]), _ptr(o["done"]),
                                          _ptr(o["terminal_obs"]), _ptr(ii), _ptr(ip), self._stream()), "drl_step")
-        self.launches += 1
+        self.launches += 2 if self._ars_bins is not None else 1    # + the failure-weighted RSI table update
         return o["obs"], o["rew"], o["done"]
 
     # ------------------------------------------------------------------ SB3 VecEnv API (numpy)
@@ -568,6 +595,36 @@ class B200MimicVecEnv:
         with torch.cuda.device(self.device):
             lib.check(self._lib.drl_set_det_init_counters(self._handle, buf.ctypes.data_as(C.c_void_p)),
                       "drl_set_det_init_counters")
+
+    def adaptive_rsi_table(self) -> dict:
+        """The failure-weighted RSI table (EnvConfig.adaptive_rsi): per bin its mocap ``step``, ``first`` sample and
+        ``width``, ``u`` (its probability under the reference's uniform draw), the decayed counts ``started`` and
+        ``difficult``, ``prob`` (the probability of the current mixture) and, per env, ``env_bin``, the start bin of
+        the running episode (-1: not counted).  Raises while the option is off."""
+        if self._ars_bins is None:
+            raise lib.DrlError("adaptive_rsi_table: the env was built with EnvConfig(adaptive_rsi=0)")
+        nb = len(self._ars_bins["u"])
+        with torch.cuda.device(self.device):
+            t = torch.zeros(3, nb, dtype=torch.float64, device=self.device)
+            eb = torch.zeros(self.num_envs, dtype=torch.int32, device=self.device)
+            lib.check(self._lib.drl_get_adaptive_rsi(self._handle, _ptr(t[0]), _ptr(t[1]), _ptr(t[2]), _ptr(eb),
+                                                     self._stream()), "drl_get_adaptive_rsi")
+            t, eb = t.cpu().numpy(), eb.cpu().numpy()
+        return dict(self._ars_bins, started=t[0], difficult=t[1], prob=t[2], env_bin=eb)
+
+    def set_adaptive_rsi_table(self, started, difficult) -> None:
+        """Restore the counts of adaptive_rsi_table() (e.g. when resuming a run); the sampling tables are rebuilt at
+        once.  float64 [n_bins] each, 0 <= difficult <= started.  Raises while the option is off."""
+        if self._ars_bins is None:
+            raise lib.DrlError("set_adaptive_rsi_table: the env was built with EnvConfig(adaptive_rsi=0)")
+        nb = len(self._ars_bins["u"])
+        s = np.ascontiguousarray(started, np.float64)
+        f = np.ascontiguousarray(difficult, np.float64)
+        if s.shape != (nb,) or f.shape != (nb,):
+            raise ValueError(f"set_adaptive_rsi_table: started and difficult must have shape ({nb},)")
+        with torch.cuda.device(self.device):
+            lib.check(self._lib.drl_set_adaptive_rsi_counts(self._handle, s.ctypes.data_as(C.c_void_p),
+                                                            f.ctypes.data_as(C.c_void_p)), "drl_set_adaptive_rsi_counts")
 
     def launch_info(self) -> dict:
         vals = [C.c_int32() for _ in range(4)]

@@ -293,6 +293,38 @@ int drl_set_contact_termination(DrlEnv* env, uint32_t body_mask);
  * was never enabled on this env. */
 int drl_get_contact_terminations(DrlEnv* env, int32_t* out, void* stream);
 
+/* Failure-weighted reference state initialisation (not in the reference, whose RSI draw is uniform: a uniform mocap
+ * step, then a uniform sample in it, straight:460-474 / base:79-85).  The mocap is cut into bins of at most bin_samples
+ * consecutive samples inside each step (bins never straddle steps), in step order.  Per bin b the env keeps two
+ * decayed float64 counts: s_b, episodes that started in b, and f_b, those of them that were "difficult" by Monitor's
+ * rule (ep_len < 0.75 * ep_len_smoothed after the smoothing update, monitor_wrapper.py:123-124).  After every
+ * drl_step a one-block kernel on the same stream applies x <- rho x + dx (rho = 2^(-1/halflife_steps)) and builds the
+ * weighted distribution q_b = u_b rate_b / sum(u rate), rate_b = (f_b + 1) / (s_b + 2), u_b = the probability of b
+ * under the uniform draw; an empty table gives q = u.  A random RSI draw tosses its own counter-based coin: with
+ * probability lambda it picks a bin from q and a sample uniform in the bin, otherwise it is the uniform draw, bit for
+ * bit.  Resets in step k sample the table as it stood after step k - 1; the update is deterministic (integer atomics
+ * for the increments, a fixed-order float64 pass for the rest).  Counted: episodes whose start was a random RSI draw
+ * (either branch).  Not counted: deterministic inits (evaluation mode, speed profile), injected draws, states set
+ * with drl_set_state, playback.  Each env (each rank of a sharded run) keeps its own table; nothing is exchanged.
+ * lambda = 0 turns it off (drl_step then enqueues one kernel, as without it); the tables are kept.  DRL_ERR_INVALID
+ * for lambda outside [0, 1], halflife_steps <= 0 or bin_samples <= 0; DRL_ERR_STATE before drl_upload_mocap.  The
+ * first enable for a mocap upload and bin width allocates a zeroed table and marks every running episode uncounted.
+ * While it is on, drl_upload_mocap returns DRL_ERR_STATE (the bins would go stale).  Synchronises the device (not for
+ * the stepping loop; a captured CUDA graph keeps the kernels and arguments it captured). */
+int drl_set_adaptive_rsi(DrlEnv* env, float lambda, int32_t halflife_steps, int32_t bin_samples);
+
+/* The table: started, difficult, prob (the full mixture (1 - lambda) u_b + lambda q_b): device float64 [n_bins];
+ * env_bin: device int32 [N], the start bin of every running episode (-1: not counted).  Each pointer is nullable.
+ * n_bins follows from the mocap step lengths and bin_samples as described above.  DRL_ERR_STATE if the option was
+ * never enabled on this env. */
+int drl_get_adaptive_rsi(DrlEnv* env, double* started, double* difficult, double* prob, int32_t* env_bin,
+                         void* stream);
+
+/* Overwrite the counts (HOST float64 [n_bins] each, 0 <= difficult <= started, finite), e.g. to resume a run, and
+ * rebuild the sampling tables; pending increments are dropped.  DRL_ERR_STATE if the option was never enabled,
+ * DRL_ERR_INVALID for a bad count.  Synchronises the device. */
+int drl_set_adaptive_rsi_counts(DrlEnv* env, const double* started, const double* difficult);
+
 /* MimicEnv.playback_ref_trajectories (mimic_env.py:265-282): while on, drl_step skips the physics and, after
  * refs.next(), sets qpos / qvel from the mocap (set_joint_kinematics_in_sim, mimic_env.py:284-293) before the
  * observation, reward and termination logic run.  A kinematic check of tables, cursor and ground shift: the imitation

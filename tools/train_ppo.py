@@ -8,6 +8,7 @@ Usage: python tools/train_ppo.py --envs 4096 --steps 16000000 --out gpurun_out/p
               on the CPU oracle stack: the comparison curve of BASELINE.json configs[4])
        python tools/train_ppo.py --actuation pd --kp 300 --kv 10 ...   (PD position servos instead of torque motors)
        python tools/train_ppo.py --contact-termination ...   (DeepMimic early termination on non-foot floor contact)
+       python tools/train_ppo.py --adaptive-rsi 0.5 ...   (failure-weighted reference state initialisation)
 """
 import argparse
 import json
@@ -45,6 +46,9 @@ def main():
     ap.add_argument("--contact-termination", action="store_true",
                     help="end an episode when a body other than the feet touches the floor "
                          "(EnvConfig.contact_termination)")
+    ap.add_argument("--adaptive-rsi", type=float, default=0.0, metavar="LAMBDA",
+                    help="share of random RSI draws weighted towards the mocap phases where episodes end early "
+                         "(EnvConfig.adaptive_rsi; 0 = off)")
     args = ap.parse_args()
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", "0"), ("WORLD_SIZE", "1"), ("LOCAL_RANK", "0")))
     if world > 1:
@@ -54,16 +58,16 @@ def main():
         torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local),
                                              timeout=datetime.timedelta(seconds=90))
     env_cfg = None
-    if args.actuation == "pd" or args.contact_termination:
+    if args.actuation == "pd" or args.contact_termination or args.adaptive_rsi > 0.0:
         if args.cpu_oracle:
-            ap.error("--actuation pd and --contact-termination run on the GPU env only")
+            ap.error("--actuation pd, --contact-termination and --adaptive-rsi run on the GPU env only")
         from drloco_b200.config import EnvConfig
         pd = dict()
         if args.actuation == "pd":
             gain = lambda g: None if g is None else (g[0] if len(g) == 1 else tuple(g))   # noqa: E731
             pd = dict(actuation="pd", pd_kp=gain(args.kp), pd_kv=gain(args.kv))
         env_cfg = EnvConfig(env_id="StraightMimicWalker", seed=33 + args.seed + 100 * rank,
-                            contact_termination=args.contact_termination, **pd)
+                            contact_termination=args.contact_termination, adaptive_rsi=args.adaptive_rsi, **pd)
     if args.cpu_oracle:
         from tools.oracle_tensor_env import OracleTensorEnv
         env = OracleTensorEnv("StraightMimicWalker", args.envs, seed=33 + args.seed)
@@ -111,6 +115,10 @@ def main():
         print("evaluation (deterministic policy, 20 deterministic inits):", json.dumps(ev), flush=True)
         ev2 = evaluate_walking(agent.policy, env, steady_state_counters=True)
         print("evaluation with the training-time desired-velocity counter (Q3):", json.dumps(ev2), flush=True)
+    ars = None
+    if args.adaptive_rsi > 0.0:
+        t = env.venv.adaptive_rsi_table()
+        ars = {k: t[k].tolist() for k in ("step", "first", "width", "u", "started", "difficult", "prob")}
     if rank == 0:
         os.makedirs(os.path.dirname(args.out) or ".", exist_ok=True)
         with open(args.out, "w") as f:
@@ -119,9 +127,9 @@ def main():
                        "env_steps_per_s_incl_learning": agent.num_timesteps / wall,
                        "replicas_bit_identical": lockstep,
                        "actuation": args.actuation, "pd_kp": args.kp, "pd_kv": args.kv,
-                       "contact_termination": args.contact_termination,
+                       "contact_termination": args.contact_termination, "adaptive_rsi": args.adaptive_rsi,
                        "config": {k: v for k, v in vars(cfg).items()}, "curve": agent.log, "evaluation": ev,
-                       "evaluation_steady_state_counters": ev2}, f, indent=1)
+                       "evaluation_steady_state_counters": ev2, "adaptive_rsi_table_at_end": ars}, f, indent=1)
         print("done: %.1f s, %.2e env-steps/s incl. learning, replicas bit-identical: %s"
               % (wall, agent.num_timesteps / wall, lockstep))
     if world > 1:
