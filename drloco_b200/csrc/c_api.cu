@@ -104,6 +104,15 @@ struct DrlEnv {
   int* ars_bins = nullptr;                // [n_bins][3] step, first, width; [n_steps] first bin of each step
   unsigned* ars_inc = nullptr;            // [2][n_bins]
   int* ars_env_bin = nullptr;             // [N]
+  // mocap library (drl_set_mocap_clips); one clip spanning the table after every drl_upload_mocap.  Device tables only
+  // while there is more than one clip.
+  std::vector<int> clip_first_h;          // [n_clips + 1]
+  std::vector<double> clip_weight_h;      // [n_clips] normalised
+  int* clip_first = nullptr;              // [n_clips + 1]
+  int* step_clip = nullptr;               // [n_steps]
+  double* clip_cdf = nullptr;             // [n_clips]
+  unsigned long long* clip_stats = nullptr;   // [n_clips][kClipStatCount]
+  ClipLibrary* d_clips = nullptr;         // the device struct StepArgs::clips points at
   // per-step statistics rows (one per thread block of the step kernel) + the ticket that elects the summing block
   double* cta_rows = nullptr;
   unsigned* cta_ticket = nullptr;
@@ -158,7 +167,7 @@ extern "C" int drl_destroy(DrlEnv* e) {
   free_state(e);
   // mocap tables, speed profile, debug dump
   void* ptrs[] = {e->ref, e->step_off, e->step_len, e->left_step, e->step_vel, e->step_last_comx, e->des_vel_prefix,
-                  e->speed_profile, e->debug};
+                  e->speed_profile, e->debug, e->clip_first, e->step_clip, e->clip_cdf, e->clip_stats, e->d_clips};
   for (void* p : ptrs)
     if (p) cudaFree(p);
   delete e;
@@ -420,8 +429,8 @@ extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t incremen
     return fail(DRL_ERR_STATE, "drl_upload_mocap: failure-weighted RSI is on (its bins would go stale); set lambda 0 first");
   if (cursor_mode != DRL_CURSOR_STEPWISE && cursor_mode != DRL_CURSOR_WRAP)
     return fail(DRL_ERR_INVALID, "drl_upload_mocap: unknown cursor mode");
-  if (cursor_mode == DRL_CURSOR_WRAP && (n_steps != 1 || !des_vel_prefix))
-    return fail(DRL_ERR_INVALID, "drl_upload_mocap: wrap mode needs one step and the desired-velocity prefix sums");
+  if (cursor_mode == DRL_CURSOR_WRAP && !des_vel_prefix)
+    return fail(DRL_ERR_INVALID, "drl_upload_mocap: wrap mode needs the desired-velocity prefix sums");
   for (int i = 0; i < n_steps; i++) {
     if (step_off[i] < 0 || step_len[i] <= 2 * increment || step_off[i] + step_len[i] > n_samples)
       return fail(DRL_ERR_INVALID, "drl_upload_mocap: step %d out of range or shorter than two increments", i);
@@ -440,7 +449,8 @@ extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t incremen
       upload(&e->step_last_comx, step_last_comx, n_steps))
     return fail(DRL_ERR_CUDA, "drl_upload_mocap: device copy failed");
   if (des_vel_prefix) {
-    if (upload(&e->des_vel_prefix, des_vel_prefix, (size_t)(n_samples + 1) * 2))
+    // one leading zero row per step: the prefix sums restart at every step (every clip of a wrap-mode library)
+    if (upload(&e->des_vel_prefix, des_vel_prefix, (size_t)(n_samples + n_steps) * 2))
       return fail(DRL_ERR_CUDA, "drl_upload_mocap: device copy failed");
   }
   DevModel& d = e->hm;
@@ -448,6 +458,16 @@ extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t incremen
   d.com_z_col = com_z_col; d.des_vel_window = des_vel_window;
   CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
   e->step_len_h.assign(step_len, step_len + n_steps);
+  // one clip spanning the table
+  if (e->clip_first) CUDA_TRY(cudaDeviceSynchronize());   // enqueued steps may still read the library tables
+  void** clip_ptrs[] = {(void**)&e->clip_first, (void**)&e->step_clip, (void**)&e->clip_cdf, (void**)&e->clip_stats,
+                        (void**)&e->d_clips};
+  for (void** p : clip_ptrs) {
+    if (*p) CUDA_TRY(cudaFree(*p));
+    *p = nullptr;
+  }
+  e->clip_first_h = {0, n_steps};
+  e->clip_weight_h = {1.0};
   e->mocap_gen++;
   e->have_mocap = true;
   return DRL_OK;
@@ -456,6 +476,84 @@ extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t incremen
 static int ready(DrlEnv* e, const char* who) {
   if (!e) return fail(DRL_ERR_INVALID, "%s: null env", who);
   if (!e->have_model || !e->have_mocap) return fail(DRL_ERR_STATE, "%s: model and mocap must be uploaded first", who);
+  if (e->hm.cursor_mode == DRL_CURSOR_WRAP && (int)e->clip_first_h.size() != e->hm.n_steps + 1)
+    return fail(DRL_ERR_STATE, "%s: a wrap-mode mocap of %d steps needs drl_set_mocap_clips with one clip per step", who,
+                e->hm.n_steps);
+  return DRL_OK;
+}
+
+extern "C" int drl_set_mocap_clips(DrlEnv* e, int32_t n_clips, const int32_t* clip_first_step, const double* clip_weight) {
+  if (!e || !clip_first_step || !clip_weight) return fail(DRL_ERR_INVALID, "drl_set_mocap_clips: null argument");
+  if (!e->have_model || !e->have_mocap) return fail(DRL_ERR_STATE, "drl_set_mocap_clips: upload the mocap first");
+  if (e->ars_lambda > 0.f)
+    return fail(DRL_ERR_STATE, "drl_set_mocap_clips: failure-weighted RSI is on (its bins would go stale); set lambda 0 first");
+  const int n_steps = e->hm.n_steps;
+  const bool wrap = e->hm.cursor_mode == DRL_CURSOR_WRAP;
+  if (n_clips < 1 || n_clips > n_steps) return fail(DRL_ERR_INVALID, "drl_set_mocap_clips: n_clips = %d outside [1, %d]",
+                                                    n_clips, n_steps);
+  if (clip_first_step[0] != 0 || clip_first_step[n_clips] != n_steps)
+    return fail(DRL_ERR_INVALID, "drl_set_mocap_clips: the clips must start at step 0 and end at step %d", n_steps);
+  double total = 0.0;
+  for (int k = 0; k < n_clips; k++) {
+    const int len = clip_first_step[k + 1] - clip_first_step[k];
+    // the reference's wrap (straight:330-333) goes to the clip's step 0 or 1
+    if (wrap ? len != 1 : len < 2)
+      return fail(DRL_ERR_INVALID, "drl_set_mocap_clips: clip %d has %d steps (%s)", k, len,
+                  wrap ? "a wrap-mode clip is one step" : "a stepwise clip needs at least 2");
+    if (!(isfinite(clip_weight[k]) && clip_weight[k] >= 0.0))
+      return fail(DRL_ERR_INVALID, "drl_set_mocap_clips: clip_weight[%d] = %g must be finite and >= 0", k, clip_weight[k]);
+    total += clip_weight[k];
+  }
+  if (!(total > 0.0 && isfinite(total)))
+    return fail(DRL_ERR_INVALID, "drl_set_mocap_clips: the clip weights must have a positive finite sum");
+  DeviceGuard guard__(e->cfg.device);
+  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the tables
+  void** ptrs[] = {(void**)&e->clip_first, (void**)&e->step_clip, (void**)&e->clip_cdf, (void**)&e->clip_stats,
+                   (void**)&e->d_clips};
+  for (void** p : ptrs) {
+    if (*p) CUDA_TRY(cudaFree(*p));
+    *p = nullptr;
+  }
+  e->clip_first_h.assign(clip_first_step, clip_first_step + n_clips + 1);
+  e->clip_weight_h.resize(n_clips);
+  for (int k = 0; k < n_clips; k++) e->clip_weight_h[k] = clip_weight[k] / total;
+  e->mocap_gen++;                             // the failure-weighted RSI bins weigh the clips: rebuild them
+  if (n_clips > 1) {
+    std::vector<int> step_clip(n_steps);
+    for (int k = 0; k < n_clips; k++)
+      for (int s = clip_first_step[k]; s < clip_first_step[k + 1]; s++) step_clip[s] = k;
+    // CDF of the clip draw; 1 from the last clip with a positive weight on, so that no rounding selects a trailing
+    // zero-weight clip
+    int last_pos = 0;
+    for (int k = 0; k < n_clips; k++)
+      if (clip_weight[k] > 0.0) last_pos = k;
+    std::vector<double> cdf(n_clips);
+    double acc = 0.0;
+    for (int k = 0; k < n_clips; k++) {
+      acc += clip_weight[k];
+      cdf[k] = k >= last_pos ? 1.0 : acc / total;
+    }
+    const size_t ns = (size_t)n_clips * kClipStatCount;
+    if (upload(&e->clip_first, clip_first_step, (size_t)n_clips + 1) || upload(&e->step_clip, step_clip.data(), n_steps) ||
+        upload(&e->clip_cdf, cdf.data(), n_clips))
+      return fail(DRL_ERR_CUDA, "drl_set_mocap_clips: device copy failed");
+    CUDA_TRY(cudaMalloc(&e->clip_stats, ns * sizeof(unsigned long long)));
+    CUDA_TRY(cudaMemset(e->clip_stats, 0, ns * sizeof(unsigned long long)));
+    ClipLibrary h;
+    h.n_clips = n_clips; h.clip_first = e->clip_first; h.step_clip = e->step_clip; h.clip_cdf = e->clip_cdf;
+    h.clip_stats = e->clip_stats;
+    CUDA_TRY(cudaMalloc(&e->d_clips, sizeof(ClipLibrary)));
+    CUDA_TRY(cudaMemcpy(e->d_clips, &h, sizeof(ClipLibrary), cudaMemcpyHostToDevice));
+  }
+  return DRL_OK;
+}
+
+extern "C" int drl_get_clip_stats(DrlEnv* e, int64_t* out, void* stream) {
+  if (!e || !out) return fail(DRL_ERR_INVALID, "drl_get_clip_stats: null argument");
+  if (!e->clip_stats) return fail(DRL_ERR_STATE, "drl_get_clip_stats: the mocap has a single clip");
+  DeviceGuard guard__(e->cfg.device);
+  const size_t n = (e->clip_first_h.size() - 1) * kClipStatCount;
+  CUDA_TRY(cudaMemcpyAsync(out, e->clip_stats, n * sizeof(int64_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -490,6 +588,7 @@ static StepArgs make_args(DrlEnv* e) {
     a.ars_n_bins = e->ars_n_bins; a.ars_bin_samples = e->ars_bin_samples;
     a.ars_cdf = e->ars_cdf; a.ars_bins = e->ars_bins; a.ars_inc = e->ars_inc; a.ars_env_bin = e->ars_env_bin;
   }
+  a.clips = e->d_clips;
   a.vn_ret = e->vn_ret; a.vn_gamma = e->vn_gamma; a.packed = e->vn_packed;
   if (e->playback) a.frame_skip = 0;
   a.debug = e->debug;
@@ -757,11 +856,18 @@ extern "C" int drl_get_contact_terminations(DrlEnv* e, int32_t* out, void* strea
 // the bin layout of the failure-weighted RSI table for the current mocap: bins of at most bin_samples consecutive samples
 // inside each mocap step, in step order.  Fills bins ([n_bins][3] step, first, width, then [n_steps] first bin of each
 // step) and u (the probability of each bin under the reference's uniform draw).
-static void ars_layout(const std::vector<int>& step_len, int bin_samples, std::vector<int>& bins, std::vector<double>& u) {
+static void ars_layout(const std::vector<int>& step_len, const std::vector<int>& clip_first,
+                       const std::vector<double>& clip_weight, int bin_samples, std::vector<int>& bins,
+                       std::vector<double>& u) {
   bins.clear(); u.clear();
   std::vector<int> first_bin;
-  const double inv_steps = 1.0 / (double)step_len.size();
+  size_t k = 0;                               // clip of step s: a step of clip k is drawn with weight_k / steps_k
+  double inv_steps = 0.0;
   for (size_t s = 0; s < step_len.size(); s++) {
+    if (s == 0 || (int)s == clip_first[k + 1]) {
+      if (s != 0) k++;
+      inv_steps = clip_weight[k] / (double)(clip_first[k + 1] - clip_first[k]);
+    }
     first_bin.push_back((int)u.size());
     for (int p = 0; p < step_len[s]; p += bin_samples) {
       const int w = step_len[s] - p < bin_samples ? step_len[s] - p : bin_samples;
@@ -786,7 +892,7 @@ extern "C" int drl_set_adaptive_rsi(DrlEnv* e, float lambda, int32_t halflife_st
     // first enable for this mocap and bin width: a new, empty table; every running episode is uncounted
     std::vector<int> bins;
     std::vector<double> u;
-    ars_layout(e->step_len_h, bin_samples, bins, u);
+    ars_layout(e->step_len_h, e->clip_first_h, e->clip_weight_h, bin_samples, bins, u);
     const size_t nb = u.size(), N = (size_t)e->cfg.num_envs;
     void** ptrs[] = {(void**)&e->ars_counts, (void**)&e->ars_u, (void**)&e->ars_cdf, (void**)&e->ars_prob,
                      (void**)&e->ars_bins, (void**)&e->ars_inc, (void**)&e->ars_env_bin};

@@ -92,6 +92,16 @@ constexpr int kCurIstep = 0, kCurPos = 1, kCurCount = 2, kCurEpDur = 3, kCurRsiS
 constexpr int kCurCount8 = 8;
 constexpr int kStatGroup = 16;        // blocks per group in the step kernel's two-level statistics sum
 
+// A mocap library in global memory (drl_set_mocap_clips): clips are runs of consecutive mocap steps; an episode never
+// leaves the clip it started in.
+struct ClipLibrary {
+  int n_clips;
+  const int* clip_first;             // [n_clips + 1] first mocap step of each clip, then n_steps
+  const int* step_clip;              // [n_steps] clip of each mocap step
+  const double* clip_cdf;            // [n_clips] cumulative distribution of the RSI clip draw
+  unsigned long long* clip_stats;    // [n_clips][kClipStatCount] episode counts by start clip
+};
+
 struct StepArgs {
   const DevModel* model;
   int num_envs;
@@ -108,7 +118,7 @@ struct StepArgs {
   const unsigned char* left_step;
   const float* step_vel;
   const float* step_last_comx;
-  const double* des_vel_prefix;      // [n_samples+1][2] or null (float64 prefix sums)
+  const double* des_vel_prefix;      // [n_samples+n_steps][2] or null (float64 prefix sums, restarting at every step)
   // io
   const float* actions;              // [N][act_dim]
   float* obs;                        // [N][obs_dim]
@@ -156,7 +166,14 @@ struct StepArgs {
   const int* ars_bins;               // [n_bins][3] mocap step, first sample, width; then [n_steps] first bin of each step
   unsigned* ars_inc;                 // [2][n_bins] episodes started / difficult in each bin since the last update
   int* ars_env_bin;                  // [N] start bin of the running episode, -1 = not counted
+  // mocap library (drl_set_mocap_clips), null with one clip.  Behind one pointer so that the parameter block, which
+  // the kernel copies to its stack, grows by 8 bytes only.
+  const ClipLibrary* clips;
 };
+
+// per-clip episode counters (drl_get_clip_stats)
+constexpr int kClipEpisodes = 0, kClipLenSum = 1, kClipFalls = 2, kClipTimeouts = 3, kClipBlowups = 4;
+constexpr int kClipStatCount = 5;
 
 // one-block kernel that folds a step's increments into the decayed counts and rebuilds the sampling tables
 struct AdaptiveRsiArgs {

@@ -47,15 +47,26 @@ constexpr int kFlagReadStep0 = 4, kFlagDetEpisode = 8;
 __device__ __forceinline__ int data_step(const Cursor& c) { return (c.flags & kFlagReadStep0) ? 0 : c.i_step; }
 __device__ __forceinline__ int shift_step(const Cursor& c) { return (c.flags & kFlagDetEpisode) ? 0 : c.rsi_step; }
 
-// StraightWalkingTrajectories.next (straight:141-159, :322-348) / BaseReferenceTrajectories.next (base:95-103)
+// mocap library (A.clips != null): first and last mocap step of the clip that holds step s
+__device__ __forceinline__ int clip_bounds(const ClipLibrary* L, int s, int& last) {
+  const int* first = L->clip_first;
+  const int k = __ldg(L->step_clip + s);
+  last = __ldg(first + k + 1) - 1;
+  return __ldg(first + k);
+}
+
+// StraightWalkingTrajectories.next (straight:141-159, :322-348) / BaseReferenceTrajectories.next (base:95-103).
+// Library: the reference's wrap rule applies per clip, so an episode stays in the clip it started in.
 __device__ __forceinline__ void cursor_next(const DevModel& M, const StepArgs& A, Cursor& c, float& dist) {
   const int len = A.step_len[data_step(c)];
   c.pos += M.increment;
   if (M.cursor_mode == DRL_CURSOR_STEPWISE) {
     const int dif = c.pos - len + 1;
     if (dif > 0) {
-      if (c.i_step >= M.n_steps - 1) {
-        c.i_step = A.left_step[c.i_step] ? 0 : 1;
+      int first = 0, last = M.n_steps - 1;
+      if (A.clips) first = clip_bounds(A.clips, c.i_step, last);
+      if (c.i_step >= last) {
+        c.i_step = first + (A.left_step[c.i_step] ? 0 : 1);
       } else {
         c.i_step += 1;
         c.count += 1;
@@ -199,17 +210,22 @@ __device__ __forceinline__ void desired_velocity(const DevModel& M, const StepAr
     d0 = A.speed_profile[c.ep_dur % A.speed_profile_len];
   } else if (M.cursor_mode == DRL_CURSOR_STEPWISE) {
     int idx = c.i_step - c.count + 1;
-    d0 = A.step_vel[idx < 0 ? 0 : idx];
+    int lo = 0;                                // library: clamped at the first step of the episode's clip
+    if (A.clips) { int last; lo = clip_bounds(A.clips, c.i_step, last); }
+    d0 = A.step_vel[idx < lo ? lo : idx];
   } else {
-    const int len = A.step_len[0];
+    // library: i_step is the clip; its prefix sums start at row step_off + clip (one leading zero row per clip)
+    int len = A.step_len[0];
+    const double* pre = A.des_vel_prefix;
+    if (A.clips) { len = A.step_len[c.i_step]; pre += 2 * (A.step_off[c.i_step] + c.i_step); }
     int end = c.pos + M.des_vel_window;
     if (end > len - 1) end = len - 1;
     const int n = end - c.pos;
     if (n <= 0) {
       d0 = d1 = nanf("");   // mean of an empty slice (Q23)
     } else {
-      d0 = (float)((A.des_vel_prefix[2 * end] - A.des_vel_prefix[2 * c.pos]) / (double)n);
-      d1 = (float)((A.des_vel_prefix[2 * end + 1] - A.des_vel_prefix[2 * c.pos + 1]) / (double)n);
+      d0 = (float)((pre[2 * end] - pre[2 * c.pos]) / (double)n);
+      d1 = (float)((pre[2 * end + 1] - pre[2 * c.pos + 1]) / (double)n);
     }
   }
 }
@@ -364,6 +380,30 @@ __device__ __noinline__ void ars_count_episode(const StepArgs& A, int env, bool 
   if (difficult) atomicAdd(A.ars_inc + A.ars_n_bins + b, 1u);
 }
 
+// Mocap library, random RSI draw: a clip with probability clip_weight / sum (inverse CDF, binary search in global
+// memory) from an independent hash of the draw r.  Returns the clip's first step, n_steps: its number of steps.
+__device__ __noinline__ int clip_draw(const ClipLibrary* L, unsigned long long r, int& n_steps) {
+  const double x = (double)(mix64(r ^ 0x3C6EF372FE94F82Bull) >> 32) * 0x1p-32;
+  const double* cdf = L->clip_cdf;
+  int lo = 0, hi = L->n_clips - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(cdf + mid) > x) hi = mid;
+    else lo = mid + 1;
+  }
+  const int first = __ldg(L->clip_first + lo);
+  n_steps = __ldg(L->clip_first + lo + 1) - first;
+  return first;
+}
+
+// Mocap library, episode end: lane 0 counts the episode in the clip of its start step
+__device__ __noinline__ void clip_count_episode(const ClipLibrary* L, int rsi_step, int ep_len, int kind) {
+  unsigned long long* s = L->clip_stats + (size_t)__ldg(L->step_clip + rsi_step) * kClipStatCount;
+  atomicAdd(s + kClipEpisodes, 1ull);
+  atomicAdd(s + kClipLenSum, (unsigned long long)ep_len);
+  atomicAdd(s + kind, 1ull);
+}
+
 // Returns the start bin of the failure-weighted RSI table for a random RSI draw while the option is on, else -1 (the
 // episode is not counted): deterministic inits, injected draws, playback.
 template <int NV, int G, class ES>
@@ -385,7 +425,8 @@ __device__ __noinline__ int reset_env(const DevModel& M, const StepArgs& A, ES& 
     }
   } else if (A.inj_istep != nullptr && A.inj_pos != nullptr && A.inj_pos[env] >= 0) {
     c.flags &= ~(kFlagReadStep0 | kFlagDetEpisode);
-    c.i_step = M.cursor_mode == DRL_CURSOR_STEPWISE ? A.inj_istep[env] : 0;
+    // (wrap mode: the injected step is the clip of a library, and ignored with one clip)
+    c.i_step = (M.cursor_mode == DRL_CURSOR_STEPWISE || A.clips) ? A.inj_istep[env] : 0;
     c.pos = A.inj_pos[env];
   } else {                                     // straight:460-474 / base:79-85
     c.flags &= ~(kFlagReadStep0 | kFlagDetEpisode);
@@ -397,7 +438,10 @@ __device__ __noinline__ int reset_env(const DevModel& M, const StepArgs& A, ES& 
     if ((h & 0xFFFFFFFFull) < A.ars_coin) {
       start_bin = ars_weighted_draw(A, h, c.i_step, c.pos);
     } else {
-      c.i_step = (int)(((r & 0xFFFFFFFFull) * (unsigned long long)M.n_steps) >> 32);
+      // library: a weighted clip first, then the reference's draw inside it
+      int first = 0, n = M.n_steps;
+      if (A.clips) first = clip_draw(A.clips, r, n);
+      c.i_step = first + (int)(((r & 0xFFFFFFFFull) * (unsigned long long)n) >> 32);
       c.pos = (int)(((r >> 32) * (unsigned long long)A.step_len[c.i_step]) >> 32);
       if (A.ars_env_bin) start_bin = A.ars_bins[3 * A.ars_n_bins + c.i_step] + c.pos / A.ars_bin_samples;
     }
@@ -800,6 +844,9 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     }
     // failure-weighted RSI: Monitor's difficult bit of the episode, counted in its start bin (not in playback)
     if (A.ars_env_bin && !A.playback) ars_count_episode(A, env, (float)ep_len < ms[kMiscEpLenSm] * 0.75f);
+    // mocap library: the episode in the counters of the clip it started in, classified as the statistics above
+    if (A.clips)
+      clip_count_episode(A.clips, c.rsi_step, ep_len, bad ? kClipBlowups : (timeout ? kClipTimeouts : kClipFalls));
   }
   c.flags = __shfl_sync(kFull, c.flags, 0, G);
   // ---- auto-reset (DummyVecEnv.step_wait), warp-uniform: both environments compute it, only `done` ones commit -----

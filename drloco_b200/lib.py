@@ -47,6 +47,8 @@ PROTOTYPES = {
     "drl_set_adaptive_rsi": (C.c_int, [vp, f32, i32, i32]),
     "drl_get_adaptive_rsi": (C.c_int, [vp, vp, vp, vp, vp, vp]),
     "drl_set_adaptive_rsi_counts": (C.c_int, [vp, vp, vp]),
+    "drl_set_mocap_clips": (C.c_int, [vp, i32, vp, vp]),
+    "drl_get_clip_stats": (C.c_int, [vp, vp, vp]),
     "drl_launch_info": (C.c_int, [vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]),
     "drl_debug_set": (C.c_int, [vp, i32, i32, i32]),
     "drl_debug_read": (C.c_int, [vp, vp, i32]),

@@ -43,6 +43,16 @@ class MocapTables:
     des_vel_window: int = 0
     des_vel_rows: Optional[np.ndarray] = None     # float64 [2, n_samples] the velocity rows themselves (the oracle
                                                   # takes np.mean of the slice exactly like loco3d:62-68)
+    # mocap library (concat_tables): clip k = steps [clip_first_step[k], clip_first_step[k + 1]), drawn at RSI with
+    # probability clip_weight[k]; a single recording is one clip of weight 1
+    clip_first_step: Optional[np.ndarray] = None  # int32 [n_clips + 1]
+    clip_weight: Optional[np.ndarray] = None      # float64 [n_clips], sums to 1
+
+    def __post_init__(self):
+        if self.clip_first_step is None:
+            self.clip_first_step = np.array([0, self.n_steps], np.int32)
+        if self.clip_weight is None:
+            self.clip_weight = np.ones(1)
 
     @property
     def n_steps(self) -> int:
@@ -51,6 +61,63 @@ class MocapTables:
     @property
     def n_samples(self) -> int:
         return int(self.ref.shape[0])
+
+    @property
+    def n_clips(self) -> int:
+        return int(self.clip_first_step.shape[0]) - 1
+
+
+def clip_weights(weights, n_samples) -> np.ndarray:
+    """Normalised RSI clip weights: ``weights`` (finite, >= 0, positive sum, one per clip), or None for weights
+    proportional to the clips' sample counts ``n_samples``."""
+    n_samples = np.asarray(n_samples, np.float64)
+    w = n_samples if weights is None else np.asarray(weights, np.float64).reshape(-1)
+    if w.shape != n_samples.shape:
+        raise ValueError(f"clip_weights: need one weight per clip ({n_samples.size}), got {w.size}")
+    if not np.all(np.isfinite(w)) or np.any(w < 0) or not w.sum() > 0:
+        raise ValueError(f"clip_weights must be finite and >= 0 with a positive sum, got {w.tolist()}")
+    return w / np.add.accumulate(w)[-1]          # summed in order, as drl_set_mocap_clips does
+
+
+def concat_tables(clips: Sequence[MocapTables], weights=None) -> MocapTables:
+    """A mocap library: the single-recording tables ``clips`` one after the other.  Step offsets are shifted by the
+    samples before each clip; the per-step tables and, in wrap mode, the desired-velocity prefix sums (which restart at
+    every clip) and rows are concatenated.  ``weights``: see clip_weights.  Every clip keeps the row map it was compiled
+    with (a 38-row and a 40-row straight-walking file can share a library).  Raises for an empty list, a clip that is
+    itself a library, mixed cursor modes, increments, COM-Z columns, desired-velocity windows or widths, a
+    stepwise clip of fewer than 2 steps or a wrap-mode clip of other than 1 step."""
+    clips = list(clips)
+    if not clips:
+        raise ValueError("concat_tables: no clips")
+    t0 = clips[0]
+    for k, t in enumerate(clips):
+        if t.n_clips != 1:
+            raise ValueError(f"concat_tables: clip {k} is already a library of {t.n_clips} clips")
+        for name in ("cursor_mode", "increment", "com_z_col", "des_vel_window"):
+            if getattr(t, name) != getattr(t0, name):
+                raise ValueError(f"concat_tables: clip {k} has {name} {getattr(t, name)}, clip 0 has {getattr(t0, name)}")
+        if t.ref.shape[1] != t0.ref.shape[1]:
+            raise ValueError(f"concat_tables: clip {k} has {t.ref.shape[1]} reference columns, clip 0 {t0.ref.shape[1]}")
+        if t.cursor_mode == CURSOR_STEPWISE and t.n_steps < 2:
+            raise ValueError(f"concat_tables: clip {k} has {t.n_steps} steps; the per-clip wrap "
+                             "(straight_walk_trajecs.py:330-333) needs at least 2")
+        if t.cursor_mode == CURSOR_WRAP and t.n_steps != 1:
+            raise ValueError(f"concat_tables: wrap-mode clip {k} has {t.n_steps} steps, not 1")
+    n_samples = np.array([t.n_samples for t in clips], np.int64)
+    sample0 = np.concatenate([[0], np.cumsum(n_samples)[:-1]])
+    wrap = t0.cursor_mode == CURSOR_WRAP
+    return MocapTables(
+        cursor_mode=t0.cursor_mode, increment=t0.increment, ref=np.concatenate([t.ref for t in clips]),
+        step_off=np.concatenate([t.step_off + s0 for t, s0 in zip(clips, sample0)]).astype(np.int32),
+        step_len=np.concatenate([t.step_len for t in clips]).astype(np.int32),
+        left_step=np.concatenate([t.left_step for t in clips]).astype(np.uint8),
+        step_vel=np.concatenate([t.step_vel for t in clips]),
+        step_last_comx=np.concatenate([t.step_last_comx for t in clips]), com_z_col=t0.com_z_col,
+        des_vel_prefix=np.concatenate([t.des_vel_prefix for t in clips]) if wrap else None,
+        des_vel_window=t0.des_vel_window,
+        des_vel_rows=np.concatenate([t.des_vel_rows for t in clips], axis=1) if wrap else None,
+        clip_first_step=np.concatenate([[0], np.cumsum([t.n_steps for t in clips])]).astype(np.int32),
+        clip_weight=clip_weights(weights, n_samples))
 
 
 class BaseReferenceTrajectories:

@@ -15,13 +15,14 @@ from __future__ import annotations
 import ctypes as C
 import os
 from collections.abc import Sequence
-from typing import Any, List, Optional, Tuple
+from typing import Any, List, Optional, Tuple, Union
 
 import numpy as np
 import torch
 
 from . import cabi, config as cfgm, lib
 from .model import contact_body_mask
+from .ref_trajecs.base_ref_trajecs import CURSOR_STEPWISE
 from .walkers import WalkerSpec, make_spec, speed_profile
 
 
@@ -144,14 +145,24 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+CLIP_STAT_NAMES = ("episodes", "ep_len_sum", "falls", "timeouts", "blowups")   # drl_get_clip_stats columns
 ADAPTIVE_RSI_BIN_STEPS = 20      # failure-weighted RSI: a bin spans this many control steps of reference motion
 
 
-def adaptive_rsi_bins(step_len, bin_samples: int) -> dict:
+def adaptive_rsi_bins(step_len, bin_samples: int, clip_first_step=None, clip_weight=None) -> dict:
     """Bin layout of the failure-weighted RSI table (drl_set_adaptive_rsi): runs of at most bin_samples consecutive
     samples inside each mocap step, in step order.  Per bin: ``step``, ``first`` sample, ``width``, and ``u``, the
-    probability of the bin under the reference's RSI draw (a uniform step, then a uniform sample in it)."""
+    probability of the bin under the reference's RSI draw (a uniform step, then a uniform sample in it).  Over a mocap
+    library (``clip_first_step`` [n_clips + 1], normalised ``clip_weight`` [n_clips]) the base draw picks clip c with
+    probability clip_weight[c] first: u = clip_weight[c] / steps of c * width / step length."""
     step_len = np.asarray(step_len, np.int64)
+    if clip_first_step is not None and len(clip_first_step) > 2:
+        cf = np.asarray(clip_first_step, np.int64)
+        w = np.asarray(clip_weight, np.float64)
+        w = w / np.add.accumulate(w)[-1]          # normalised again, in order, as drl_set_mocap_clips does
+        per_step = np.repeat(w / np.diff(cf), np.diff(cf))
+    else:
+        per_step = np.full(step_len.size, 1.0 / step_len.size)
     steps, first, width = [], [], []
     for s, n in enumerate(step_len.tolist()):
         f = np.arange(0, n, bin_samples)
@@ -159,7 +170,7 @@ def adaptive_rsi_bins(step_len, bin_samples: int) -> dict:
         first.append(f)
         width.append(np.minimum(bin_samples, n - f))
     steps, first, width = (np.concatenate(x).astype(np.int32) for x in (steps, first, width))
-    u = (1.0 / step_len.size) * width.astype(np.float64) / step_len[steps].astype(np.float64)
+    u = per_step[steps] * width.astype(np.float64) / step_len[steps].astype(np.float64)
     return dict(step=steps, first=first, width=width, u=u)
 
 
@@ -169,8 +180,9 @@ class B200MimicVecEnv:
     metadata = {"render.modes": []}
 
     def __init__(self, env_id: str = cfgm.STRAIGHT_WALKER, num_envs: int = 4096, device="cuda:0",
-                 seed: int = 33, cfg: Optional[cfgm.EnvConfig] = None, mocap_path: Optional[str] = None,
-                 env_id_offset: int = 0, lanes_per_env: int = 0, spec: Optional[WalkerSpec] = None):
+                 seed: int = 33, cfg: Optional[cfgm.EnvConfig] = None,
+                 mocap_path: Union[None, str, Sequence[Optional[str]]] = None, env_id_offset: int = 0,
+                 lanes_per_env: int = 0, spec: Optional[WalkerSpec] = None, clip_weights=None):
         self._lib = lib.load()                       # raises when the CUDA library is missing
         if not torch.cuda.is_available():
             raise lib.DrlError("drloco_b200 needs a CUDA device (there is no CPU path)")
@@ -178,7 +190,8 @@ class B200MimicVecEnv:
         if self.device.type != "cuda":
             raise lib.DrlError(f"device must be a CUDA device, got {device}")
         self.cfg = cfg or (spec.cfg if spec is not None else cfgm.EnvConfig(env_id=env_id, seed=seed))
-        self.spec = spec or make_spec(self.cfg, mocap_path)
+        # mocap_path: one recording or a library of them (make_spec), clip_weights: the library's RSI clip weights
+        self.spec = spec or make_spec(self.cfg, mocap_path, clip_weights)
         self.num_envs = int(num_envs)
         self.obs_dim, self.act_dim = self.spec.obs_dim, self.spec.act_dim
         m = self.spec.model
@@ -205,7 +218,8 @@ class B200MimicVecEnv:
         if self.cfg.adaptive_rsi > 0.0:
             # failure-weighted RSI (EnvConfig.adaptive_rsi): bins of 20 control steps of reference motion
             bin_samples = ADAPTIVE_RSI_BIN_STEPS * self.spec.mocap.increment
-            self._ars_bins = adaptive_rsi_bins(self.spec.mocap.step_len, bin_samples)
+            t = self.spec.mocap
+            self._ars_bins = adaptive_rsi_bins(t.step_len, bin_samples, t.clip_first_step, t.clip_weight)
             lib.check(self._lib.drl_set_adaptive_rsi(self._handle, float(self.cfg.adaptive_rsi),
                                                      int(self.cfg.adaptive_rsi_halflife), bin_samples),
                       "drl_set_adaptive_rsi")
@@ -283,6 +297,10 @@ class B200MimicVecEnv:
                                              p(arrs["off"]), p(arrs["ln"]), p(arrs["left"]), p(arrs["vel"]),
                                              p(arrs["lastx"]), t.n_steps, t.com_z_col, p(pre), t.des_vel_window),
                   "drl_upload_mocap")
+        if t.n_clips > 1:
+            first = np.ascontiguousarray(t.clip_first_step, np.int32)
+            w = np.ascontiguousarray(t.clip_weight, np.float64)
+            lib.check(self._lib.drl_set_mocap_clips(self._handle, t.n_clips, p(first), p(w)), "drl_set_mocap_clips")
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
@@ -516,6 +534,7 @@ class B200MimicVecEnv:
         idx = self._indices(indices)
         self._config_epoch += 1
         if method_name == "activate_evaluation":             # mimic_env.py:245
+            self._check_deterministic_inits("activate_evaluation")
             lib.check(self._lib.drl_set_eval_mode(self._handle, 1), "drl_set_eval_mode")
             return [None] * len(idx)
         if method_name == "activate_speed_control":          # mimic_env.py:298-327
@@ -535,6 +554,8 @@ class B200MimicVecEnv:
         its only caller and is off by default, Q26); the evident intent - obs[des_vel] = profile value - is what runs
         here.  An empty ``speeds`` switches speed control off (not in the reference)."""
         self._config_epoch += 1
+        if len(speeds):
+            self._check_deterministic_inits("activate_speed_control")
         prof = speed_profile(speeds, speed_profile_duration, self.cfg.ctrl_freq) if len(speeds) else \
             np.zeros(0, np.float32)
         self.desired_walking_speed_trajectory = prof
@@ -542,6 +563,38 @@ class B200MimicVecEnv:
         with torch.cuda.device(self.device):
             lib.check(self._lib.drl_set_speed_profile(self._handle, buf.ctypes.data_as(C.c_void_p) if buf.size else None,
                                                       int(buf.size)), "drl_set_speed_profile")
+
+    def _check_deterministic_inits(self, who: str) -> None:
+        """Deterministic inits start from the first eval_n_times steps of clip 0 (straight_walk_trajecs.py:237-265):
+        over a walker3d library they must not run into the next clip."""
+        t = self.spec.mocap
+        n0 = int(t.clip_first_step[1])
+        if t.n_clips > 1 and t.cursor_mode == CURSOR_STEPWISE and n0 < self.cfg.eval_n_times:
+            raise ValueError(f"{who}: clip 0 of the mocap library has {n0} steps, fewer than "
+                             f"eval_n_times = {self.cfg.eval_n_times}")
+
+    def mocap_clips(self) -> List[dict]:
+        """The clips of the mocap: per clip its ``path`` (None: the walker's default recording), ``first_step``,
+        ``steps``, ``samples`` and normalised RSI ``weight``.  A single recording is one clip of weight 1."""
+        t = self.spec.mocap
+        out = []
+        for k in range(t.n_clips):
+            a, b = int(t.clip_first_step[k]), int(t.clip_first_step[k + 1])
+            out.append(dict(path=self.spec.mocap_paths[k], first_step=a, steps=b - a,
+                            samples=int(t.step_len[a:b].sum()), weight=float(t.clip_weight[k])))
+        return out
+
+    def clip_stats(self) -> dict:
+        """Per-clip episode counts of a mocap library, by the clip each episode started in, since the env was built:
+        int64 [n_clips] arrays ``episodes``, ``ep_len_sum``, ``falls`` (every terminal step that is neither a timeout
+        nor a blow-up), ``timeouts`` and ``blowups``.  Exact, per env (per rank).  Raises with a single clip."""
+        if self.spec.mocap.n_clips < 2:
+            raise lib.DrlError("clip_stats: the env was built with a single mocap clip")
+        with torch.cuda.device(self.device):
+            out = torch.zeros(self.spec.mocap.n_clips, len(CLIP_STAT_NAMES), dtype=torch.int64, device=self.device)
+            lib.check(self._lib.drl_get_clip_stats(self._handle, _ptr(out), self._stream()), "drl_get_clip_stats")
+            out = out.cpu().numpy()
+        return {name: out[:, k].copy() for k, name in enumerate(CLIP_STAT_NAMES)}
 
     def set_playback(self, on: bool = True) -> None:
         """kinematic playback mode (mimic_env.py:265-293): `step` skips the physics and sets qpos/qvel from the mocap

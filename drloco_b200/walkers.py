@@ -5,7 +5,7 @@ Mirror of reference drloco/mujoco/mimic_walker3d.py, mimic_walker_165cm_65kg.py 
 from __future__ import annotations
 
 import dataclasses
-from typing import List, Optional
+from typing import List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
@@ -13,7 +13,7 @@ from . import config as cfgm
 from .model import WalkerModel, get_model
 from .ref_trajecs import straight_walk_trajecs as sw
 from .ref_trajecs import loco3d_trajecs as l3
-from .ref_trajecs.base_ref_trajecs import MocapTables
+from .ref_trajecs.base_ref_trajecs import MocapTables, clip_weights as _clip_weights, concat_tables
 
 
 def w3d_qpos_indices(n_rows: int = 38) -> List[int]:
@@ -56,6 +56,7 @@ class WalkerSpec:
     phase_from_cursor: bool                # mimic_env.py:416-419
     n_des_vel: int
     mirror: bool
+    mocap_paths: Tuple[Optional[str], ...] = (None,)   # the file of every clip (None: the walker's default recording)
 
     @property
     def obs_dim(self) -> int:
@@ -93,17 +94,39 @@ def speed_profile(speeds, speed_profile_duration, control_freq) -> np.ndarray:
     return np.concatenate([np.linspace(speeds[i], speeds[i + 1], region) for i in range(n_sections)])
 
 
-def make_spec(cfg: Optional[cfgm.EnvConfig] = None, mocap_path: Optional[str] = None) -> WalkerSpec:
-    """env id -> everything the device needs (reference drloco/mujoco/config.py:9-10 ``env_map``)."""
-    cfg = cfg or cfgm.EnvConfig()
-    model = get_model(cfg.env_id)
+def _compile_mocap(cfg: cfgm.EnvConfig, mocap_path: Optional[str]) -> MocapTables:
+    """One recording -> its tables (reference drloco/mujoco/config.py:9-10 ``env_map`` and the walkers' refs)."""
     if cfg.env_id == cfgm.STRAIGHT_WALKER:
         rows, _ = sw.load_steps(mocap_path or sw.PATH_CONSTANT_SPEED)
-        refs = sw.StraightWalkingTrajectories(w3d_qpos_indices(rows.shape[0]), w3d_qvel_indices(), path=mocap_path)
-        return WalkerSpec(cfg, model, refs.tables(), [0, 1, 2], [3, 4, 5], [6, 8, 10, 12], True, 1,
-                          cfg.is_mod(cfgm.MOD_MIRR_POLICY))
+        return sw.StraightWalkingTrajectories(w3d_qpos_indices(rows.shape[0]), w3d_qvel_indices(),
+                                              path=mocap_path).tables()
     if cfg.env_id == cfgm.WALKER_165:
-        refs = l3.Loco3dReferenceTrajectories(W165_QPOS_INDICES, W165_QVEL_INDICES, {}, path=mocap_path,
-                                              control_freq=cfg.ctrl_freq)
-        return WalkerSpec(cfg, model, refs.tables(), [0, 1, 2], [3, 4, 5], [9, 12, 14, 17], False, 2, False)
+        return l3.Loco3dReferenceTrajectories(W165_QPOS_INDICES, W165_QVEL_INDICES, {}, path=mocap_path,
+                                              control_freq=cfg.ctrl_freq).tables()
     raise KeyError(cfg.env_id)
+
+
+def make_spec(cfg: Optional[cfgm.EnvConfig] = None, mocap_path: Union[None, str, Sequence[Optional[str]]] = None,
+              clip_weights=None) -> WalkerSpec:
+    """env id -> everything the device needs (reference drloco/mujoco/config.py:9-10 ``env_map``).
+
+    ``mocap_path``: one recording (None: the walker's default), or a sequence of them, a mocap library whose clips an
+    episode never leaves (concat_tables).  ``clip_weights``: one RSI weight per clip (finite, >= 0, positive sum);
+    None weighs the clips by their sample counts.  A library of one path is the single recording, bit for bit."""
+    cfg = cfg or cfgm.EnvConfig()
+    model = get_model(cfg.env_id)
+    paths = (mocap_path,) if mocap_path is None or isinstance(mocap_path, str) else tuple(mocap_path)
+    if not paths:
+        raise ValueError("make_spec: mocap_path is an empty sequence")
+    if cfg.env_id not in (cfgm.STRAIGHT_WALKER, cfgm.WALKER_165):
+        raise KeyError(cfg.env_id)
+    clips = [_compile_mocap(cfg, p) for p in paths]
+    if len(clips) == 1:
+        _clip_weights(clip_weights, [clips[0].n_samples])     # validated; one clip is always drawn
+        mocap = clips[0]
+    else:
+        mocap = concat_tables(clips, clip_weights)
+    if cfg.env_id == cfgm.STRAIGHT_WALKER:
+        return WalkerSpec(cfg, model, mocap, [0, 1, 2], [3, 4, 5], [6, 8, 10, 12], True, 1,
+                          cfg.is_mod(cfgm.MOD_MIRR_POLICY), paths)
+    return WalkerSpec(cfg, model, mocap, [0, 1, 2], [3, 4, 5], [9, 12, 14, 17], False, 2, False, paths)

@@ -149,7 +149,10 @@ int drl_upload_model(DrlEnv* env, const DrlWalkerModel* model);
 
 /* replaces BaseReferenceTrajectories._load_ref_trajecs (base_ref_trajecs.py:28, straight_walk_trajecs.py:304-320).
  * ref: host float64 [n_samples][2*nv] (qpos rows then qvel rows in model order); step tables host arrays of n_steps.
- * des_vel_prefix: host float64 [n_samples+1][2] or NULL (loco3d desired velocity, loco3d_trajecs.py:58-68). */
+ * des_vel_prefix: host float64 [n_samples+n_steps][2] or NULL (loco3d desired velocity, loco3d_trajecs.py:58-68): per
+ * step, a zero row and the running sums over its samples (one step: [n_samples+1][2]).  A wrap-mode mocap of more than
+ * one step is a library of one-step clips and needs drl_set_mocap_clips before it can be stepped.  Every upload makes
+ * the mocap one clip spanning the table. */
 int drl_upload_mocap(DrlEnv* env, int32_t cursor_mode, int32_t increment, const double* ref, int32_t n_samples,
                      const int32_t* step_off, const int32_t* step_len, const uint8_t* left_step,
                      const double* step_vel, const double* step_last_comx, int32_t n_steps, int32_t com_z_col,
@@ -324,6 +327,30 @@ int drl_get_adaptive_rsi(DrlEnv* env, double* started, double* difficult, double
  * rebuild the sampling tables; pending increments are dropped.  DRL_ERR_STATE if the option was never enabled,
  * DRL_ERR_INVALID for a bad count.  Synchronises the device. */
 int drl_set_adaptive_rsi_counts(DrlEnv* env, const double* started, const double* difficult);
+
+/* Mocap library (not in the reference, which imitates one recording): the uploaded table as n_clips clips of
+ * consecutive mocap steps, clip k = steps [clip_first_step[k], clip_first_step[k + 1]) (HOST int32 [n_clips + 1],
+ * starting at 0 and ending at n_steps).  An episode stays in the clip it started in:
+ *   - stepwise mode (walker3d): the last step of clip k wraps to its first step + (left ? 0 : 1) (straight:330-333 per
+ *     clip; a clip needs at least 2 steps), and the desired-velocity step i_step - count + 1 is clamped at the clip's
+ *     first step;
+ *   - wrap mode (loco3d): every clip is one step and i_step is the clip; the desired-velocity window stays in the clip.
+ * A random RSI draw picks clip k with probability clip_weight[k] / sum (HOST float64 [n_clips], finite, >= 0, positive
+ * sum; a zero weight is never drawn) from its own counter-based hash, then the reference's draw inside the clip.
+ * Evaluation mode and the speed profile use clip 0.  An injected inj_istep is the mocap step (stepwise) or the clip
+ * (wrap mode with more than one clip).  The failure-weighted RSI base probability of a bin becomes
+ * weight_k / steps_k * width / step_len.  With more than one clip the env keeps the per-clip episode counters of
+ * drl_get_clip_stats (zeroed here).  n_clips = 1 is the single-clip behaviour.  DRL_ERR_INVALID for clips that do not
+ * cover the table in order, a stepwise clip of fewer than 2 steps, a wrap-mode clip of other than 1 step or bad
+ * weights; DRL_ERR_STATE before drl_upload_mocap and while failure-weighted RSI is on (its bins would go stale).
+ * Synchronises the device (not for the stepping loop; a captured CUDA graph keeps the arguments it captured). */
+int drl_set_mocap_clips(DrlEnv* env, int32_t n_clips, const int32_t* clip_first_step, const double* clip_weight);
+
+/* Per-clip episode counters since drl_set_mocap_clips, by the clip of the episode's start step: out device int64
+ * [n_clips][5] = episodes, sum of episode lengths, falls (every terminal step that is neither a timeout nor a
+ * blow-up, so early and contact terminations too), timeouts, blow-ups.  Exact integer counts, per env (per rank).
+ * DRL_ERR_STATE while the mocap has a single clip. */
+int drl_get_clip_stats(DrlEnv* env, int64_t* out, void* stream);
 
 /* MimicEnv.playback_ref_trajectories (mimic_env.py:265-282): while on, drl_step skips the physics and, after
  * refs.next(), sets qpos / qvel from the mocap (set_joint_kinematics_in_sim, mimic_env.py:284-293) before the

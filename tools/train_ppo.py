@@ -9,6 +9,8 @@ Usage: python tools/train_ppo.py --envs 4096 --steps 16000000 --out gpurun_out/p
        python tools/train_ppo.py --actuation pd --kp 300 --kv 10 ...   (PD position servos instead of torque motors)
        python tools/train_ppo.py --contact-termination ...   (DeepMimic early termination on non-foot floor contact)
        python tools/train_ppo.py --adaptive-rsi 0.5 ...   (failure-weighted reference state initialisation)
+       python tools/train_ppo.py --mocap A.npz B.mat --clip-weights 1 2 ...   (a mocap library: several recordings,
+              per-clip episode counts logged with every row)
 """
 import argparse
 import json
@@ -49,6 +51,10 @@ def main():
     ap.add_argument("--adaptive-rsi", type=float, default=0.0, metavar="LAMBDA",
                     help="share of random RSI draws weighted towards the mocap phases where episodes end early "
                          "(EnvConfig.adaptive_rsi; 0 = off)")
+    ap.add_argument("--mocap", nargs="+", metavar="PATH",
+                    help="reference motion file(s); several make a mocap library (default: the shipped recording)")
+    ap.add_argument("--clip-weights", type=float, nargs="+", metavar="W",
+                    help="RSI weight of every --mocap clip (default: proportional to the clips' sample counts)")
     args = ap.parse_args()
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", "0"), ("WORLD_SIZE", "1"), ("LOCAL_RANK", "0")))
     if world > 1:
@@ -68,12 +74,16 @@ def main():
             pd = dict(actuation="pd", pd_kp=gain(args.kp), pd_kv=gain(args.kv))
         env_cfg = EnvConfig(env_id="StraightMimicWalker", seed=33 + args.seed + 100 * rank,
                             contact_termination=args.contact_termination, adaptive_rsi=args.adaptive_rsi, **pd)
+    library = args.mocap is not None and len(args.mocap) > 1
+    if (args.mocap or args.clip_weights) and args.cpu_oracle:
+        ap.error("--mocap and --clip-weights run on the GPU env only")
     if args.cpu_oracle:
         from tools.oracle_tensor_env import OracleTensorEnv
         env = OracleTensorEnv("StraightMimicWalker", args.envs, seed=33 + args.seed)
     else:
         env = vec_env("StraightMimicWalker", num_envs=args.envs, seed=33 + args.seed + 100 * rank, norm_rew=True,
-                      device=f"cuda:{local}", env_id_offset=rank * args.envs, cfg=env_cfg)
+                      device=f"cuda:{local}", env_id_offset=rank * args.envs, cfg=env_cfg,
+                      mocap_path=args.mocap if library else (args.mocap or [None])[0], clip_weights=args.clip_weights)
     cfg = PPOConfig(total_steps=args.steps)
     if args.reference_hypers:
         cfg.batch_size, cfg.minibatch_size = 4096 * 4, 512 * 4
@@ -85,6 +95,12 @@ def main():
     agent = PPO(env, cfg, seed=args.seed)
 
     def cb(a, row):
+        if library:
+            # per-clip episode counts of this rank since the start, by the clip each episode started in
+            cs = env.venv.clip_stats()
+            row = dict(row, clip_episodes=cs["episodes"].tolist(),
+                       clip_mean_ep_len=[round(float(s) / max(int(e), 1), 2) for s, e in zip(cs["ep_len_sum"],
+                                                                                               cs["episodes"])])
         if rank == 0:
             print(json.dumps({k: (round(v, 4) if isinstance(v, float) else v) for k, v in row.items()}), flush=True)
 
@@ -119,6 +135,10 @@ def main():
     if args.adaptive_rsi > 0.0:
         t = env.venv.adaptive_rsi_table()
         ars = {k: t[k].tolist() for k in ("step", "first", "width", "u", "started", "difficult", "prob")}
+    clips = None
+    if library:
+        cs = env.venv.clip_stats()
+        clips = [dict(c, **{k: int(cs[k][i]) for k in cs}) for i, c in enumerate(env.venv.mocap_clips())]
     if rank == 0:
         os.makedirs(os.path.dirname(args.out) or ".", exist_ok=True)
         with open(args.out, "w") as f:
@@ -129,7 +149,8 @@ def main():
                        "actuation": args.actuation, "pd_kp": args.kp, "pd_kv": args.kv,
                        "contact_termination": args.contact_termination, "adaptive_rsi": args.adaptive_rsi,
                        "config": {k: v for k, v in vars(cfg).items()}, "curve": agent.log, "evaluation": ev,
-                       "evaluation_steady_state_counters": ev2, "adaptive_rsi_table_at_end": ars}, f, indent=1)
+                       "evaluation_steady_state_counters": ev2, "adaptive_rsi_table_at_end": ars,
+                       "mocap_clips_at_end": clips}, f, indent=1)
         print("done: %.1f s, %.2e env-steps/s incl. learning, replicas bit-identical: %s"
               % (wall, agent.num_timesteps / wall, lockstep))
     if world > 1:
