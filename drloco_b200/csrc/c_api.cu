@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "../../include/drloco_b200.h"
+#include "dev_buf.h"
 #include "dev_model.h"
 
 namespace drl {
@@ -55,6 +56,59 @@ struct DeviceGuard {
   }
 };
 
+// The device buffers of an env, grouped by lifetime.  A call that replaces a group builds the new one complete in a
+// local, synchronises when enqueued steps may still read the old one, and only then moves it into the env together
+// with its host copies: a call that fails leaves the env as it was.
+struct StateBufs {                        // alloc_state: per-env state and statistics
+  DevBuf<float> state_f, extras_last;
+  DevBuf<int> state_i, state_as;
+  DevBuf<double> state_d, stats;
+  DevBuf<float> tor_hist, med_tor_sm;     // cfg.monitor_median_torque
+  DevBuf<float> ee_f;                     // cfg.ee_weight > 0: [N][2] last / smoothed ee_rew
+  DevBuf<double> ee_d;                    // cfg.ee_weight > 0: [N] lifetime sum of ee_rew
+  // per-step statistics rows (one per thread block of the step kernel) + the ticket that elects the summing block
+  DevBuf<double> cta_rows;
+  DevBuf<unsigned> cta_ticket;
+};
+
+struct RingBufs {                         // alloc_state: the episode ring
+  DevBuf<int> len, rsi_pos, et_pos;
+  DevBuf<float> ret;
+  DevBuf<unsigned char> difficult;
+  DevBuf<unsigned long long> head;
+};
+
+struct MocapBufs {                        // drl_upload_mocap
+  DevBuf<float> ref, step_vel, step_last_comx;
+  DevBuf<double> des_vel_prefix;          // float64: differences of long prefix sums lose ~1e-5 in float32
+  DevBuf<int> step_off, step_len;
+  DevBuf<unsigned char> left_step;
+  std::vector<int> step_len_h;            // host copy (the failure-weighted RSI bin layout is built from it)
+};
+
+// mocap library (drl_set_mocap_clips); one clip spanning the table after every drl_upload_mocap.  Device tables only
+// while there is more than one clip.
+struct ClipBufs {
+  std::vector<int> first_h;               // [n_clips + 1]
+  std::vector<double> weight_h;           // [n_clips] normalised
+  DevBuf<int> first;                      // [n_clips + 1]
+  DevBuf<int> step_clip;                  // [n_steps]
+  DevBuf<double> cdf;                     // [n_clips]
+  DevBuf<unsigned long long> stats;       // [n_clips][kClipStatCount]
+  DevBuf<ClipLibrary> lib;                // the device struct StepArgs::clips points at
+};
+
+// failure-weighted RSI (drl_set_adaptive_rsi): the table of one mocap and bin width, built when first enabled for them
+struct ArsBufs {
+  int gen = -1, bin_samples = 0;          // the mocap_gen and bin width it was built for
+  DevBuf<double> counts;                  // [2][n_bins] started, difficult
+  DevBuf<double> u, cdf, prob;            // [n_bins]
+  DevBuf<int> bins;                       // [n_bins][3] step, first, width; [n_steps] first bin of each step
+  DevBuf<unsigned> inc;                   // [2][n_bins]
+  DevBuf<int> env_bin;                    // [N]
+  int n_bins() const { return (int)u.size(); }
+};
+
 struct DrlEnv {
   DrlConfig cfg;
   DevModel hm;                 // host copy
@@ -62,60 +116,23 @@ struct DrlEnv {
   int G = 16, block = 128, nv = 0;
   int actuation = DRL_ACTUATION_TORQUE;   // drl_set_actuation
   double dof_range[kMaxDof][2];           // joint ranges in float64: the PD target map is computed from them
-  DevModel* d_model = nullptr;
-  float* state_f = nullptr;
-  int* state_i = nullptr;
-  int* state_as = nullptr;
-  double* state_d = nullptr;
-  float* extras_last = nullptr;
-  double* stats = nullptr;
-  float *ref = nullptr, *step_vel = nullptr, *step_last_comx = nullptr;
-  double* des_vel_prefix = nullptr;   // float64: differences of long prefix sums lose ~1e-5 in float32
-  int *step_off = nullptr, *step_len = nullptr;
-  unsigned char* left_step = nullptr;
-  int* ring_len = nullptr;
-  float* ring_ret = nullptr;
-  int *ring_rsi_pos = nullptr, *ring_et_pos = nullptr;
-  unsigned char* ring_difficult = nullptr;
-  unsigned long long* ring_head = nullptr;
+  DevBuf<DevModel> d_model;               // the model block hm is published to (publish_model)
+  StateBufs st;
+  RingBufs ring;
   int ring_cap = 1 << 16;
+  MocapBufs mocap;
+  int mocap_gen = 0;                      // bumped by every drl_upload_mocap and drl_set_mocap_clips
+  ClipBufs clips;
+  ArsBufs ars;
+  int ars_halflife = 0;
+  float ars_lambda = 0.f;                 // 0 = off
   int eval_mode = 0;
-  float* speed_profile = nullptr;
-  int speed_profile_len = 0;
+  DevBuf<float> speed_profile;            // drl_set_speed_profile; empty when off
   int playback = 0;
   int frame_skip_override = -1;
-  float* debug = nullptr;
-  float* tor_hist = nullptr;
-  float* med_tor_sm = nullptr;
-  // end-effector term (cfg.ee_weight > 0): last / smoothed ee_rew, lifetime sum
-  float* ee_f = nullptr;
-  double* ee_d = nullptr;
+  DevBuf<float> debug;                    // drl_debug_set
   // contact termination (drl_set_contact_termination): per-env episode count, allocated when first enabled
-  int* contact_et = nullptr;
-  // failure-weighted RSI (drl_set_adaptive_rsi): tables allocated when first enabled for a bin layout
-  std::vector<int> step_len_h;            // host copy of the mocap step lengths (the bin layout is built from them)
-  int mocap_gen = 0;                      // bumped by every drl_upload_mocap
-  int ars_gen = -1, ars_bin_samples = 0, ars_n_bins = 0, ars_halflife = 0;
-  float ars_lambda = 0.f;                 // 0 = off
-  double* ars_counts = nullptr;           // [2][n_bins] started, difficult
-  double* ars_u = nullptr;                // [n_bins]
-  double* ars_cdf = nullptr;              // [n_bins]
-  double* ars_prob = nullptr;             // [n_bins]
-  int* ars_bins = nullptr;                // [n_bins][3] step, first, width; [n_steps] first bin of each step
-  unsigned* ars_inc = nullptr;            // [2][n_bins]
-  int* ars_env_bin = nullptr;             // [N]
-  // mocap library (drl_set_mocap_clips); one clip spanning the table after every drl_upload_mocap.  Device tables only
-  // while there is more than one clip.
-  std::vector<int> clip_first_h;          // [n_clips + 1]
-  std::vector<double> clip_weight_h;      // [n_clips] normalised
-  int* clip_first = nullptr;              // [n_clips + 1]
-  int* step_clip = nullptr;               // [n_steps]
-  double* clip_cdf = nullptr;             // [n_clips]
-  unsigned long long* clip_stats = nullptr;   // [n_clips][kClipStatCount]
-  ClipLibrary* d_clips = nullptr;         // the device struct StepArgs::clips points at
-  // per-step statistics rows (one per thread block of the step kernel) + the ticket that elects the summing block
-  double* cta_rows = nullptr;
-  unsigned* cta_ticket = nullptr;
+  DevBuf<int> contact_et;
   // fused VecNormalize moments (drl_attach_vecnorm): borrowed device pointers
   float* vn_ret = nullptr;
   float vn_gamma = 0.f;
@@ -146,62 +163,39 @@ extern "C" int drl_create(const DrlConfig* cfg, DrlEnv** out) {
   return DRL_OK;
 }
 
-// the buffers of alloc_state; drl_destroy frees the rest
-static void free_state(DrlEnv* e) {
-  void** ptrs[] = {(void**)&e->d_model, (void**)&e->state_f, (void**)&e->state_i, (void**)&e->state_as,
-                   (void**)&e->state_d, (void**)&e->extras_last, (void**)&e->stats, (void**)&e->ring_len,
-                   (void**)&e->ring_ret, (void**)&e->ring_head, (void**)&e->ring_rsi_pos, (void**)&e->ring_et_pos,
-                   (void**)&e->ring_difficult, (void**)&e->cta_rows, (void**)&e->cta_ticket,
-                   (void**)&e->tor_hist, (void**)&e->med_tor_sm, (void**)&e->ee_f, (void**)&e->ee_d,
-                   (void**)&e->contact_et, (void**)&e->ars_counts, (void**)&e->ars_u, (void**)&e->ars_cdf,
-                   (void**)&e->ars_prob, (void**)&e->ars_bins, (void**)&e->ars_inc, (void**)&e->ars_env_bin};
-  for (void** p : ptrs) {
-    if (*p) cudaFree(*p);
-    *p = nullptr;
-  }
-}
-
 extern "C" int drl_destroy(DrlEnv* e) {
   if (!e) return DRL_OK;
   DeviceGuard guard__(e->cfg.device);
-  free_state(e);
-  // mocap tables, speed profile, debug dump
-  void* ptrs[] = {e->ref, e->step_off, e->step_len, e->left_step, e->step_vel, e->step_last_comx, e->des_vel_prefix,
-                  e->speed_profile, e->debug, e->clip_first, e->step_clip, e->clip_cdf, e->clip_stats, e->d_clips};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
   delete e;
   return DRL_OK;
 }
 
-// persistent per-env state; on failure the caller releases whatever was allocated (free_state)
+// persistent per-env state, statistics and episode ring, moved into the env once all of it is allocated
 static int alloc_state(DrlEnv* e, size_t N) {
-  CUDA_TRY(cudaMalloc(&e->d_model, sizeof(DevModel)));
-  CUDA_TRY(cudaMalloc(&e->state_f, N * 4 * e->G * sizeof(float)));
-  CUDA_TRY(cudaMalloc(&e->state_i, N * kCurCount8 * sizeof(int)));
-  CUDA_TRY(cudaMalloc(&e->state_as, N * e->G * sizeof(int)));
-  CUDA_TRY(cudaMemset(e->state_as, 0, N * e->G * sizeof(int)));
-  CUDA_TRY(cudaMalloc(&e->state_d, N * 4 * sizeof(double)));
-  CUDA_TRY(cudaMalloc(&e->extras_last, N * 16 * sizeof(float)));
-  CUDA_TRY(cudaMalloc(&e->stats, DRL_STATS_COUNT * sizeof(double)));
-  CUDA_TRY(cudaMalloc(&e->ring_len, e->ring_cap * sizeof(int)));
-  CUDA_TRY(cudaMalloc(&e->ring_ret, e->ring_cap * sizeof(float)));
-  CUDA_TRY(cudaMalloc(&e->ring_rsi_pos, e->ring_cap * sizeof(int)));
-  CUDA_TRY(cudaMalloc(&e->ring_et_pos, e->ring_cap * sizeof(int)));
-  CUDA_TRY(cudaMalloc(&e->ring_difficult, e->ring_cap));
-  CUDA_TRY(cudaMalloc(&e->ring_head, sizeof(unsigned long long)));
+  DevBuf<DevModel> model;
+  StateBufs s;
+  RingBufs r;
+  CUDA_TRY(model.alloc(1));
+  CUDA_TRY(s.state_f.zeros(N * 4 * e->G));
+  CUDA_TRY(s.state_i.alloc(N * kCurCount8));
+  CUDA_TRY(s.state_as.zeros(N * e->G));
+  CUDA_TRY(s.state_d.zeros(N * 4));
+  CUDA_TRY(s.extras_last.zeros(N * 16));
+  CUDA_TRY(s.stats.zeros(DRL_STATS_COUNT));
+  CUDA_TRY(r.len.alloc(e->ring_cap));
+  CUDA_TRY(r.ret.alloc(e->ring_cap));
+  CUDA_TRY(r.rsi_pos.alloc(e->ring_cap));
+  CUDA_TRY(r.et_pos.alloc(e->ring_cap));
+  CUDA_TRY(r.difficult.alloc(e->ring_cap));
+  CUDA_TRY(r.head.zeros(1));
   if (e->cfg.monitor_median_torque) {
     const size_t cap = (size_t)(e->cfg.ep_dur_max > 0 ? e->cfg.ep_dur_max : 1);
-    CUDA_TRY(cudaMalloc(&e->tor_hist, N * cap * sizeof(float)));
-    CUDA_TRY(cudaMemset(e->tor_hist, 0, N * cap * sizeof(float)));
-    CUDA_TRY(cudaMalloc(&e->med_tor_sm, N * sizeof(float)));
-    CUDA_TRY(cudaMemset(e->med_tor_sm, 0, N * sizeof(float)));
+    CUDA_TRY(s.tor_hist.zeros(N * cap));
+    CUDA_TRY(s.med_tor_sm.zeros(N));
   }
   if (e->cfg.ee_weight > 0.0) {
-    CUDA_TRY(cudaMalloc(&e->ee_f, N * 2 * sizeof(float)));
-    CUDA_TRY(cudaMemset(e->ee_f, 0, N * 2 * sizeof(float)));
-    CUDA_TRY(cudaMalloc(&e->ee_d, N * sizeof(double)));
-    CUDA_TRY(cudaMemset(e->ee_d, 0, N * sizeof(double)));
+    CUDA_TRY(s.ee_f.zeros(N * 2));
+    CUDA_TRY(s.ee_d.zeros(N));
   }
   {
     // the smallest CTA the library launches carries 32 / G environments
@@ -210,20 +204,24 @@ static int alloc_state(DrlEnv* e, size_t N) {
     // rows of the blocks, then one row per group of kStatGroup blocks (two-level fixed-order sum in the step kernel);
     // tickets: [0] counts finished groups, [1 + g] the finished blocks of group g
     const size_t max_groups = (max_blocks + kStatGroup - 1) / kStatGroup;
-    CUDA_TRY(cudaMalloc(&e->cta_rows, (max_blocks + max_groups) * row * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&e->cta_ticket, (1 + max_groups) * sizeof(unsigned)));
-    CUDA_TRY(cudaMemset(e->cta_ticket, 0, (1 + max_groups) * sizeof(unsigned)));
+    CUDA_TRY(s.cta_rows.alloc((max_blocks + max_groups) * row));
+    CUDA_TRY(s.cta_ticket.zeros(1 + max_groups));
   }
-  CUDA_TRY(cudaMemset(e->state_f, 0, N * 4 * e->G * sizeof(float)));
-  CUDA_TRY(cudaMemset(e->state_i, 0, N * kCurCount8 * sizeof(int)));
-  CUDA_TRY(cudaMemset(e->state_d, 0, N * 4 * sizeof(double)));
-  CUDA_TRY(cudaMemset(e->extras_last, 0, N * 16 * sizeof(float)));
-  CUDA_TRY(cudaMemset(e->stats, 0, DRL_STATS_COUNT * sizeof(double)));
-  CUDA_TRY(cudaMemset(e->ring_head, 0, sizeof(unsigned long long)));
   // count_steps_same_vel starts at 1 (straight_walk_trajecs.py:124)
   std::vector<int> init(N * kCurCount8, 0);
   for (size_t i = 0; i < N; i++) init[i * kCurCount8 + kCurCount] = 1;
-  CUDA_TRY(cudaMemcpy(e->state_i, init.data(), init.size() * sizeof(int), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(s.state_i.get(), init.data(), init.size() * sizeof(int), cudaMemcpyHostToDevice));
+  e->d_model = std::move(model);
+  e->st = std::move(s);
+  e->ring = std::move(r);
+  return DRL_OK;
+}
+
+// m becomes the model block on the device, then the env's host copy; the caller holds the env's DeviceGuard
+static int publish_model(DrlEnv* e, const DevModel& m) {
+  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the model block
+  CUDA_TRY(cudaMemcpy(e->d_model.get(), &m, sizeof(DevModel), cudaMemcpyHostToDevice));
+  e->hm = m;
   return DRL_OK;
 }
 
@@ -398,23 +396,11 @@ extern "C" int drl_upload_model(DrlEnv* e, const DrlWalkerModel* m) {
   DeviceGuard guard__(c.device);
   const int rc = alloc_state(e, (size_t)c.num_envs);
   if (rc != DRL_OK) {            // e.g. out of memory for a very large batch: leave the env without a model
-    free_state(e);
     (void)cudaGetLastError();     // a failed cudaMalloc also parks its code as the "last error": clear it
     return rc;
   }
   e->have_model = true;
-  if (e->have_mocap) CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
-  return DRL_OK;
-}
-
-template <typename T, typename S>
-static int upload(T** dst, const S* src, size_t n) {
-  std::vector<T> tmp(n);
-  for (size_t i = 0; i < n; i++) tmp[i] = (T)src[i];
-  if (*dst) cudaFree(*dst);
-  if (cudaMalloc(dst, n * sizeof(T)) != cudaSuccess) return -1;
-  if (cudaMemcpy(*dst, tmp.data(), n * sizeof(T), cudaMemcpyHostToDevice) != cudaSuccess) return -1;
-  return 0;
+  return e->have_mocap ? publish_model(e, e->hm) : DRL_OK;
 }
 
 extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t increment, const double* ref, int32_t n_samples,
@@ -443,31 +429,20 @@ extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t incremen
       padded[(size_t)t * 2 * G + j] = (float)ref[(size_t)t * 2 * nv + j];
       padded[(size_t)t * 2 * G + G + j] = (float)ref[(size_t)t * 2 * nv + nv + j];
     }
-  if (upload(&e->ref, padded.data(), padded.size())) return fail(DRL_ERR_CUDA, "drl_upload_mocap: device copy failed");
-  if (upload(&e->step_off, step_off, n_steps) || upload(&e->step_len, step_len, n_steps) ||
-      upload(&e->left_step, left_step, n_steps) || upload(&e->step_vel, step_vel, n_steps) ||
-      upload(&e->step_last_comx, step_last_comx, n_steps))
+  MocapBufs t;
+  // des_vel_prefix: one leading zero row per step (the prefix sums restart at every clip of a wrap-mode library)
+  if (t.ref.from_host(padded.data(), padded.size()) || t.step_off.from_host(step_off, n_steps) ||
+      t.step_len.from_host(step_len, n_steps) || t.left_step.from_host(left_step, n_steps) ||
+      t.step_vel.from_host(step_vel, n_steps) || t.step_last_comx.from_host(step_last_comx, n_steps) ||
+      (des_vel_prefix && t.des_vel_prefix.from_host(des_vel_prefix, (size_t)(n_samples + n_steps) * 2)))
     return fail(DRL_ERR_CUDA, "drl_upload_mocap: device copy failed");
-  if (des_vel_prefix) {
-    // one leading zero row per step: the prefix sums restart at every step (every clip of a wrap-mode library)
-    if (upload(&e->des_vel_prefix, des_vel_prefix, (size_t)(n_samples + n_steps) * 2))
-      return fail(DRL_ERR_CUDA, "drl_upload_mocap: device copy failed");
-  }
-  DevModel& d = e->hm;
+  t.step_len_h.assign(step_len, step_len + n_steps);
+  DevModel d = e->hm;
   d.cursor_mode = cursor_mode; d.increment = increment; d.n_steps = n_steps; d.n_samples = n_samples;
   d.com_z_col = com_z_col; d.des_vel_window = des_vel_window;
-  CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
-  e->step_len_h.assign(step_len, step_len + n_steps);
-  // one clip spanning the table
-  if (e->clip_first) CUDA_TRY(cudaDeviceSynchronize());   // enqueued steps may still read the library tables
-  void** clip_ptrs[] = {(void**)&e->clip_first, (void**)&e->step_clip, (void**)&e->clip_cdf, (void**)&e->clip_stats,
-                        (void**)&e->d_clips};
-  for (void** p : clip_ptrs) {
-    if (*p) CUDA_TRY(cudaFree(*p));
-    *p = nullptr;
-  }
-  e->clip_first_h = {0, n_steps};
-  e->clip_weight_h = {1.0};
+  if (const int rc = publish_model(e, d)) return rc;   // synchronises: enqueued steps may still read the old tables
+  e->mocap = std::move(t);
+  e->clips = ClipBufs{{0, n_steps}, {1.0}};    // one clip spanning the table
   e->mocap_gen++;
   e->have_mocap = true;
   return DRL_OK;
@@ -476,7 +451,7 @@ extern "C" int drl_upload_mocap(DrlEnv* e, int32_t cursor_mode, int32_t incremen
 static int ready(DrlEnv* e, const char* who) {
   if (!e) return fail(DRL_ERR_INVALID, "%s: null env", who);
   if (!e->have_model || !e->have_mocap) return fail(DRL_ERR_STATE, "%s: model and mocap must be uploaded first", who);
-  if (e->hm.cursor_mode == DRL_CURSOR_WRAP && (int)e->clip_first_h.size() != e->hm.n_steps + 1)
+  if (e->hm.cursor_mode == DRL_CURSOR_WRAP && (int)e->clips.first_h.size() != e->hm.n_steps + 1)
     return fail(DRL_ERR_STATE, "%s: a wrap-mode mocap of %d steps needs drl_set_mocap_clips with one clip per step", who,
                 e->hm.n_steps);
   return DRL_OK;
@@ -507,17 +482,10 @@ extern "C" int drl_set_mocap_clips(DrlEnv* e, int32_t n_clips, const int32_t* cl
   if (!(total > 0.0 && isfinite(total)))
     return fail(DRL_ERR_INVALID, "drl_set_mocap_clips: the clip weights must have a positive finite sum");
   DeviceGuard guard__(e->cfg.device);
-  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the tables
-  void** ptrs[] = {(void**)&e->clip_first, (void**)&e->step_clip, (void**)&e->clip_cdf, (void**)&e->clip_stats,
-                   (void**)&e->d_clips};
-  for (void** p : ptrs) {
-    if (*p) CUDA_TRY(cudaFree(*p));
-    *p = nullptr;
-  }
-  e->clip_first_h.assign(clip_first_step, clip_first_step + n_clips + 1);
-  e->clip_weight_h.resize(n_clips);
-  for (int k = 0; k < n_clips; k++) e->clip_weight_h[k] = clip_weight[k] / total;
-  e->mocap_gen++;                             // the failure-weighted RSI bins weigh the clips: rebuild them
+  ClipBufs c;
+  c.first_h.assign(clip_first_step, clip_first_step + n_clips + 1);
+  c.weight_h.resize(n_clips);
+  for (int k = 0; k < n_clips; k++) c.weight_h[k] = clip_weight[k] / total;
   if (n_clips > 1) {
     std::vector<int> step_clip(n_steps);
     for (int k = 0; k < n_clips; k++)
@@ -533,65 +501,67 @@ extern "C" int drl_set_mocap_clips(DrlEnv* e, int32_t n_clips, const int32_t* cl
       acc += clip_weight[k];
       cdf[k] = k >= last_pos ? 1.0 : acc / total;
     }
-    const size_t ns = (size_t)n_clips * kClipStatCount;
-    if (upload(&e->clip_first, clip_first_step, (size_t)n_clips + 1) || upload(&e->step_clip, step_clip.data(), n_steps) ||
-        upload(&e->clip_cdf, cdf.data(), n_clips))
+    if (c.first.from_host(clip_first_step, (size_t)n_clips + 1) || c.step_clip.from_host(step_clip.data(), n_steps) ||
+        c.cdf.from_host(cdf.data(), n_clips))
       return fail(DRL_ERR_CUDA, "drl_set_mocap_clips: device copy failed");
-    CUDA_TRY(cudaMalloc(&e->clip_stats, ns * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMemset(e->clip_stats, 0, ns * sizeof(unsigned long long)));
-    ClipLibrary h;
-    h.n_clips = n_clips; h.clip_first = e->clip_first; h.step_clip = e->step_clip; h.clip_cdf = e->clip_cdf;
-    h.clip_stats = e->clip_stats;
-    CUDA_TRY(cudaMalloc(&e->d_clips, sizeof(ClipLibrary)));
-    CUDA_TRY(cudaMemcpy(e->d_clips, &h, sizeof(ClipLibrary), cudaMemcpyHostToDevice));
+    CUDA_TRY(c.stats.zeros((size_t)n_clips * kClipStatCount));
+    const ClipLibrary h{n_clips, c.first.get(), c.step_clip.get(), c.cdf.get(), c.stats.get()};
+    CUDA_TRY(c.lib.from_host(&h, 1));
   }
+  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the tables
+  e->clips = std::move(c);
+  e->mocap_gen++;                             // the failure-weighted RSI bins weigh the clips: rebuild them
   return DRL_OK;
 }
 
 extern "C" int drl_get_clip_stats(DrlEnv* e, int64_t* out, void* stream) {
   if (!e || !out) return fail(DRL_ERR_INVALID, "drl_get_clip_stats: null argument");
-  if (!e->clip_stats) return fail(DRL_ERR_STATE, "drl_get_clip_stats: the mocap has a single clip");
+  if (!e->clips.stats.get()) return fail(DRL_ERR_STATE, "drl_get_clip_stats: the mocap has a single clip");
   DeviceGuard guard__(e->cfg.device);
-  const size_t n = (e->clip_first_h.size() - 1) * kClipStatCount;
-  CUDA_TRY(cudaMemcpyAsync(out, e->clip_stats, n * sizeof(int64_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  CUDA_TRY(cudaMemcpyAsync(out, e->clips.stats.get(), e->clips.stats.size() * sizeof(int64_t), cudaMemcpyDeviceToDevice,
+                           (cudaStream_t)stream));
   return DRL_OK;
 }
 
 static AdaptiveRsiArgs ars_args(DrlEnv* e, double rho) {
   AdaptiveRsiArgs a;
-  a.n_bins = e->ars_n_bins; a.rho = rho; a.lambda = (double)e->ars_lambda;
-  a.u = e->ars_u; a.counts = e->ars_counts; a.inc = e->ars_inc; a.cdf = e->ars_cdf; a.prob = e->ars_prob;
+  a.n_bins = e->ars.n_bins(); a.rho = rho; a.lambda = (double)e->ars_lambda;
+  a.u = e->ars.u.get(); a.counts = e->ars.counts.get(); a.inc = e->ars.inc.get(); a.cdf = e->ars.cdf.get();
+  a.prob = e->ars.prob.get();
   return a;
 }
 
 static StepArgs make_args(DrlEnv* e) {
   StepArgs a;
   memset(&a, 0, sizeof a);
-  a.model = e->d_model; a.num_envs = e->cfg.num_envs;
+  const StateBufs& s = e->st;
+  const MocapBufs& m = e->mocap;
+  const RingBufs& r = e->ring;
+  a.model = e->d_model.get(); a.num_envs = e->cfg.num_envs;
   a.frame_skip = e->frame_skip_override >= 0 ? e->frame_skip_override : e->cfg.frame_skip;
-  a.state_f = e->state_f; a.state_i = e->state_i; a.state_as = e->state_as; a.state_d = e->state_d;
-  a.ref = e->ref; a.step_off = e->step_off; a.step_len = e->step_len; a.left_step = e->left_step;
-  a.step_vel = e->step_vel; a.step_last_comx = e->step_last_comx; a.des_vel_prefix = e->des_vel_prefix;
-  a.extras = e->extras_last; a.stats = e->stats;
-  a.ring_len = e->ring_len; a.ring_ret = e->ring_ret; a.ring_head = e->ring_head; a.ring_cap = e->ring_cap;
-  a.ring_rsi_pos = e->ring_rsi_pos; a.ring_et_pos = e->ring_et_pos; a.ring_difficult = e->ring_difficult;
+  a.state_f = s.state_f.get(); a.state_i = s.state_i.get(); a.state_as = s.state_as.get(); a.state_d = s.state_d.get();
+  a.ref = m.ref.get(); a.step_off = m.step_off.get(); a.step_len = m.step_len.get(); a.left_step = m.left_step.get();
+  a.step_vel = m.step_vel.get(); a.step_last_comx = m.step_last_comx.get(); a.des_vel_prefix = m.des_vel_prefix.get();
+  a.extras = s.extras_last.get(); a.stats = s.stats.get();
+  a.ring_len = r.len.get(); a.ring_ret = r.ret.get(); a.ring_head = r.head.get(); a.ring_cap = e->ring_cap;
+  a.ring_rsi_pos = r.rsi_pos.get(); a.ring_et_pos = r.et_pos.get(); a.ring_difficult = r.difficult.get();
   a.eval_mode = e->eval_mode;
-  a.speed_profile = e->speed_profile_len > 0 ? e->speed_profile : nullptr;
-  a.speed_profile_len = e->speed_profile_len;
+  a.speed_profile = e->speed_profile.get(); a.speed_profile_len = (int)e->speed_profile.size();   // null / 0 when off
   a.playback = e->playback;
-  a.cta_rows = e->cta_rows; a.cta_ticket = e->cta_ticket;
-  a.tor_hist = e->tor_hist; a.med_tor_sm = e->med_tor_sm;
-  a.ee_f = e->ee_f; a.ee_d = e->ee_d;
-  a.contact_et = e->hm.et_contact_mask ? e->contact_et : nullptr;
+  a.cta_rows = s.cta_rows.get(); a.cta_ticket = s.cta_ticket.get();
+  a.tor_hist = s.tor_hist.get(); a.med_tor_sm = s.med_tor_sm.get();
+  a.ee_f = s.ee_f.get(); a.ee_d = s.ee_d.get();
+  a.contact_et = e->hm.et_contact_mask ? e->contact_et.get() : nullptr;
   if (e->ars_lambda > 0.f) {
     a.ars_coin = (unsigned long long)llround((double)e->ars_lambda * 4294967296.0);
-    a.ars_n_bins = e->ars_n_bins; a.ars_bin_samples = e->ars_bin_samples;
-    a.ars_cdf = e->ars_cdf; a.ars_bins = e->ars_bins; a.ars_inc = e->ars_inc; a.ars_env_bin = e->ars_env_bin;
+    a.ars_n_bins = e->ars.n_bins(); a.ars_bin_samples = e->ars.bin_samples;
+    a.ars_cdf = e->ars.cdf.get(); a.ars_bins = e->ars.bins.get(); a.ars_inc = e->ars.inc.get();
+    a.ars_env_bin = e->ars.env_bin.get();
   }
-  a.clips = e->d_clips;
+  a.clips = e->clips.lib.get();
   a.vn_ret = e->vn_ret; a.vn_gamma = e->vn_gamma; a.packed = e->vn_packed;
   if (e->playback) a.frame_skip = 0;
-  a.debug = e->debug;
+  a.debug = e->debug.get();
   return a;
 }
 
@@ -619,9 +589,9 @@ extern "C" int drl_step(DrlEnv* e, const float* actions, float* obs, float* rew,
   a.actions = actions; a.obs = obs; a.rew = rew; a.done = done; a.terminal_obs = terminal_obs;
   a.inj_istep = inj_istep; a.inj_pos = inj_pos;
   const bool rk4 = e->cfg.integrator == DRL_INTEGRATOR_RK4, pd = e->actuation == DRL_ACTUATION_PD;
-  if (e->debug && rk4) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for the Euler integrator only");
-  if (e->debug && pd) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for torque actuation only");
-  CUDA_TRY(launch_step(a, e->nv, e->G, rk4, 0, e->block, e->debug != nullptr, pd, (cudaStream_t)stream));
+  if (a.debug && rk4) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for the Euler integrator only");
+  if (a.debug && pd) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for torque actuation only");
+  CUDA_TRY(launch_step(a, e->nv, e->G, rk4, 0, e->block, a.debug != nullptr, pd, (cudaStream_t)stream));
   if (e->ars_lambda > 0.f) CUDA_TRY(launch_adaptive_rsi_update(ars_args(e, pow(2.0, -1.0 / e->ars_halflife)),
                                                                (cudaStream_t)stream));
   return DRL_OK;
@@ -639,8 +609,8 @@ extern "C" int drl_get_state(DrlEnv* e, float* qpos, float* qvel, int32_t* curso
   int rc = ready(e, "drl_get_state");
   if (rc) return rc;
   DeviceGuard guard__(e->cfg.device);
-  CUDA_TRY(launch_state_copy(e->state_f, e->state_i, e->state_as, qpos, qvel, cursor, e->cfg.num_envs, e->nv, e->G, 0,
-                             (cudaStream_t)stream));
+  CUDA_TRY(launch_state_copy(e->st.state_f.get(), e->st.state_i.get(), e->st.state_as.get(), qpos, qvel, cursor,
+                             e->cfg.num_envs, e->nv, e->G, 0, (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -648,11 +618,12 @@ extern "C" int drl_set_state(DrlEnv* e, const float* qpos, const float* qvel, co
   int rc = ready(e, "drl_set_state");
   if (rc) return rc;
   DeviceGuard guard__(e->cfg.device);
-  CUDA_TRY(launch_state_copy(e->state_f, e->state_i, e->state_as, const_cast<float*>(qpos), const_cast<float*>(qvel),
-                             const_cast<int32_t*>(cursor), e->cfg.num_envs, e->nv, e->G, 1, (cudaStream_t)stream));
+  CUDA_TRY(launch_state_copy(e->st.state_f.get(), e->st.state_i.get(), e->st.state_as.get(), const_cast<float*>(qpos),
+                             const_cast<float*>(qvel), const_cast<int32_t*>(cursor), e->cfg.num_envs, e->nv, e->G, 1,
+                             (cudaStream_t)stream));
   // an episode that continues from a state set here is no longer one that started with a random RSI draw
-  if (e->ars_env_bin)
-    CUDA_TRY(cudaMemsetAsync(e->ars_env_bin, 0xFF, (size_t)e->cfg.num_envs * sizeof(int), (cudaStream_t)stream));
+  if (e->ars.env_bin.get())
+    CUDA_TRY(cudaMemsetAsync(e->ars.env_bin.get(), 0xFF, (size_t)e->cfg.num_envs * sizeof(int), (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -661,7 +632,8 @@ extern "C" int drl_get_extras(DrlEnv* e, float* extras, void* stream) {
   if (rc) return rc;
   DeviceGuard guard__(e->cfg.device);
   if (!extras) return fail(DRL_ERR_INVALID, "drl_get_extras: null tensor");
-  CUDA_TRY(launch_extras(e->state_f, e->extras_last, extras, e->cfg.num_envs, e->G, (cudaStream_t)stream));
+  CUDA_TRY(launch_extras(e->st.state_f.get(), e->st.extras_last.get(), extras, e->cfg.num_envs, e->G,
+                         (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -670,7 +642,7 @@ extern "C" int drl_get_stats(DrlEnv* e, double* stats, void* stream) {
   if (rc) return rc;
   DeviceGuard guard__(e->cfg.device);
   if (!stats) return fail(DRL_ERR_INVALID, "drl_get_stats: null tensor");
-  CUDA_TRY(cudaMemcpyAsync(stats, e->stats, DRL_STATS_COUNT * sizeof(double), cudaMemcpyDeviceToDevice,
+  CUDA_TRY(cudaMemcpyAsync(stats, e->st.stats.get(), DRL_STATS_COUNT * sizeof(double), cudaMemcpyDeviceToDevice,
                            (cudaStream_t)stream));
   return DRL_OK;
 }
@@ -679,7 +651,7 @@ extern "C" int drl_reset_stats(DrlEnv* e, void* stream) {
   int rc = ready(e, "drl_reset_stats");
   if (rc) return rc;
   DeviceGuard guard__(e->cfg.device);
-  CUDA_TRY(cudaMemsetAsync(e->stats, 0, DRL_STATS_COUNT * sizeof(double), (cudaStream_t)stream));
+  CUDA_TRY(cudaMemsetAsync(e->st.stats.get(), 0, DRL_STATS_COUNT * sizeof(double), (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -690,13 +662,14 @@ extern "C" int drl_get_episode_ring(DrlEnv* e, int32_t* ep_len, float* ep_ret, i
   DeviceGuard guard__(e->cfg.device);
   if (!total_episodes) return fail(DRL_ERR_INVALID, "drl_get_episode_ring: null argument");
   cudaStream_t st = (cudaStream_t)stream;
+  const RingBufs& r = e->ring;
   unsigned long long head = 0;
-  CUDA_TRY(cudaMemcpyAsync(&head, e->ring_head, sizeof head, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaMemcpyAsync(&head, r.head.get(), sizeof head, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));     // the count is returned to the host by value
   *total_episodes = (int64_t)head;
   const int n = capacity < e->ring_cap ? capacity : e->ring_cap;
-  if (ep_len && n > 0) CUDA_TRY(cudaMemcpyAsync(ep_len, e->ring_len, n * sizeof(int), cudaMemcpyDeviceToDevice, st));
-  if (ep_ret && n > 0) CUDA_TRY(cudaMemcpyAsync(ep_ret, e->ring_ret, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  if (ep_len && n > 0) CUDA_TRY(cudaMemcpyAsync(ep_len, r.len.get(), n * sizeof(int), cudaMemcpyDeviceToDevice, st));
+  if (ep_ret && n > 0) CUDA_TRY(cudaMemcpyAsync(ep_ret, r.ret.get(), n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return DRL_OK;
 }
 
@@ -708,9 +681,9 @@ extern "C" int drl_get_episode_positions(DrlEnv* e, int32_t* rsi_pos, int32_t* e
   cudaStream_t st = (cudaStream_t)stream;
   const int n = capacity < e->ring_cap ? capacity : e->ring_cap;
   if (n <= 0) return DRL_OK;
-  if (rsi_pos) CUDA_TRY(cudaMemcpyAsync(rsi_pos, e->ring_rsi_pos, n * sizeof(int), cudaMemcpyDeviceToDevice, st));
-  if (et_pos) CUDA_TRY(cudaMemcpyAsync(et_pos, e->ring_et_pos, n * sizeof(int), cudaMemcpyDeviceToDevice, st));
-  if (difficult) CUDA_TRY(cudaMemcpyAsync(difficult, e->ring_difficult, n, cudaMemcpyDeviceToDevice, st));
+  if (rsi_pos) CUDA_TRY(cudaMemcpyAsync(rsi_pos, e->ring.rsi_pos.get(), n * sizeof(int), cudaMemcpyDeviceToDevice, st));
+  if (et_pos) CUDA_TRY(cudaMemcpyAsync(et_pos, e->ring.et_pos.get(), n * sizeof(int), cudaMemcpyDeviceToDevice, st));
+  if (difficult) CUDA_TRY(cudaMemcpyAsync(difficult, e->ring.difficult.get(), n, cudaMemcpyDeviceToDevice, st));
   return DRL_OK;
 }
 
@@ -719,7 +692,7 @@ extern "C" int drl_get_running_rsi_positions(DrlEnv* e, int32_t* rsi_pos, void* 
   if (rc) return rc;
   DeviceGuard guard__(e->cfg.device);
   if (!rsi_pos) return fail(DRL_ERR_INVALID, "drl_get_running_rsi_positions: null tensor");
-  CUDA_TRY(launch_running_rsi(e->state_i, rsi_pos, e->cfg.num_envs, (cudaStream_t)stream));
+  CUDA_TRY(launch_running_rsi(e->st.state_i.get(), rsi_pos, e->cfg.num_envs, (cudaStream_t)stream));
   return DRL_OK;
 }
 
@@ -728,8 +701,8 @@ extern "C" int drl_get_median_torque(DrlEnv* e, float* out, void* stream) {
   if (rc) return rc;
   DeviceGuard guard__(e->cfg.device);
   if (!out) return fail(DRL_ERR_INVALID, "drl_get_median_torque: null tensor");
-  if (!e->med_tor_sm) return fail(DRL_ERR_STATE, "drl_get_median_torque: the env was created with monitor_median_torque = 0");
-  CUDA_TRY(cudaMemcpyAsync(out, e->med_tor_sm, (size_t)e->cfg.num_envs * sizeof(float), cudaMemcpyDeviceToDevice,
+  if (!e->st.med_tor_sm.get()) return fail(DRL_ERR_STATE, "drl_get_median_torque: the env was created with monitor_median_torque = 0");
+  CUDA_TRY(cudaMemcpyAsync(out, e->st.med_tor_sm.get(), (size_t)e->cfg.num_envs * sizeof(float), cudaMemcpyDeviceToDevice,
                            (cudaStream_t)stream));
   return DRL_OK;
 }
@@ -738,15 +711,16 @@ extern "C" int drl_get_ee_reward(DrlEnv* e, float* last, float* smoothed, void* 
   int rc = ready(e, "drl_get_ee_reward");
   if (rc) return rc;
   DeviceGuard guard__(e->cfg.device);
-  if (!e->ee_f) return fail(DRL_ERR_STATE, "drl_get_ee_reward: the env was created with ee_weight = 0");
+  const float* ee_f = e->st.ee_f.get();
+  if (!ee_f) return fail(DRL_ERR_STATE, "drl_get_ee_reward: the env was created with ee_weight = 0");
   const size_t n = (size_t)e->cfg.num_envs;
   cudaStream_t st = (cudaStream_t)stream;
   // columns of the [N][2] rows
   if (last)
-    CUDA_TRY(cudaMemcpy2DAsync(last, sizeof(float), e->ee_f, 2 * sizeof(float), sizeof(float), n,
+    CUDA_TRY(cudaMemcpy2DAsync(last, sizeof(float), ee_f, 2 * sizeof(float), sizeof(float), n,
                                cudaMemcpyDeviceToDevice, st));
   if (smoothed)
-    CUDA_TRY(cudaMemcpy2DAsync(smoothed, sizeof(float), e->ee_f + 1, 2 * sizeof(float), sizeof(float), n,
+    CUDA_TRY(cudaMemcpy2DAsync(smoothed, sizeof(float), ee_f + 1, 2 * sizeof(float), sizeof(float), n,
                                cudaMemcpyDeviceToDevice, st));
   return DRL_OK;
 }
@@ -766,7 +740,7 @@ extern "C" int drl_set_det_init_counters(DrlEnv* e, const int32_t* counts) {
       return fail(DRL_ERR_INVALID, "drl_set_det_init_counters: counts[%d] = %d outside [0, eval_n_times)", i, counts[i]);
   DeviceGuard guard__(e->cfg.device);
   CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy2D(e->state_i + kCurNDet, kCurCount8 * sizeof(int), counts, sizeof(int), sizeof(int), (size_t)n,
+  CUDA_TRY(cudaMemcpy2D(e->st.state_i.get() + kCurNDet, kCurCount8 * sizeof(int), counts, sizeof(int), sizeof(int), (size_t)n,
                         cudaMemcpyHostToDevice));
   return DRL_OK;
 }
@@ -774,12 +748,12 @@ extern "C" int drl_set_det_init_counters(DrlEnv* e, const int32_t* counts) {
 extern "C" int drl_set_seed(DrlEnv* e, uint64_t seed) {
   if (!e) return fail(DRL_ERR_INVALID, "drl_set_seed: null env");
   if (!e->have_model) return fail(DRL_ERR_STATE, "drl_set_seed: upload the model first");
-  e->cfg.seed = seed;
-  e->hm.seed = seed;
   DeviceGuard guard__(e->cfg.device);
-  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the model block
-  CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
-  return DRL_OK;
+  DevModel d = e->hm;
+  d.seed = seed;
+  const int rc = publish_model(e, d);
+  if (rc == DRL_OK) e->cfg.seed = seed;
+  return rc;
 }
 
 extern "C" int drl_set_actuation(DrlEnv* e, int32_t mode, const double* kp, const double* kv) {
@@ -787,7 +761,7 @@ extern "C" int drl_set_actuation(DrlEnv* e, int32_t mode, const double* kp, cons
   if (mode != DRL_ACTUATION_TORQUE && mode != DRL_ACTUATION_PD)
     return fail(DRL_ERR_INVALID, "drl_set_actuation: unknown mode %d", mode);
   if (!e->have_model) return fail(DRL_ERR_STATE, "drl_set_actuation: upload the model first");
-  DevModel& d = e->hm;
+  DevModel d = e->hm;
   if (mode == DRL_ACTUATION_PD) {
     if (!kp || !kv) return fail(DRL_ERR_INVALID, "drl_set_actuation: PD needs kp and kv");
     for (int u = 0; u < d.nu; u++) {
@@ -814,17 +788,16 @@ extern "C" int drl_set_actuation(DrlEnv* e, int32_t mode, const double* kp, cons
       d.pd_half[u] = (float)(0.5 * (hi - lo));
     }
   }
-  e->actuation = mode;
   DeviceGuard guard__(e->cfg.device);
-  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the model block
-  CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
-  return DRL_OK;
+  const int rc = publish_model(e, d);
+  if (rc == DRL_OK) e->actuation = mode;
+  return rc;
 }
 
 extern "C" int drl_set_contact_termination(DrlEnv* e, uint32_t body_mask) {
   if (!e) return fail(DRL_ERR_INVALID, "drl_set_contact_termination: null env");
   if (!e->have_model) return fail(DRL_ERR_STATE, "drl_set_contact_termination: upload the model first");
-  DevModel& d = e->hm;
+  DevModel d = e->hm;
   if (body_mask >> d.nb) return fail(DRL_ERR_INVALID, "drl_set_contact_termination: mask 0x%x names a body >= nb = %d",
                                      body_mask, d.nb);
   // the reset puts the lowest foot-corner site on the floor: a body that carries one would end every episode at once
@@ -832,23 +805,20 @@ extern "C" int drl_set_contact_termination(DrlEnv* e, uint32_t body_mask) {
     if ((body_mask >> d.site_body[s]) & 1u)
       return fail(DRL_ERR_INVALID, "drl_set_contact_termination: body %d carries a foot-corner site", d.site_body[s]);
   DeviceGuard guard__(e->cfg.device);
-  if (body_mask && !e->contact_et) {
-    const size_t N = (size_t)e->cfg.num_envs;
-    CUDA_TRY(cudaMalloc(&e->contact_et, N * sizeof(int)));
-    CUDA_TRY(cudaMemset(e->contact_et, 0, N * sizeof(int)));
-  }
+  DevBuf<int> counts;
+  if (body_mask && !e->contact_et.get()) CUDA_TRY(counts.zeros((size_t)e->cfg.num_envs));
   d.et_contact_mask = body_mask;
-  CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the model block
-  CUDA_TRY(cudaMemcpy(e->d_model, &e->hm, sizeof(DevModel), cudaMemcpyHostToDevice));
-  return DRL_OK;
+  const int rc = publish_model(e, d);
+  if (rc == DRL_OK && counts.get()) e->contact_et = std::move(counts);
+  return rc;
 }
 
 extern "C" int drl_get_contact_terminations(DrlEnv* e, int32_t* out, void* stream) {
   if (!e || !out) return fail(DRL_ERR_INVALID, "drl_get_contact_terminations: null argument");
-  if (!e->contact_et)
+  if (!e->contact_et.get())
     return fail(DRL_ERR_STATE, "drl_get_contact_terminations: contact termination was never enabled on this env");
   DeviceGuard guard__(e->cfg.device);
-  CUDA_TRY(cudaMemcpyAsync(out, e->contact_et, (size_t)e->cfg.num_envs * sizeof(int32_t), cudaMemcpyDeviceToDevice,
+  CUDA_TRY(cudaMemcpyAsync(out, e->contact_et.get(), (size_t)e->cfg.num_envs * sizeof(int32_t), cudaMemcpyDeviceToDevice,
                            (cudaStream_t)stream));
   return DRL_OK;
 }
@@ -888,38 +858,27 @@ extern "C" int drl_set_adaptive_rsi(DrlEnv* e, float lambda, int32_t halflife_st
     return fail(DRL_ERR_STATE, "drl_set_adaptive_rsi: model and mocap must be uploaded first");
   DeviceGuard guard__(e->cfg.device);
   CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the tables
-  if (lambda > 0.f && (e->ars_gen != e->mocap_gen || e->ars_bin_samples != bin_samples)) {
+  if (lambda > 0.f && (e->ars.gen != e->mocap_gen || e->ars.bin_samples != bin_samples)) {
     // first enable for this mocap and bin width: a new, empty table; every running episode is uncounted
     std::vector<int> bins;
     std::vector<double> u;
-    ars_layout(e->step_len_h, e->clip_first_h, e->clip_weight_h, bin_samples, bins, u);
+    ars_layout(e->mocap.step_len_h, e->clips.first_h, e->clips.weight_h, bin_samples, bins, u);
     const size_t nb = u.size(), N = (size_t)e->cfg.num_envs;
-    void** ptrs[] = {(void**)&e->ars_counts, (void**)&e->ars_u, (void**)&e->ars_cdf, (void**)&e->ars_prob,
-                     (void**)&e->ars_bins, (void**)&e->ars_inc, (void**)&e->ars_env_bin};
-    for (void** p : ptrs) {
-      if (*p) CUDA_TRY(cudaFree(*p));
-      *p = nullptr;
-    }
-    e->ars_gen = -1;
-    CUDA_TRY(cudaMalloc(&e->ars_counts, 2 * nb * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&e->ars_u, nb * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&e->ars_cdf, nb * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&e->ars_prob, nb * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&e->ars_bins, bins.size() * sizeof(int)));
-    CUDA_TRY(cudaMalloc(&e->ars_inc, 2 * nb * sizeof(unsigned)));
-    CUDA_TRY(cudaMalloc(&e->ars_env_bin, N * sizeof(int)));
-    CUDA_TRY(cudaMemset(e->ars_counts, 0, 2 * nb * sizeof(double)));
-    CUDA_TRY(cudaMemset(e->ars_inc, 0, 2 * nb * sizeof(unsigned)));
-    CUDA_TRY(cudaMemset(e->ars_env_bin, 0xFF, N * sizeof(int)));
-    CUDA_TRY(cudaMemcpy(e->ars_u, u.data(), nb * sizeof(double), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(e->ars_bins, bins.data(), bins.size() * sizeof(int), cudaMemcpyHostToDevice));
-    e->ars_n_bins = (int)nb;
-    e->ars_bin_samples = bin_samples;
-    e->ars_gen = e->mocap_gen;
+    ArsBufs t;
+    t.gen = e->mocap_gen; t.bin_samples = bin_samples;
+    CUDA_TRY(t.counts.zeros(2 * nb));
+    CUDA_TRY(t.u.from_host(u.data(), nb));
+    CUDA_TRY(t.cdf.alloc(nb));
+    CUDA_TRY(t.prob.alloc(nb));
+    CUDA_TRY(t.bins.from_host(bins.data(), bins.size()));
+    CUDA_TRY(t.inc.zeros(2 * nb));
+    CUDA_TRY(t.env_bin.alloc(N));
+    CUDA_TRY(cudaMemset(t.env_bin.get(), 0xFF, N * sizeof(int)));
+    e->ars = std::move(t);
   }
   e->ars_lambda = lambda;
   e->ars_halflife = halflife_steps;
-  if (e->ars_counts) {                        // rebuild the sampling tables (and prob, which depends on lambda)
+  if (e->ars.counts.get()) {                  // rebuild the sampling tables (and prob, which depends on lambda)
     CUDA_TRY(launch_adaptive_rsi_update(ars_args(e, 1.0), nullptr));
     CUDA_TRY(cudaDeviceSynchronize());
   }
@@ -929,32 +888,33 @@ extern "C" int drl_set_adaptive_rsi(DrlEnv* e, float lambda, int32_t halflife_st
 extern "C" int drl_get_adaptive_rsi(DrlEnv* e, double* started, double* difficult, double* prob, int32_t* env_bin,
                                     void* stream) {
   if (!e) return fail(DRL_ERR_INVALID, "drl_get_adaptive_rsi: null env");
-  if (!e->ars_counts) return fail(DRL_ERR_STATE, "drl_get_adaptive_rsi: failure-weighted RSI was never enabled");
+  const double* counts = e->ars.counts.get();
+  if (!counts) return fail(DRL_ERR_STATE, "drl_get_adaptive_rsi: failure-weighted RSI was never enabled");
   DeviceGuard guard__(e->cfg.device);
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t nb = (size_t)e->ars_n_bins;
-  if (started) CUDA_TRY(cudaMemcpyAsync(started, e->ars_counts, nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
-  if (difficult)
-    CUDA_TRY(cudaMemcpyAsync(difficult, e->ars_counts + nb, nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
-  if (prob) CUDA_TRY(cudaMemcpyAsync(prob, e->ars_prob, nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  const size_t nb = (size_t)e->ars.n_bins();
+  if (started) CUDA_TRY(cudaMemcpyAsync(started, counts, nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  if (difficult) CUDA_TRY(cudaMemcpyAsync(difficult, counts + nb, nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  if (prob) CUDA_TRY(cudaMemcpyAsync(prob, e->ars.prob.get(), nb * sizeof(double), cudaMemcpyDeviceToDevice, st));
   if (env_bin)
-    CUDA_TRY(cudaMemcpyAsync(env_bin, e->ars_env_bin, (size_t)e->cfg.num_envs * sizeof(int), cudaMemcpyDeviceToDevice,
-                             st));
+    CUDA_TRY(cudaMemcpyAsync(env_bin, e->ars.env_bin.get(), (size_t)e->cfg.num_envs * sizeof(int),
+                             cudaMemcpyDeviceToDevice, st));
   return DRL_OK;
 }
 
 extern "C" int drl_set_adaptive_rsi_counts(DrlEnv* e, const double* started, const double* difficult) {
   if (!e || !started || !difficult) return fail(DRL_ERR_INVALID, "drl_set_adaptive_rsi_counts: null argument");
-  if (!e->ars_counts) return fail(DRL_ERR_STATE, "drl_set_adaptive_rsi_counts: failure-weighted RSI was never enabled");
-  const int nb = e->ars_n_bins;
+  double* counts = e->ars.counts.get();
+  if (!counts) return fail(DRL_ERR_STATE, "drl_set_adaptive_rsi_counts: failure-weighted RSI was never enabled");
+  const int nb = e->ars.n_bins();
   for (int b = 0; b < nb; b++)
     if (!(isfinite(started[b]) && difficult[b] >= 0.0 && difficult[b] <= started[b]))
       return fail(DRL_ERR_INVALID, "drl_set_adaptive_rsi_counts: bin %d: need 0 <= difficult <= started < inf", b);
   DeviceGuard guard__(e->cfg.device);
   CUDA_TRY(cudaDeviceSynchronize());          // enqueued steps may still read the tables
-  CUDA_TRY(cudaMemcpy(e->ars_counts, started, nb * sizeof(double), cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemcpy(e->ars_counts + nb, difficult, nb * sizeof(double), cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemset(e->ars_inc, 0, 2 * (size_t)nb * sizeof(unsigned)));
+  CUDA_TRY(cudaMemcpy(counts, started, nb * sizeof(double), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(counts + nb, difficult, nb * sizeof(double), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemset(e->ars.inc.get(), 0, 2 * (size_t)nb * sizeof(unsigned)));
   CUDA_TRY(launch_adaptive_rsi_update(ars_args(e, 1.0), nullptr));
   CUDA_TRY(cudaDeviceSynchronize());
   return DRL_OK;
@@ -971,15 +931,10 @@ extern "C" int drl_set_speed_profile(DrlEnv* e, const float* speeds, int32_t n) 
   if (n < 0 || (n > 0 && !speeds)) return fail(DRL_ERR_INVALID, "drl_set_speed_profile: n=%d with %s table", n,
                                                speeds ? "a" : "a null");
   DeviceGuard guard__(e->cfg.device);
+  DevBuf<float> table;
+  if (n > 0) CUDA_TRY(table.from_host(speeds, (size_t)n));
   CUDA_TRY(cudaDeviceSynchronize());   // the previous table may still be read by enqueued steps
-  if (e->speed_profile) CUDA_TRY(cudaFree(e->speed_profile));
-  e->speed_profile = nullptr;
-  e->speed_profile_len = 0;
-  if (n > 0) {
-    CUDA_TRY(cudaMalloc(&e->speed_profile, (size_t)n * sizeof(float)));
-    CUDA_TRY(cudaMemcpy(e->speed_profile, speeds, (size_t)n * sizeof(float), cudaMemcpyHostToDevice));
-    e->speed_profile_len = n;
-  }
+  e->speed_profile = std::move(table);
   return DRL_OK;
 }
 
@@ -997,25 +952,23 @@ extern "C" int drl_launch_info(DrlEnv* e, int32_t* lanes_per_env, int32_t* block
 // ---- test / tuning hooks (declared in include/drloco_b200.h under "debug") ----
 extern "C" int drl_debug_set(DrlEnv* e, int32_t frame_skip_override, int32_t block_threads, int32_t enable_dump) {
   if (!e) return fail(DRL_ERR_INVALID, "drl_debug_set: null env");
-  e->frame_skip_override = frame_skip_override;
-  if (block_threads > 0) {
-    if (block_threads % 32 != 0 || block_threads > 128) return fail(DRL_ERR_INVALID, "drl_debug_set: block size must be 32, 64, 96 or 128");
-    e->block = block_threads;
-  }
+  if (block_threads > 0 && (block_threads % 32 != 0 || block_threads > 128))
+    return fail(DRL_ERR_INVALID, "drl_debug_set: block size must be 32, 64, 96 or 128");
   DeviceGuard guard__(e->cfg.device);
-  if (enable_dump && !e->debug) {
-    const size_t n = (size_t)e->cfg.num_envs * 32 * 40;
-    CUDA_TRY(cudaMalloc(&e->debug, n * sizeof(float)));
-    CUDA_TRY(cudaMemset(e->debug, 0, n * sizeof(float)));
-  } else if (!enable_dump && e->debug) {
-    cudaFree(e->debug);
-    e->debug = nullptr;
+  if (enable_dump && !e->debug.get()) {
+    DevBuf<float> dump;
+    CUDA_TRY(dump.zeros((size_t)e->cfg.num_envs * 32 * 40));
+    e->debug = std::move(dump);
+  } else if (!enable_dump) {
+    e->debug = DevBuf<float>();
   }
+  e->frame_skip_override = frame_skip_override;
+  if (block_threads > 0) e->block = block_threads;
   return DRL_OK;
 }
 
 extern "C" int drl_debug_read(DrlEnv* e, float* host_out, int32_t n_floats) {
-  if (!e || !e->debug) return fail(DRL_ERR_STATE, "drl_debug_read: dump not enabled");
-  CUDA_TRY(cudaMemcpy(host_out, e->debug, (size_t)n_floats * sizeof(float), cudaMemcpyDeviceToHost));
+  if (!e || !e->debug.get()) return fail(DRL_ERR_STATE, "drl_debug_read: dump not enabled");
+  CUDA_TRY(cudaMemcpy(host_out, e->debug.get(), (size_t)n_floats * sizeof(float), cudaMemcpyDeviceToHost));
   return DRL_OK;
 }

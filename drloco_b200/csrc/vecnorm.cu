@@ -10,7 +10,10 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <memory>
+
 #include "../../include/drloco_b200.h"
+#include "dev_buf.h"
 
 namespace drl {
 
@@ -115,13 +118,11 @@ constexpr int kMaxPayload = 2 * DRL_MAX_OBS + 3;
 
 struct DrlComm {
   int world = 1, rank = 0, payload = 0, device = 0;
-  void* base = nullptr;                  // local mailbox allocation (exported): mail [2][world][payload] f64, flags [2][world] u64
-  double* mail = nullptr;
-  unsigned long long* flags = nullptr;
-  unsigned long long* step = nullptr;    // [2] device-side counters (the chain is CUDA-graph capturable): exchanges done so
+  drl::DevBuf<char> base;                // local mailbox allocation (exported): mail [2][world][payload] f64, flags [2][world] u64
+  drl::DevBuf<unsigned long long> step;  // [2] device-side counters (the chain is CUDA-graph capturable): exchanges done so
                                          // far (mailbox parity / flag value), cycle calls since the last merge
-  unsigned* ticket = nullptr;
-  double* pending = nullptr;             // [payload] moments accumulated since the last exchange
+  drl::DevBuf<unsigned> ticket;
+  drl::DevBuf<double> pending;           // [payload] moments accumulated since the last exchange
   void* peer_base[kMaxPeers] = {};
   bool connected = false;
 };
@@ -263,25 +264,19 @@ __global__ void __launch_bounds__(256) vecnorm_step_kernel(
 extern "C" int drl_comm_create(int32_t world, int32_t rank, int32_t obs_dim, DrlComm** out) {
   if (!out || world < 1 || world > kMaxPeers || rank < 0 || rank >= world || obs_dim <= 0 || obs_dim > DRL_MAX_OBS)
     return DRL_ERR_INVALID;
-  DrlComm* c = new DrlComm();
+  auto c = std::make_unique<DrlComm>();
   c->world = world; c->rank = rank; c->payload = 2 * obs_dim + 3;
   VN_TRY(cudaGetDevice(&c->device));
   const size_t mail_bytes = (size_t)2 * world * c->payload * sizeof(double);
   const size_t flag_bytes = (size_t)2 * world * sizeof(unsigned long long);
-  VN_TRY(cudaMalloc(&c->base, mail_bytes + flag_bytes));
-  VN_TRY(cudaMemset(c->base, 0, mail_bytes + flag_bytes));
-  c->mail = (double*)c->base;
-  c->flags = (unsigned long long*)((char*)c->base + mail_bytes);
-  VN_TRY(cudaMalloc(&c->step, 2 * sizeof(unsigned long long)));
-  VN_TRY(cudaMemset(c->step, 0, 2 * sizeof(unsigned long long)));
-  VN_TRY(cudaMalloc(&c->ticket, sizeof(unsigned)));
-  VN_TRY(cudaMemset(c->ticket, 0, sizeof(unsigned)));
-  VN_TRY(cudaMalloc(&c->pending, c->payload * sizeof(double)));
-  VN_TRY(cudaMemset(c->pending, 0, c->payload * sizeof(double)));
+  VN_TRY(c->base.zeros(mail_bytes + flag_bytes));
+  VN_TRY(c->step.zeros(2));
+  VN_TRY(c->ticket.zeros(1));
+  VN_TRY(c->pending.zeros(c->payload));
   VN_TRY(cudaDeviceSynchronize());
-  c->peer_base[rank] = c->base;
+  c->peer_base[rank] = c->base.get();
   c->connected = world == 1;
-  *out = c;
+  *out = c.release();
   return DRL_OK;
 }
 
@@ -289,7 +284,7 @@ extern "C" int drl_comm_export(DrlComm* c, void* handle64) {
   if (!c || !handle64) return DRL_ERR_INVALID;
   static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
   cudaIpcMemHandle_t h;
-  VN_TRY(cudaIpcGetMemHandle(&h, c->base));
+  VN_TRY(cudaIpcGetMemHandle(&h, c->base.get()));
   memcpy(handle64, &h, 64);
   return DRL_OK;
 }
@@ -313,10 +308,6 @@ extern "C" int drl_comm_destroy(DrlComm* c) {
   cudaDeviceSynchronize();
   for (int r = 0; r < c->world; r++)
     if (r != c->rank && c->peer_base[r]) cudaIpcCloseMemHandle(c->peer_base[r]);
-  if (c->base) cudaFree(c->base);
-  if (c->step) cudaFree(c->step);
-  if (c->ticket) cudaFree(c->ticket);
-  if (c->pending) cudaFree(c->pending);
   delete c;
   return DRL_OK;
 }
@@ -331,8 +322,9 @@ extern "C" int drl_vecnorm_step(const float* obs_in, float* obs_out, const float
   if (c->payload != 2 * d + 3 || !c->connected || sync_every < 0) return DRL_ERR_STATE;
   drl::CommView cv;
   cv.world = c->world; cv.rank = c->rank; cv.payload = c->payload; cv.sync_every = sync_every;
-  cv.mail = c->mail; cv.flags = c->flags; cv.step = c->step; cv.ticket = c->ticket; cv.pending = c->pending;
   const size_t mail_bytes = (size_t)2 * c->world * c->payload * sizeof(double);
+  cv.mail = (const double*)c->base.get(); cv.flags = (const unsigned long long*)(c->base.get() + mail_bytes);
+  cv.step = c->step.get(); cv.ticket = c->ticket.get(); cv.pending = c->pending.get();
   for (int r = 0; r < kMaxPeers; r++) {
     cv.peer_mail[r] = r < c->world ? (double*)c->peer_base[r] : nullptr;
     cv.peer_flags[r] = r < c->world ? (unsigned long long*)((char*)c->peer_base[r] + mail_bytes) : nullptr;
@@ -421,23 +413,24 @@ extern "C" int drl_fp32_peak_probe(int32_t device, double* tflops_out) {
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return DRL_ERR_CUDA;
   const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 16;
-  float* buf = nullptr;
-  if (cudaMalloc(&buf, (size_t)blocks * threads * sizeof(float)) != cudaSuccess) return DRL_ERR_CUDA;
-  cudaEvent_t e0, e1;
-  cudaEventCreate(&e0); cudaEventCreate(&e1);
+  drl::DevBuf<float> buf;
+  if (buf.alloc((size_t)blocks * threads) != cudaSuccess) return DRL_ERR_CUDA;
+  struct Events {                        // destroyed on every return
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    ~Events() { if (e0) cudaEventDestroy(e0); if (e1) cudaEventDestroy(e1); }
+  } ev;
+  if (cudaEventCreate(&ev.e0) != cudaSuccess || cudaEventCreate(&ev.e1) != cudaSuccess) return DRL_ERR_CUDA;
   double best = 0.0;
   for (int rep = 0; rep < 4; rep++) {
-    cudaEventRecord(e0);
-    drl::ffma_probe_kernel<<<blocks, threads>>>(buf, iters, 0.999f, 1e-3f);
-    cudaEventRecord(e1);
-    if (cudaEventSynchronize(e1) != cudaSuccess) { cudaFree(buf); return DRL_ERR_CUDA; }
+    cudaEventRecord(ev.e0);
+    drl::ffma_probe_kernel<<<blocks, threads>>>(buf.get(), iters, 0.999f, 1e-3f);
+    cudaEventRecord(ev.e1);
+    if (cudaEventSynchronize(ev.e1) != cudaSuccess) return DRL_ERR_CUDA;
     float ms = 0.f;
-    cudaEventElapsedTime(&ms, e0, e1);
+    cudaEventElapsedTime(&ms, ev.e0, ev.e1);
     const double flops = 2.0 * 8.0 * (double)iters * blocks * threads;
     if (rep > 0 && ms > 0.f) best = fmax(best, flops / (ms * 1e-3) / 1e12);
   }
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
-  cudaFree(buf);
   *tflops_out = best;
   return DRL_OK;
 }
