@@ -12,6 +12,7 @@ import numpy as np
 DRL_ABI_VERSION = 4
 MAX_DOF, MAX_BODY, MAX_ACT, MAX_SPHERE, MAX_BOX, MAX_SITE, MAX_OBS, MAX_PHASE_JOINTS = 24, 12, 16, 16, 8, 16, 64, 4
 MAX_EE = 4
+MAX_REF_OBS = 3        # DRL_MAX_REF_OBS: reference-pose frames of drl_set_ref_obs (EnvConfig.ref_obs_offsets)
 INTEGRATOR_RK4, INTEGRATOR_EULER = 0, 1
 CURSOR_STEPWISE, CURSOR_WRAP = 0, 1
 PHASE_FROM_CURSOR, PHASE_FROM_JOINTS = 0, 1

@@ -12,6 +12,8 @@ from typing import Optional, Tuple, Union
 
 import numpy as np
 
+from .cabi import MAX_REF_OBS   # reference-pose frames (DRL_MAX_REF_OBS)
+
 # environment ids (reference drloco/mujoco/config.py:5-6)
 STRAIGHT_WALKER = "StraightMimicWalker"
 WALKER_165 = "MimicWalker165cm65kg"
@@ -64,6 +66,11 @@ class EnvConfig:
                                                         # "Failure-weighted RSI")
     adaptive_rsi_halflife: int = 2000                   # half-life of its per-phase counts, in control steps of the
                                                         # batch (a choice, not a tuned value)
+    ref_obs_offsets: Tuple[int, ...] = ()               # reference-pose observations: one frame of reference qpos[1:]
+                                                        # per offset (control steps ahead, ints in [1, 256], strictly
+                                                        # increasing, at most 3) appended to the observation; () = off,
+                                                        # the reference's layout (see README "Reference-pose
+                                                        # observations")
     gamma: float = 0.0                                  # 0 -> by ctrl_freq, hypers.py:68
     integrator: str = "rk4"                             # xml:11; "euler" = MuJoCo semi-implicit Euler (fast mode)
     seed: int = 33                                      # utils.py:97
@@ -91,6 +98,17 @@ class EnvConfig:
         hl = self.adaptive_rsi_halflife
         if isinstance(hl, bool) or not isinstance(hl, (int, np.integer)) or hl <= 0 or hl >= 2 ** 31:
             raise ValueError(f"adaptive_rsi_halflife must be a positive int32 number of control steps, got {hl!r}")
+        offs = self.ref_obs_offsets
+        if isinstance(offs, (str, bytes)) or not isinstance(offs, (tuple, list)):
+            raise ValueError(f"ref_obs_offsets must be a tuple of ints, got {offs!r}")
+        if len(offs) > MAX_REF_OBS:
+            raise ValueError(f"ref_obs_offsets: at most {MAX_REF_OBS} frames, got {len(offs)}")
+        for k in offs:
+            if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= k <= 256:
+                raise ValueError(f"ref_obs_offsets: every offset must be an int in [1, 256], got {offs!r}")
+        if any(b <= a for a, b in zip(offs, offs[1:])):
+            raise ValueError(f"ref_obs_offsets must be strictly increasing, got {offs!r}")
+        self.ref_obs_offsets = tuple(int(k) for k in offs)
 
     def pd_gains(self, nu: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
         """(kp, kv) of actuation='pd' as float64 arrays in actuator order, scalars broadcast to the walker's nu

@@ -130,6 +130,8 @@ struct DrlEnv {
   DevBuf<float> speed_profile;            // drl_set_speed_profile; empty when off
   int playback = 0;
   int frame_skip_override = -1;
+  unsigned ref_obs = 0;                   // drl_set_ref_obs, packed as StepArgs::ref_obs; 0 = off
+  bool stepped = false;                   // a drl_reset or drl_step has been enqueued
   DevBuf<float> debug;                    // drl_debug_set
   // contact termination (drl_set_contact_termination): per-env episode count, allocated when first enabled
   DevBuf<int> contact_et;
@@ -170,6 +172,16 @@ extern "C" int drl_destroy(DrlEnv* e) {
   return DRL_OK;
 }
 
+// the smallest CTA the library launches carries 32 / G environments
+static size_t max_cta_blocks(const DrlEnv* e, size_t N) { return (N + (32 / e->G) - 1) / (32 / e->G); }
+
+// per-step statistics rows for observation rows of obs_row floats: one per block, then one per group of kStatGroup
+// blocks (two-level fixed-order sum in the step kernel)
+static cudaError_t alloc_cta_rows(const DrlEnv* e, size_t N, int obs_row, DevBuf<double>& rows) {
+  const size_t max_blocks = max_cta_blocks(e, N), max_groups = (max_blocks + kStatGroup - 1) / kStatGroup;
+  return rows.alloc((max_blocks + max_groups) * (2 * (size_t)obs_row + 2 + DRL_STATS_COUNT));
+}
+
 // persistent per-env state, statistics and episode ring, moved into the env once all of it is allocated
 static int alloc_state(DrlEnv* e, size_t N) {
   DevBuf<DevModel> model;
@@ -198,13 +210,9 @@ static int alloc_state(DrlEnv* e, size_t N) {
     CUDA_TRY(s.ee_d.zeros(N));
   }
   {
-    // the smallest CTA the library launches carries 32 / G environments
-    const size_t max_blocks = (N + (32 / e->G) - 1) / (32 / e->G);
-    const size_t row = 2 * (size_t)e->cfg.obs_dim + 2 + DRL_STATS_COUNT;
-    // rows of the blocks, then one row per group of kStatGroup blocks (two-level fixed-order sum in the step kernel);
+    const size_t max_groups = (max_cta_blocks(e, N) + kStatGroup - 1) / kStatGroup;
+    CUDA_TRY(alloc_cta_rows(e, N, e->cfg.obs_dim, s.cta_rows));
     // tickets: [0] counts finished groups, [1 + g] the finished blocks of group g
-    const size_t max_groups = (max_blocks + kStatGroup - 1) / kStatGroup;
-    CUDA_TRY(s.cta_rows.alloc((max_blocks + max_groups) * row));
     CUDA_TRY(s.cta_ticket.zeros(1 + max_groups));
   }
   // count_steps_same_vel starts at 1 (straight_walk_trajecs.py:124)
@@ -370,6 +378,7 @@ extern "C" int drl_upload_model(DrlEnv* e, const DrlWalkerModel* m) {
   d.eval_n_times = c.eval_n_times > 0 ? c.eval_n_times : 1;
   for (int i = 0; i < 4; i++) d.phase_joints[i] = c.phase_joints[i];
   d.obs_dim = c.obs_dim; d.act_dim = c.act_dim;
+  d.obs_row = c.obs_dim;   // drl_set_ref_obs widens it
   d.n_phase_obs = c.phase_mode == DRL_PHASE_FROM_CURSOR ? 1 : 2 * c.n_phase_joints;
   d.n_des_vel = c.obs_dim - d.n_phase_obs - (m->nv - 1) - m->nv;
   if (d.n_des_vel < 1 || d.n_des_vel > 2) return fail(DRL_ERR_INVALID, "config: obs_dim inconsistent with the model");
@@ -559,6 +568,7 @@ static StepArgs make_args(DrlEnv* e) {
     a.ars_env_bin = e->ars.env_bin.get();
   }
   a.clips = e->clips.lib.get();
+  a.ref_obs = e->ref_obs;
   a.vn_ret = e->vn_ret; a.vn_gamma = e->vn_gamma; a.packed = e->vn_packed;
   if (e->playback) a.frame_skip = 0;
   a.debug = e->debug.get();
@@ -576,6 +586,7 @@ extern "C" int drl_reset(DrlEnv* e, const uint8_t* mask, const int32_t* inj_iste
   a.debug = nullptr;
   CUDA_TRY(launch_step(a, e->nv, e->G, e->cfg.integrator == DRL_INTEGRATOR_RK4, 1, e->block, false, false,
                        (cudaStream_t)stream));
+  e->stepped = true;
   return DRL_OK;
 }
 
@@ -592,6 +603,7 @@ extern "C" int drl_step(DrlEnv* e, const float* actions, float* obs, float* rew,
   if (a.debug && rk4) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for the Euler integrator only");
   if (a.debug && pd) return fail(DRL_ERR_UNSUPPORTED, "drl_step: the dump variant exists for torque actuation only");
   CUDA_TRY(launch_step(a, e->nv, e->G, rk4, 0, e->block, a.debug != nullptr, pd, (cudaStream_t)stream));
+  e->stepped = true;
   if (e->ars_lambda > 0.f) CUDA_TRY(launch_adaptive_rsi_update(ars_args(e, pow(2.0, -1.0 / e->ars_halflife)),
                                                                (cudaStream_t)stream));
   return DRL_OK;
@@ -923,6 +935,40 @@ extern "C" int drl_set_adaptive_rsi_counts(DrlEnv* e, const double* started, con
 extern "C" int drl_set_playback(DrlEnv* e, int32_t on) {
   if (!e) return fail(DRL_ERR_INVALID, "drl_set_playback: null env");
   e->playback = on ? 1 : 0;
+  return DRL_OK;
+}
+
+extern "C" int drl_set_ref_obs(DrlEnv* e, int32_t n, const int32_t* offsets) {
+  if (!e) return fail(DRL_ERR_INVALID, "drl_set_ref_obs: null env");
+  if (!e->have_model) return fail(DRL_ERR_STATE, "drl_set_ref_obs: upload the model first");
+  if (e->stepped) return fail(DRL_ERR_STATE, "drl_set_ref_obs: the env has been reset or stepped (the row width is fixed)");
+  if (e->vn_packed) return fail(DRL_ERR_STATE, "drl_set_ref_obs: a VecNormalize is attached (its moments have the old width)");
+  if (n < 0 || n > DRL_MAX_REF_OBS) return fail(DRL_ERR_INVALID, "drl_set_ref_obs: n = %d outside [0, %d]", n, DRL_MAX_REF_OBS);
+  if (n > 0 && !offsets) return fail(DRL_ERR_INVALID, "drl_set_ref_obs: null offsets");
+  unsigned packed = (unsigned)n;
+  for (int f = 0; f < n; f++) {
+    if (offsets[f] < 1 || offsets[f] > 256)
+      return fail(DRL_ERR_INVALID, "drl_set_ref_obs: offsets[%d] = %d outside [1, 256]", f, offsets[f]);
+    if (f > 0 && offsets[f] <= offsets[f - 1])
+      return fail(DRL_ERR_INVALID, "drl_set_ref_obs: the offsets must be strictly increasing");
+    packed |= (unsigned)(offsets[f] - 1) << (8 * f + 8);
+  }
+  DevModel d = e->hm;
+  const int nq = d.nv - 1, B = d.n_phase_obs + d.n_des_vel;
+  if (d.mirror_policy)      // a frame is mirrored through the qpos-block part of the table: it must stay in the block
+    for (int k = B; k < B + nq; k++)
+      if (d.mirror_obs_idx[k] < B || d.mirror_obs_idx[k] >= B + nq)
+        return fail(DRL_ERR_INVALID, "drl_set_ref_obs: mirror_obs_idx[%d] = %d leaves the qpos block [%d, %d)", k,
+                    d.mirror_obs_idx[k], B, B + nq);
+  const int row = d.obs_dim + n * nq;
+  if (row > DRL_MAX_OBS_TOTAL) return fail(DRL_ERR_INVALID, "drl_set_ref_obs: row of %d floats > %d", row, DRL_MAX_OBS_TOTAL);
+  DeviceGuard guard__(e->cfg.device);
+  DevBuf<double> rows;
+  CUDA_TRY(alloc_cta_rows(e, (size_t)e->cfg.num_envs, row, rows));
+  d.obs_row = row;
+  if (const int rc = publish_model(e, d)) return rc;   // synchronises: no step reads the old rows any more
+  e->st.cta_rows = std::move(rows);
+  e->ref_obs = n > 0 ? packed : 0u;
   return DRL_OK;
 }
 

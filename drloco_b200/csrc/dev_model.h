@@ -59,7 +59,8 @@ struct alignas(16) DevModel {
   int early_termination, trunk_dof0;   // do_terminate_early: off/on, first of the three trunk rotation dofs
   unsigned et_contact_mask;          // DeepMimic contact termination (drl_set_contact_termination): bodies that end
                                      // the episode when they touch the floor; 0 = off
-  int pad_et_;
+  int obs_row;                       // floats per obs / terminal_obs row: obs_dim, plus the reference-pose frames of
+                                     // drl_set_ref_obs
   // ---- mocap ----
   int cursor_mode, increment, n_steps, n_samples, com_z_col, des_vel_window;
   unsigned long long seed;
@@ -121,10 +122,10 @@ struct StepArgs {
   const double* des_vel_prefix;      // [n_samples+n_steps][2] or null (float64 prefix sums, restarting at every step)
   // io
   const float* actions;              // [N][act_dim]
-  float* obs;                        // [N][obs_dim]
+  float* obs;                        // [N][obs_row]
   float* rew;                        // [N]
   unsigned char* done;               // [N]
-  float* terminal_obs;               // [N][obs_dim] nullable
+  float* terminal_obs;               // [N][obs_row] nullable
   const unsigned char* reset_mask;   // reset kernel only, nullable
   const int* inj_istep;              // nullable
   const int* inj_pos;                // nullable
@@ -147,12 +148,12 @@ struct StepArgs {
   float* med_tor_sm;                 // [N] smoothed median, written at episode ends
   // per-step statistics without atomics: every thread block writes one row of sums, the last block of every group of
   // kStatGroup blocks adds the group's rows, the last group to finish adds the group rows
-  double* cta_rows;                  // [grid + groups][2*obs_dim + 2 + DRL_STATS_COUNT]
+  double* cta_rows;                  // [grid + groups][2*obs_row + 2 + DRL_STATS_COUNT]
   unsigned* cta_ticket;              // [1 + groups]
   // fused VecNormalize (drl_attach_vecnorm; null = not attached)
   float* vn_ret;                     // [N] discounted-return accumulator, in/out
   float vn_gamma;
-  double* packed;                    // [2*obs_dim + 3] batch moments of the step, out
+  double* packed;                    // [2*obs_row + 3] batch moments of the step, out
   // end-effector term, allocated only when it is on (DevModel::w_ee != 0), null otherwise
   float* ee_f;                       // [N][2] ee_rew of the last step (1 after a reset), Monitor-smoothed mean
   double* ee_d;                      // [N] lifetime sum of ee_rew (Monitor never clears its per-step lists)
@@ -169,6 +170,9 @@ struct StepArgs {
   // mocap library (drl_set_mocap_clips), null with one clip.  Behind one pointer so that the parameter block, which
   // the kernel copies to its stack, grows by 8 bytes only.
   const ClipLibrary* clips;
+  // reference-pose observations (drl_set_ref_obs), 0 while off: byte 0 = the number of frames, byte f + 1 = frame f's
+  // offset in control steps, minus 1.  Each frame appends the reference qpos[1:] (nv - 1 floats) to the row.
+  unsigned ref_obs;
 };
 
 // per-clip episode counters (drl_get_clip_stats)

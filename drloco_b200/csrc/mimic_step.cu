@@ -281,6 +281,68 @@ __device__ __forceinline__ void write_obs(const DevModel& M, ES& E, int l, bool 
   __syncwarp();
 }
 
+// Reference-pose observations (drl_set_ref_obs, A.ref_obs != 0): frame f of the row is the reference qpos[1:] at the
+// cursor that cursor_next would reach after offset_f more control steps from the cursor (i_step, pos, flags, rsi_step)
+// the observation was built at: the target the pose reward compares against offset_f steps from now.  The cursor copy
+// advances once per step transition (pos accumulates, so this equals offset_f calls of cursor_next).  Every frame is
+// mirrored with the observation's own decision, through the qpos-block part of the mirror table (closed: the host
+// checks it).  dst / dst2 (nullable): row starts; `enable` predicates the stores, `moments` also stores x, x^2 into the
+// statistics row srow.  Called by every lane of the warp; no shared memory.
+template <int G>
+__device__ __noinline__ void ref_obs_frames(const DevModel& M, const StepArgs& A, int i_step, int pos, int flags,
+                                            int rsi_step, float zoff, int l, bool mirror, bool enable,
+                                            float* __restrict__ dst, float* __restrict__ dst2, double* srow,
+                                            bool moments) {
+  Cursor c;
+  c.i_step = i_step; c.pos = pos; c.flags = flags; c.rsi_step = rsi_step;
+  const int nq = M.nv - 1, B = M.n_phase_obs + M.n_des_vel, inc = M.increment;
+  const bool own = l >= 1 && l < M.nv;            // lane l carries qpos[l], column l - 1 of a frame
+  int src = l;
+  float sgn = 1.f;
+  if (mirror && own) { src = M.mirror_obs_idx[B + l - 1] - B + 1; sgn = M.mirror_obs_sign[B + l - 1]; }
+  const int n = (int)(A.ref_obs & 0xFFu);
+  int ahead = 0;
+  for (int f = 0; f < n; f++) {
+    const int k = (int)((A.ref_obs >> (8 * f + 8)) & 0xFFu) + 1;
+    int r = k - ahead;                            // control steps from the previous frame's cursor (offsets increase)
+    ahead = k;
+    while (r > 0) {
+      const int len = A.step_len[data_step(c)];
+      const int room = len - 1 - c.pos;
+      if (M.cursor_mode == DRL_CURSOR_STEPWISE) {
+        // cursor_next steps to the next mocap step on the first call that takes pos past len - 1
+        const int j = room < 0 ? 1 : room / inc + 1;
+        if (j > r) { c.pos += r * inc; break; }
+        int first = 0, last = M.n_steps - 1;
+        if (A.clips) first = clip_bounds(A.clips, c.i_step, last);
+        c.i_step = c.i_step >= last ? first + (A.left_step[c.i_step] ? 0 : 1) : c.i_step + 1;
+        c.pos += j * inc - len + 1;
+        c.flags &= ~kFlagReadStep0;
+        r -= j;
+      } else {
+        // ... and wraps to pos 0 on the first call that takes pos to len - 1 or beyond
+        const int j = room <= 0 ? 1 : (room + inc - 1) / inc;
+        if (j > r) { c.pos += r * inc; break; }
+        c.pos = 0;
+        r -= j;
+      }
+    }
+    float rq, rv;
+    ref_lookup(M, A, c, 0.f, zoff, l, G, own, rq, rv);   // (dist only moves lane 0, the dropped root x)
+    const float o = __shfl_sync(kFull, rq, src, G);
+    const float x = (mirror && own) ? sgn * o : rq;
+    if (enable && own) {
+      const int col = M.obs_dim + f * nq + l - 1;
+      dst[col] = x;
+      if (dst2) dst2[col] = x;
+      if (moments) {
+        srow[col] = (double)x;
+        srow[M.obs_row + col] = (double)x * (double)x;
+      }
+    }
+  }
+}
+
 // cos / sin of every hinge angle (slides: displacement) of the joint configuration q into E.cssn, the input of
 // tree_kinematics
 template <class ES>
@@ -530,7 +592,7 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     AS.bits[0] = pk & 0xFu; AS.bits[1] = (pk >> 4) & 0xFu; AS.prev_act = (pk >> 8) & 3u;
     AS.lbit = (pk >> 10) & 1u; AS.prev_lim = (pk >> 11) & 1u;
   }
-  float* obs_out = A.obs + (size_t)env * M.obs_dim;
+  float* obs_out = A.obs + (size_t)env * M.obs_row;
 
   if (do_reset_only) {
     // VecEnv.reset(): (masked) reset of the episode state
@@ -541,6 +603,9 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     build_obs<G>(M, A, E, L, c, q, v, ph, dv);
     const bool left = M.mirror_policy && A.left_step[c.i_step];
     write_obs<G>(M, E, l, left, want, obs_out);
+    if (A.ref_obs)
+      ref_obs_frames<G>(M, A, c.i_step, c.pos, c.flags, c.rsi_step, zoff, l, left, want, obs_out, nullptr, nullptr,
+                        false);
     if (want) {
       sf[l] = q; sf[G + l] = v; sf[2 * G + l] = 0.f;
       if (l == 0) {
@@ -744,18 +809,23 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     if (M.w_ee != 0.f) imit = fmaf(M.w_ee, ee_rew, imit);
     reward = imit * M.rew_scale + M.alive_bonus;
   }
-  {
-    const bool left1 = M.mirror_policy && A.left_step[c.i_step];
-    float* dst = (done && A.terminal_obs) ? A.terminal_obs + (size_t)env * M.obs_dim : obs_out;
-    write_obs<G>(M, E, l, left1, live && !bad, dst, done ? nullptr : ov);
-  }
+  const bool left1 = M.mirror_policy && A.left_step[c.i_step];
+  float* const dst1 = (done && A.terminal_obs) ? A.terminal_obs + (size_t)env * M.obs_row : obs_out;
+  write_obs<G>(M, E, l, left1, live && !bad, dst1, done ? nullptr : ov);
   // ---- per-environment row of sums for the step's statistics: [ sum obs[D] | sum obs^2[D] | ret, ret^2 | stats[20] ].
   // It lives in this environment's (now dead) solver scratch; the rows of a thread block are added up in a fixed order
   // at the end of the kernel, the blocks' rows by the last block to finish: no atomics, bit-reproducible sums.
-  const int kRowStats = 2 * M.obs_dim + 2, kRowLen = kRowStats + DRL_STATS_COUNT;
+  // (D = obs_row: with reference-pose frames the row reaches the end of E.Mt, over the union's W and U, which nothing
+  //  after this point writes: reset_env and build_obs touch the body frames, E.cssn and E.obsbuf, group_median the
+  //  scratch before E.Mt)
+  const int kRowStats = 2 * M.obs_row + 2, kRowLen = kRowStats + DRL_STATS_COUNT;
   double* srow = reinterpret_cast<double*>(E.Mt);
   for (int i = l; i < kRowLen; i += G) srow[i] = 0.0;
   __syncwarp();
+  // the frames of the terminal or returned observation, at the cursor it was built at; the returned one's moments
+  if (A.ref_obs)
+    ref_obs_frames<G>(M, A, c.i_step, c.pos, c.flags, c.rsi_step, zoff, l, left1, live && !bad, dst1, nullptr, srow,
+                      !done);
   // ---- Monitor.step (monitor_wrapper.py:88-166) --------------------------------------------------------------------
   ep_ret += reward;
   ep_tor += mean_abs_torque;
@@ -797,8 +867,8 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     if (A.vn_ret) {
       const float r = A.vn_ret[env] * A.vn_gamma + reward;
       A.vn_ret[env] = done ? 0.f : r;
-      srow[2 * M.obs_dim] = (double)r;
-      srow[2 * M.obs_dim + 1] = (double)r * (double)r;
+      srow[2 * M.obs_row] = (double)r;
+      srow[2 * M.obs_row + 1] = (double)r * (double)r;
     }
     if (A.extras) {
       float* ex = A.extras + (size_t)env * 16;
@@ -858,8 +928,11 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     build_obs<G>(M, A, E, L, c2, q2, v2, ph, dv);
     const bool left2 = M.mirror_policy && A.left_step[c2.i_step];
     write_obs<G>(M, E, l, left2, live && done, obs_out, ov);
-    write_obs<G>(M, E, l, left2, live && bad && A.terminal_obs != nullptr,
-                 A.terminal_obs ? A.terminal_obs + (size_t)env * M.obs_dim : obs_out);
+    float* const tdst = A.terminal_obs ? A.terminal_obs + (size_t)env * M.obs_row : obs_out;
+    write_obs<G>(M, E, l, left2, live && bad && A.terminal_obs != nullptr, tdst);
+    if (A.ref_obs)       // the returned observation's frames and moments (a blow-up's terminal observation is the same)
+      ref_obs_frames<G>(M, A, c2.i_step, c2.pos, c2.flags, c2.rsi_step, zoff2, l, left2, live && done, obs_out,
+                        (bad && A.terminal_obs) ? tdst : nullptr, srow, true);
     if (done) {
       c = c2; q = q2; v = v2; dist = dist2; zoff = zoff2;
       a = 0.f;
@@ -894,7 +967,7 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
       if (k < M.obs_dim) {
         const double x = (double)ov[t];
         srow[k] = x;
-        srow[M.obs_dim + k] = x * x;
+        srow[M.obs_row + k] = x * x;
       }
     }
   }
@@ -951,7 +1024,7 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     if (col < kRowStats) {
       if (A.packed) {
         // packed layout of the VecNormalize kernels: [ sum obs[D], sumsq obs[D], n, sum ret, sumsq ret ]
-        const int D = M.obs_dim;
+        const int D = M.obs_row;
         A.packed[col < 2 * D ? col : col + 1] = tot;
       }
     } else {
@@ -959,7 +1032,7 @@ __global__ void __launch_bounds__(128, 4) mimic_step_kernel(const StepArgs A, co
     }
   }
   if (threadIdx.x == 0) {
-    if (A.packed) A.packed[2 * M.obs_dim] = (double)A.num_envs;
+    if (A.packed) A.packed[2 * M.obs_row] = (double)A.num_envs;
     *A.cta_ticket = 0u;
   }
 }
@@ -1061,6 +1134,11 @@ __global__ void state_copy_kernel(float* state_f, int* state_i, int* state_as, f
 // 4 x (model + 8 environments + 1 KB reserved) <= 228 KB
 static_assert(4 * (sizeof(DevModel) + 8 * sizeof(EnvSmem<16>) + 1024) <= 228 * 1024,
               "walker3d: four blocks per SM must fit in shared memory");
+// the statistics row of an environment, 2 * obs_row + 2 + DRL_STATS_COUNT doubles, lives in E.Mt: it fits the widest
+// row, walker_165cm_65kg (47 base columns, nv 19) with DRL_MAX_REF_OBS reference-pose frames
+static_assert(47 + DRL_MAX_REF_OBS * (19 - 1) <= DRL_MAX_OBS_TOTAL, "DRL_MAX_OBS_TOTAL holds the widest row");
+static_assert(2 * DRL_MAX_OBS_TOTAL + 2 + DRL_STATS_COUNT <= (int)(sizeof(EnvSmem<32>::Mt) / sizeof(double)),
+              "the statistics row of the widest observation fits E.Mt");
 
 size_t step_smem_bytes(int G, int envs_per_block, bool pd) {
   const size_t model = pd ? sizeof(DevModel) : kModelBytesTorque;

@@ -114,7 +114,7 @@ extern "C" int drl_vecnorm_moments(const float* obs, int32_t n, int32_t d, const
 // last merge.  "Immediate" calls (VecNormalize.reset) exchange their own moments at once and leave the cycle alone.
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int kMaxPeers = 8;
-constexpr int kMaxPayload = 2 * DRL_MAX_OBS + 3;
+constexpr int kMaxPayload = 2 * DRL_MAX_OBS_TOTAL + 3;
 
 struct DrlComm {
   int world = 1, rank = 0, payload = 0, device = 0;
@@ -155,7 +155,7 @@ __global__ void __launch_bounds__(256) vecnorm_step_kernel(
     unsigned char* __restrict__ done_out, float clip_obs, float clip_rew, float eps, int upd_obs, int upd_ret,
     int norm_obs, int norm_rew, const CommView cv) {
   __shared__ double s_tot[kMaxPayload];
-  __shared__ float s_mean[DRL_MAX_OBS], s_inv[DRL_MAX_OBS + 1];
+  __shared__ float s_mean[DRL_MAX_OBS_TOTAL], s_inv[DRL_MAX_OBS_TOTAL + 1];
   __shared__ unsigned long long s_ctr[2];
   const int P = cv.payload;        // 2d + 3
   if (threadIdx.x < 2) s_ctr[threadIdx.x] = reinterpret_cast<volatile unsigned long long*>(cv.step)[threadIdx.x];
@@ -262,7 +262,7 @@ __global__ void __launch_bounds__(256) vecnorm_step_kernel(
   } while (0)
 
 extern "C" int drl_comm_create(int32_t world, int32_t rank, int32_t obs_dim, DrlComm** out) {
-  if (!out || world < 1 || world > kMaxPeers || rank < 0 || rank >= world || obs_dim <= 0 || obs_dim > DRL_MAX_OBS)
+  if (!out || world < 1 || world > kMaxPeers || rank < 0 || rank >= world || obs_dim <= 0 || obs_dim > DRL_MAX_OBS_TOTAL)
     return DRL_ERR_INVALID;
   auto c = std::make_unique<DrlComm>();
   c->world = world; c->rank = rank; c->payload = 2 * obs_dim + 3;
@@ -317,7 +317,7 @@ extern "C" int drl_vecnorm_step(const float* obs_in, float* obs_out, const float
                                 int32_t d, const double* packed, const double* rms_in, double* rms_out, float* ret,
                                 const uint8_t* done, uint8_t* done_out, float clip_obs, float clip_rew, float eps,
                                 int32_t flags, DrlComm* c, int32_t sync_every, void* stream) {
-  if (!obs_in || !obs_out || !rms_in || !rms_out || n <= 0 || d <= 0 || d > DRL_MAX_OBS || rms_in == rms_out || !c)
+  if (!obs_in || !obs_out || !rms_in || !rms_out || n <= 0 || d <= 0 || d > DRL_MAX_OBS_TOTAL || rms_in == rms_out || !c)
     return DRL_ERR_INVALID;
   if (c->payload != 2 * d + 3 || !c->connected || sync_every < 0) return DRL_ERR_STATE;
   drl::CommView cv;

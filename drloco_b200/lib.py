@@ -41,6 +41,7 @@ PROTOTYPES = {
     "drl_set_speed_profile": (C.c_int, [vp, vp, i32]),
     "drl_set_seed": (C.c_int, [vp, C.c_uint64]),
     "drl_set_playback": (C.c_int, [vp, i32]),
+    "drl_set_ref_obs": (C.c_int, [vp, i32, vp]),
     "drl_set_actuation": (C.c_int, [vp, i32, vp, vp]),
     "drl_set_contact_termination": (C.c_int, [vp, C.c_uint32]),
     "drl_get_contact_terminations": (C.c_int, [vp, vp, vp]),

@@ -214,6 +214,13 @@ class B200MimicVecEnv:
             lib.check(self._lib.drl_set_contact_termination(self._handle, contact_body_mask(m)),
                       "drl_set_contact_termination")
         self._upload_mocap()
+        offs = self.cfg.ref_obs_offsets
+        if offs:
+            # reference-pose observations (EnvConfig.ref_obs_offsets): every row gets one frame per offset
+            self.spec.ref_frame_mirror()           # raises when the mirror table does not keep the qpos block
+            arr = np.ascontiguousarray(offs, np.int32)
+            lib.check(self._lib.drl_set_ref_obs(self._handle, len(offs), arr.ctypes.data_as(C.c_void_p)),
+                      "drl_set_ref_obs")
         self._ars_bins = None
         if self.cfg.adaptive_rsi > 0.0:
             # failure-weighted RSI (EnvConfig.adaptive_rsi): bins of 20 control steps of reference motion
@@ -268,9 +275,9 @@ class B200MimicVecEnv:
             c.rew_weights[i] = cfg.rew_weights[i]
         c.rew_scale, c.alive_bonus, c.fall_z = cfg.rew_scale, cfg.alive_bonus, cfg.fall_z
         c.seed, c.env_id_offset = int(seed) & (2 ** 64 - 1), int(env_id_offset)
-        c.obs_dim, c.act_dim = s.obs_dim, s.act_dim
+        c.obs_dim, c.act_dim = s.base_obs_dim, s.act_dim      # the frames of ref_obs_offsets: drl_set_ref_obs
         oi, osn, ai, asn = s.mirror_tables()
-        for i in range(s.obs_dim):
+        for i in range(s.base_obs_dim):
             c.mirror_obs_idx[i], c.mirror_obs_sign[i] = int(oi[i]), float(osn[i])
         for i in range(s.act_dim):
             c.mirror_act_idx[i], c.mirror_act_sign[i] = int(ai[i]), float(asn[i])
@@ -1122,8 +1129,17 @@ class B200VecNormalize:
                     clip_obs=self.clip_obs, clip_reward=self.clip_reward, gamma=self.gamma, epsilon=self.epsilon,
                     norm_obs=self.norm_obs, norm_reward=self.norm_reward)
 
+    @staticmethod
+    def _check_width(sd: dict, D: int) -> None:
+        for k in ("obs_mean", "obs_var"):
+            w = np.size(sd[k])
+            if w != D:
+                raise ValueError(f"VecNormalize statistics: {k} has {w} columns, the observation of this env has {D} "
+                                 "(reference-pose frames change the width: EnvConfig.ref_obs_offsets)")
+
     def load_state_dict(self, sd: dict) -> None:
         D = self._D
+        self._check_width(sd, D)
         r = np.zeros(2 * D + 4)
         r[:D], r[D:2 * D], r[2 * D] = sd["obs_mean"], sd["obs_var"], sd["obs_count"]
         r[2 * D + 1], r[2 * D + 2], r[2 * D + 3] = sd["ret_mean"], sd["ret_var"], sd["ret_count"]
@@ -1155,6 +1171,8 @@ class B200VecNormalize:
         if not isinstance(sd, dict):
             from .checkpoint import read_sb3_vecnormalize
             sd = read_sb3_vecnormalize(path)
+        # before the wrapper attaches to the env: a refused file leaves the env as it was
+        B200VecNormalize._check_width(sd, venv.obs_dim)
         vn = B200VecNormalize(venv)
         vn.load_state_dict(sd)
         if "training" in sd:                      # SB3's VecNormalize.load restores the pickled flag

@@ -59,9 +59,20 @@ class WalkerSpec:
     mocap_paths: Tuple[Optional[str], ...] = (None,)   # the file of every clip (None: the walker's default recording)
 
     @property
+    def base_obs_dim(self) -> int:
+        """the reference's observation (phase | desired velocity | qpos[1:] | qvel): DrlConfig.obs_dim, the width of
+        the mirror tables"""
+        return self.qpos_block + (self.model.nv - 1) + self.model.nv
+
+    @property
+    def qpos_block(self) -> int:
+        """first column of the observation's qpos[1:] block"""
+        return (1 if self.phase_from_cursor else 2 * len(self.phase_joints)) + self.n_des_vel
+
+    @property
     def obs_dim(self) -> int:
-        n_phase = 1 if self.phase_from_cursor else 2 * len(self.phase_joints)
-        return n_phase + self.n_des_vel + (self.model.nv - 1) + self.model.nv
+        """the full row: the base observation, then one frame of nv - 1 reference qpos per EnvConfig.ref_obs_offsets"""
+        return self.base_obs_dim + len(self.cfg.ref_obs_offsets) * (self.model.nv - 1)
 
     @property
     def act_dim(self) -> int:
@@ -72,8 +83,8 @@ class WalkerSpec:
         return self.cfg.frame_skip
 
     def mirror_tables(self):
-        """(obs_idx, obs_sign, act_idx, act_sign); identity when mirroring is off."""
-        D, A = self.obs_dim, self.act_dim
+        """(obs_idx, obs_sign, act_idx, act_sign) of the base observation; identity when mirroring is off."""
+        D, A = self.base_obs_dim, self.act_dim
         oi, osn = np.arange(D, dtype=np.int32), np.ones(D, np.float32)
         ai, asn = np.arange(A, dtype=np.int32), np.ones(A, np.float32)
         if self.mirror:
@@ -82,6 +93,21 @@ class WalkerSpec:
             ai = np.array(MIRROR_ACT_IDX, np.int32)
             asn[MIRROR_ACT_NEG] = -1.0
         return oi, osn, ai, asn
+
+    def ref_frame_mirror(self):
+        """(idx, sign) [nv - 1] of a reference-pose frame: entry j of a mirrored frame is sign[j] * frame[idx[j]], the
+        qpos-block part of the observation's mirror table (ref_frame_mirror_map)."""
+        oi, osn, _, _ = self.mirror_tables()
+        return ref_frame_mirror_map(oi, osn, self.qpos_block, self.model.nv - 1)
+
+
+def ref_frame_mirror_map(obs_idx, obs_sign, block: int, n: int):
+    """The part of an observation mirror table (obs[k] <- sign[k] * obs[idx[k]]) over the columns [block, block + n),
+    relative to the block; ValueError when it reads a column outside the block (the map is not closed)."""
+    idx = np.asarray(obs_idx, np.int64)[block:block + n] - block
+    if idx.shape != (n,) or (idx < 0).any() or (idx >= n).any():
+        raise ValueError(f"the mirror table does not map the qpos block [{block}, {block + n}) onto itself")
+    return idx.astype(np.int32), np.asarray(obs_sign, np.float32)[block:block + n].copy()
 
 
 def speed_profile(speeds, speed_profile_duration, control_freq) -> np.ndarray:

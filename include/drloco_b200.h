@@ -29,9 +29,11 @@ extern "C" {
 #define DRL_MAX_SPHERE 16
 #define DRL_MAX_BOX 8
 #define DRL_MAX_SITE 16
-#define DRL_MAX_OBS 64
+#define DRL_MAX_OBS 64             /* DrlConfig.obs_dim and its mirror tables */
 #define DRL_MAX_PHASE_JOINTS 4
 #define DRL_MAX_EE 4
+#define DRL_MAX_REF_OBS 3          /* reference-pose frames of drl_set_ref_obs */
+#define DRL_MAX_OBS_TOTAL 101      /* widest observation row: obs_dim + the frames (walker_165cm_65kg: 47 + 3 * 18) */
 
 typedef enum {
   DRL_OK = 0,
@@ -160,7 +162,8 @@ int drl_upload_mocap(DrlEnv* env, int32_t cursor_mode, int32_t increment, const 
 
 /* VecEnv.reset (SB3) = MujocoEnv.reset + MimicEnv.reset_model (mimic_env.py:526-572) for every env whose mask byte is
  * non-zero (mask == NULL: all).  inj_istep/inj_pos (device int32[N], nullable) inject the RSI draw instead of the
- * library's generator (parity tests; straight_walk_trajecs.py:460-474).  obs: device float [N][obs_dim]. */
+ * library's generator (parity tests; straight_walk_trajecs.py:460-474).  obs: device float [N][obs_dim] (with
+ * reference-pose frames, drl_set_ref_obs: [N][obs_dim + n * (nv - 1)], as every obs row below). */
 int drl_reset(DrlEnv* env, const uint8_t* mask, const int32_t* inj_istep, const int32_t* inj_pos, float* obs,
               void* stream);
 
@@ -358,6 +361,23 @@ int drl_get_clip_stats(DrlEnv* env, int64_t* out, void* stream);
  * reward of every such step is its maximum.  Rendering is not part of this library. */
 int drl_set_playback(DrlEnv* env, int32_t on);
 
+/* Reference-pose observations (not in the reference, whose policy sees the phase, the desired velocity and its own
+ * state only): n frames are appended to every observation row, frame f = the reference qpos[1:] (nv - 1 floats, the
+ * entries of the observation's own qpos block) offsets[f] control steps ahead.  Exactly: for the cursor c the
+ * observation was built at, apply StraightWalkingTrajectories.next / BaseReferenceTrajectories.next (the library's
+ * per-clip wrap included) offsets[f] times to a copy of c and read the reference qpos there with the episode's COM-Z
+ * shift: the target the pose reward compares against that many steps later if the episode runs on.  A mirrored
+ * observation (mirror_policy, a left step) mirrors every frame with its own decision, through the qpos-block part of
+ * mirror_obs_idx / mirror_obs_sign, which must map the block onto itself.  Frames are in every row the library writes:
+ * obs, terminal_obs (at the pre-reset cursor), the auto-reset and drl_reset observations, in playback, evaluation mode
+ * and with a speed profile.  From the call on, drl_reset / drl_step write rows of obs_dim + n * (nv - 1) floats and the
+ * fused VecNormalize moments (drl_attach_vecnorm) cover the whole row: packed has 2 * that + 3 doubles.  n = 0 is off,
+ * the state after drl_upload_model.  offsets: HOST int32 [n], strictly increasing, each in [1, 256]; n <=
+ * DRL_MAX_REF_OBS.  DRL_ERR_STATE before drl_upload_model, after the first drl_reset or drl_step, and while a
+ * VecNormalize is attached; DRL_ERR_INVALID for bad offsets or a mirror map that leaves the qpos block.  Synchronises
+ * the device; a failed call changes nothing. */
+int drl_set_ref_obs(DrlEnv* env, int32_t n, const int32_t* offsets);
+
 /* test / tuning hooks: frame_skip_override >= 0 replaces cfg.frame_skip (0 = environment logic only, used to test the
  * reward / cursor / reset path on injected states); block_threads > 0 sets the CTA size; enable_dump keeps, per env, the
  * intermediate results of the last dynamics evaluation (mass matrix, bias force, qacc) for drl_debug_read (host buffer). */
@@ -375,7 +395,7 @@ int drl_vecnorm_moments(const float* obs, int32_t n, int32_t d, const float* rew
 /* Fused VecNormalize path (what B200VecNormalize uses): ONE kernel per step after drl_step.
  *
  * drl_attach_vecnorm: from now on drl_step itself maintains ret = ret*gamma + rew (device float [N], in/out) and leaves
- *   the batch moments of the step in packed (device double [2*obs_dim+3], layout as drl_vecnorm_moments) - computed in
+ *   the batch moments of the step in packed (device double [2*D+3], D the row width, layout as drl_vecnorm_moments) - computed in
  *   the step kernel's epilogue from the observations it returns, block sums then a fixed-order grid sum, no atomics:
  *   the moments (and the Monitor statistics, drl_get_stats) are bit-reproducible.  Two NULLs detach.
  * DrlComm: the statistics exchange between the ranks of one node (one process per GPU) without a host-issued

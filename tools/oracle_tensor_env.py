@@ -24,7 +24,8 @@ from oracle.physics import OraclePhysics              # noqa: E402
 class _Inner:
     def __init__(self, venv, spec):
         self._v, self.spec = venv, spec
-        self.num_envs, self.obs_dim, self.act_dim = venv.num_envs, spec.obs_dim, spec.act_dim
+        # the oracle restates the reference's observation: the base width, no reference-pose frames
+        self.num_envs, self.obs_dim, self.act_dim = venv.num_envs, spec.base_obs_dim, spec.act_dim
         self.device = torch.device("cpu")
         self._reset_counts()
 

@@ -55,6 +55,9 @@ def main():
                     help="reference motion file(s); several make a mocap library (default: the shipped recording)")
     ap.add_argument("--clip-weights", type=float, nargs="+", metavar="W",
                     help="RSI weight of every --mocap clip (default: proportional to the clips' sample counts)")
+    ap.add_argument("--ref-obs", type=int, nargs="+", metavar="K", default=[],
+                    help="append the reference pose K control steps ahead to the observation, one frame per K "
+                         "(EnvConfig.ref_obs_offsets; at most 3, strictly increasing)")
     args = ap.parse_args()
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", "0"), ("WORLD_SIZE", "1"), ("LOCAL_RANK", "0")))
     if world > 1:
@@ -64,16 +67,17 @@ def main():
         torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local),
                                              timeout=datetime.timedelta(seconds=90))
     env_cfg = None
-    if args.actuation == "pd" or args.contact_termination or args.adaptive_rsi > 0.0:
+    if args.actuation == "pd" or args.contact_termination or args.adaptive_rsi > 0.0 or args.ref_obs:
         if args.cpu_oracle:
-            ap.error("--actuation pd, --contact-termination and --adaptive-rsi run on the GPU env only")
+            ap.error("--actuation pd, --contact-termination, --adaptive-rsi and --ref-obs run on the GPU env only")
         from drloco_b200.config import EnvConfig
         pd = dict()
         if args.actuation == "pd":
             gain = lambda g: None if g is None else (g[0] if len(g) == 1 else tuple(g))   # noqa: E731
             pd = dict(actuation="pd", pd_kp=gain(args.kp), pd_kv=gain(args.kv))
         env_cfg = EnvConfig(env_id="StraightMimicWalker", seed=33 + args.seed + 100 * rank,
-                            contact_termination=args.contact_termination, adaptive_rsi=args.adaptive_rsi, **pd)
+                            contact_termination=args.contact_termination, adaptive_rsi=args.adaptive_rsi,
+                            ref_obs_offsets=tuple(args.ref_obs), **pd)
     library = args.mocap is not None and len(args.mocap) > 1
     if (args.mocap or args.clip_weights) and args.cpu_oracle:
         ap.error("--mocap and --clip-weights run on the GPU env only")
@@ -138,7 +142,9 @@ def main():
     clips = None
     if library:
         cs = env.venv.clip_stats()
-        clips = [dict(c, **{k: int(cs[k][i]) for k in cs}) for i, c in enumerate(env.venv.mocap_clips())]
+        # file names only: a curve records which recordings it used, not where they were on the machine
+        clips = [dict(c, path=None if c["path"] is None else os.path.basename(c["path"]),
+                      **{k: int(cs[k][i]) for k in cs}) for i, c in enumerate(env.venv.mocap_clips())]
     if rank == 0:
         os.makedirs(os.path.dirname(args.out) or ".", exist_ok=True)
         with open(args.out, "w") as f:
@@ -148,6 +154,7 @@ def main():
                        "replicas_bit_identical": lockstep,
                        "actuation": args.actuation, "pd_kp": args.kp, "pd_kv": args.kv,
                        "contact_termination": args.contact_termination, "adaptive_rsi": args.adaptive_rsi,
+                       "ref_obs_offsets": args.ref_obs, "obs_dim": int(env.venv.obs_dim) if not args.cpu_oracle else None,
                        "config": {k: v for k, v in vars(cfg).items()}, "curve": agent.log, "evaluation": ev,
                        "evaluation_steady_state_counters": ev2, "adaptive_rsi_table_at_end": ars,
                        "mocap_clips_at_end": clips}, f, indent=1)
